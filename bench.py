@@ -2,7 +2,7 @@
 """Benchmark of the KGE hot path: KG triples/s of the fused train step (headline) plus users/s of
 the fused full-sort top-k, on synthetic KGs of BASELINE.json's shapes.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One JSON line on stdout (rank 0).  `value` = positive (rec + KG) triples per second over all
@@ -12,6 +12,10 @@ loss.item() (D2H) every step.  `roofline` follows SURVEY.md 8(d): algorithmic by
 triple = 24*d*T*(2+K) + 8*(3+K), over the measured HBM peak.  `--impl reference` times the
 reference's own algorithm on the host cores (the torch-CPU oracle port: the same torch operators
 the reference's Python calls, dense autograd + dense torch.optim.Adam).
+
+`--dump-outputs DIR` writes what the headline train step hands its caller after the last timed step -- the loss and
+the updated tables -- as DIR/<name>.npy (float32), so that two builds can be compared output for output on the same
+seeded inputs.
 """
 
 from __future__ import annotations
@@ -26,6 +30,9 @@ import time
 
 import numpy as np
 import torch
+
+# the benchmark leaves the tree it runs from as it found it (that tree may be read-only): no bytecode caches
+sys.dont_write_bytecode = True
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -219,6 +226,28 @@ def time_train_device(model, dev_batches, steps, warmup, flush_buf, world):
     fwd = np.array([e[0].elapsed_time(e[1]) for e in ev])
     upd = np.array([e[1].elapsed_time(e[2]) for e in ev])
     return fwd, upd, float(loss.item())   # per-step milliseconds (forward / backward = exchange + Adam)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, state, loss):
+    """The loss of the last timed step and the tables it left (`state`: the model's state_dict(), which first brings
+    every lazily updated row to the current step, as it does for any caller), as float32 .npy files of at most
+    DUMP_BYTES in all.  Smaller tables are written whole; what does not fit shares the rest of the budget equally, as
+    a sorted sample of rows drawn with a fixed seed, so every run and every build writes the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([loss], dtype=np.float32))
+    tables = sorted(state.items(), key=lambda kv: kv[1].numel())
+    budget = DUMP_BYTES - 4096   # (the loss file and the .npy headers)
+    for i, (name, t) in enumerate(tables):
+        row_bytes = 4 * t[0].numel()
+        keep = min(t.shape[0], budget // (len(tables) - i) // row_bytes)
+        budget -= keep * row_bytes
+        if keep < t.shape[0]:
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], keep, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
 
 
 def time_train_e2e(model, host_batches, steps, warmup, world, device, reference_order=False):
@@ -540,7 +569,12 @@ def main():
     ap.add_argument("--workload", default="cfg2_transe_ml1m", choices=sorted(WORKLOADS))
     ap.add_argument("--no-extras", action="store_true", help="headline only (used under ncu)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and the tables of the last timed train step as DIR/<name>.npy (float32, at "
+                         "most 64 MB: larger tables as a fixed, seeded sample of rows)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA train step computed: it needs --impl ours")
     args.warmup = max(args.warmup, 3)
     rank, world, local = dist_info()
     # stdout carries the one JSON line and nothing else: libraries that print to fd 1 (NCCL's version banner,
@@ -628,6 +662,11 @@ def main():
     with ClockSampler(local) as clocks:
         fwd, upd, last_loss = time_train_device(model, dev_t, args.steps, args.warmup, flush_buf, world)
     clk = clocks.summary()
+    if args.dump_outputs:
+        state = model.state_dict()   # on every rank: the lazy-row flush is the same work on all of them
+        if rank == 0:
+            dump_outputs(args.dump_outputs, state, last_loss)
+        del state
     per_step = fwd + upd
     step_ms = max_over_ranks(float(per_step.mean()), device, world)          # EXACTLY K timed steps, max over ranks
     step_med_ms = max_over_ranks(float(np.median(per_step)), device, world)

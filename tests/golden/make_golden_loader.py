@@ -46,10 +46,11 @@ def main():
         "inter_user": inter["user_id"].numpy().astype(np.int32), "inter_item": inter["item_id"].numpy().astype(np.int32),
         "kg_head": kg["head_id"].numpy().astype(np.int32), "kg_rel": kg["relation_id"].numpy().astype(np.int32),
         "kg_tail": kg["tail_id"].numpy().astype(np.int32),
-        # what the reference KGSampler filters with: the dataset's full head / tail arrays (sampler.py:321-336)
-        "sampler_heads": np.asarray(dataset.head_entities).astype(np.int32),
-        "sampler_tails": np.asarray(dataset.tail_entities).astype(np.int32),
     }
+    # what the reference KGSampler filters with, the dataset's full head / tail arrays (sampler.py:321-336), are the
+    # KG triples' own columns: the tests filter with kg_head / kg_tail, so they are not stored twice
+    assert np.array_equal(np.asarray(dataset.head_entities), out["kg_head"])
+    assert np.array_equal(np.asarray(dataset.tail_entities), out["kg_tail"])
     # the rec sampler's train-phase used ids (sampler.py:229-252) as COO
     used = gl._sampler.used_ids
     uu, ii = [], []

@@ -20,7 +20,7 @@ def test_device_kg_loader_gpu_matches_reference_epochs():
     stream = MTStream(state=("MT19937", g["mt_key"], int(g["mt_pos"])))
     n_users, n_items, n_ent = int(g["n_users"]), int(g["n_items"]), int(g["n_entities"])
     rec = RecSampler(g["used_user"].astype(np.int64), g["used_item"].astype(np.int64), n_users, n_items, stream=stream)
-    kg = KGSampler(heads=g["sampler_heads"].astype(np.int64), tails=g["sampler_tails"].astype(np.int64), entity_num=n_ent,
+    kg = KGSampler(heads=g["kg_head"].astype(np.int64), tails=g["kg_tail"].astype(np.int64), entity_num=n_ent,
                    stream=stream)
     loader = DeviceKGLoader(g["inter_user"], g["inter_item"], g["kg_head"], g["kg_rel"], g["kg_tail"], rec, kg,
                             batch_size=int(g["batch"]), seed=int(g["seed"]), device="cuda")
@@ -48,7 +48,7 @@ def test_device_kg_loader_feeds_the_fused_step():
     stream = MTStream(seed=2024)
     n_users, n_items, n_ent, n_rel = (int(g[k]) for k in ("n_users", "n_items", "n_entities", "n_relations"))
     rec = RecSampler(g["used_user"].astype(np.int64), g["used_item"].astype(np.int64), n_users, n_items, stream=stream)
-    kg = KGSampler(heads=g["sampler_heads"].astype(np.int64), tails=g["sampler_tails"].astype(np.int64), entity_num=n_ent,
+    kg = KGSampler(heads=g["kg_head"].astype(np.int64), tails=g["kg_tail"].astype(np.int64), entity_num=n_ent,
                    stream=stream)
     loader = DeviceKGLoader(g["inter_user"], g["inter_item"], g["kg_head"], g["kg_rel"], g["kg_tail"], rec, kg,
                             batch_size=2048, seed=2024)

@@ -39,7 +39,7 @@ def _loader(g):
     gen.set_state(("MT19937", g["mt_key"], int(g["mt_pos"])))
     n_users, n_items, n_ent = int(g["n_users"]), int(g["n_items"]), int(g["n_entities"])
     rec = _OracleSampler(gen, g["used_user"], g["used_item"], n_users, n_items)
-    kg = _OracleSampler(gen, g["sampler_heads"], g["sampler_tails"], n_ent, n_ent)
+    kg = _OracleSampler(gen, g["kg_head"], g["kg_tail"], n_ent, n_ent)
     loader = DeviceKGLoader(g["inter_user"], g["inter_item"], g["kg_head"], g["kg_rel"], g["kg_tail"], rec, kg,
                             batch_size=int(g["batch"]), seed=int(g["seed"]), device="cpu", gather=lambda table, idx: table.index_select(0, idx))
     return loader, gen
