@@ -3,7 +3,7 @@
 Public surface (mirrors the reference names so a hopwise user can switch imports):
   TransE, DistMult, RotatE, ComplEx      KnowledgeRecommender-compatible models (recommender.py)
   KGSampler, RecSampler                  bit-exact GPU negative samplers (sampler.py)
-  FusedCollector, evaluate_full_sort     fused full-sort top-k evaluation (evaluator.py)
+  FusedCollector, evaluate_full_sort     fused full-sort top-k and GAUC evaluation (evaluator.py)
   enable_row_sparse_data_parallel        row-sparse / dense gradient exchange over NCCL (distributed.py)
   DevicePrefetcher                       host->device batch staging one step ahead (loader.py)
 """

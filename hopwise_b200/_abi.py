@@ -112,6 +112,11 @@ PROTOTYPES = {
         C.c_int,
         [_MP, _P, _P, C.c_int64, C.c_int, C.c_int64, _P, _P, C.c_int, C.c_int32, _P, _P, _P, C.c_int64, _P],
     ),
+    "kge_full_sort_rank_workspace_bytes": (C.c_int64, [_MP, C.c_int64, C.c_int64, C.c_int64]),
+    "kge_full_sort_rank_counts": (
+        C.c_int,
+        [_MP, _P, _P, C.c_int64, C.c_int, C.c_int64, _P, _P, C.c_int, _P, _P, _P, _P, _P, _P, C.c_int64, _P],
+    ),
     "kge_copy_h2d_async": (C.c_int, [_P, _P, C.c_int64, _P]),
     "kge_multimem_all_reduce_f32": (C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, _P]),
     "kge_owner_adam_step": (

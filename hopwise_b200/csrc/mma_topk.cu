@@ -1122,50 +1122,10 @@ __global__ void __launch_bounds__(RS_WARPS * 32, KGE_RS_MINB) rescore_topk_kerne
             }
           }
           if (ok) {
-            // the CUDA-core kernel's chain: parts in order, columns ascending, one fmaf per column; the
-            // loads of a 64-column block are all issued before the chain consumes them
+            // the CUDA-core kernel's chain: parts in order, columns ascending, one fmaf per column
             float acc = 0.f;
-            for (int p = 0; p < a.parts; ++p) {
-              const float* t = a.s.m.entity.w[p] + j * d;
-              const float* qp = q + p * d;
-              if ((d & 3) == 0) {
-                for (int c0 = 0; c0 < d; c0 += 64) {
-                  float4 tv[16];
-#pragma unroll
-                  for (int x = 0; x < 16; ++x)
-                    if (c0 + 4 * x < d) tv[x] = __ldg(reinterpret_cast<const float4*>(t + c0) + x);
-#pragma unroll
-                  for (int x = 0; x < 16; ++x) {
-                    if (c0 + 4 * x < d) {
-                      const float4 qv = *reinterpret_cast<const float4*>(qp + c0 + 4 * x);
-                      if (DIST) {
-                        const float e0 = qv.x - tv[x].x, e1 = qv.y - tv[x].y, e2 = qv.z - tv[x].z, e3 = qv.w - tv[x].w;
-                        acc = fmaf(e0, e0, acc);
-                        acc = fmaf(e1, e1, acc);
-                        acc = fmaf(e2, e2, acc);
-                        acc = fmaf(e3, e3, acc);
-                      } else {
-                        acc = fmaf(qv.x, tv[x].x, acc);
-                        acc = fmaf(qv.y, tv[x].y, acc);
-                        acc = fmaf(qv.z, tv[x].z, acc);
-                        acc = fmaf(qv.w, tv[x].w, acc);
-                      }
-                    }
-                  }
-                }
-              } else {
-#pragma unroll 8
-                for (int c = 0; c < d; ++c) {
-                  const float tv = __ldg(t + c);
-                  if (DIST) {
-                    const float e0 = qp[c] - tv;
-                    acc = fmaf(e0, e0, acc);
-                  } else {
-                    acc = fmaf(qp[c], tv, acc);
-                  }
-                }
-              }
-            }
+            for (int p = 0; p < a.parts; ++p)
+              acc = exact_chain<DIST ? MODE_DIST : MODE_DOT>(q + p * d, a.s.m.entity.w[p] + j * d, d, acc);
             const bool in = !have_tau || (DIST ? (acc <= hi_acc) : (acc >= lo_a));
             if (in) key = make_key(DIST ? (margin - sqrtf(acc)) : acc, (uint32_t)j);
           }

@@ -18,7 +18,9 @@
 // of 32 floats; each thread accumulates a 4x4 register block.  The epilogue either stores
 // the dense [n, n_targets] scores (API parity: the unchanged trainer mutates that tensor) or
 // keeps a per-row sorted top-k list of 64-bit (score, ~id) keys in shared memory, so the dense
-// matrix never exists (800 GB at 1M x 200k).  Order: score descending, id ascending.
+// matrix never exists (800 GB at 1M x 200k).  Order: score descending, id ascending.  A third
+// epilogue counts, for listed targets (the positives), the targets scoring above and equal to
+// them over the whole masked row: the exact ranks GAUC reads (collector.py's rec.meanrank).
 #include <math.h>
 
 #include "common.cuh"
@@ -186,7 +188,19 @@ struct TileArgs {
   const int32_t* row_map;
   const int32_t* row_count;
   int64_t row_begin, row_end;
+  // rank epilogue (see rank_thresholds_kernel): the positives CSR, their scores sorted per row and the counters
+  const int64_t* pos_off;
+  const float* rank_thr;       // [n_pos] sorted ascending inside every row
+  const float* rank_lo;        // [n] lowest finite threshold of the row (+inf: none)
+  uint64_t* rank_bins;         // [2 * n_pos]
+  uint64_t* rank_unmasked;     // [n]
+  uint64_t* rank_ninf;         // [n]
+  int64_t rank_cap;            // positives the workspace holds
 };
+
+// Epilogue of the tile kernel: the dense scores, the per-row top-k, or the rank counts of listed targets.
+constexpr int EPI_DENSE = 0, EPI_TOPK = 1, EPI_RANK = 2;
+constexpr int RANK_SM = 16;   // thresholds a row keeps in shared memory; rows with more count in global memory
 
 __device__ __forceinline__ void build_queries(const ScoreArgs& a, const int64_t* rowid, int nrows, int kpad, float* Qs,
                                               const float* proj = nullptr) {
@@ -231,14 +245,13 @@ __device__ __forceinline__ void load_target_chunk(const float* __restrict__ W, i
   }
 }
 
-// MODE: how a (query, target) pair of rows is contracted -- 0 dot product, 1 squared distance (score = margin - sqrt),
-// 2 torus distance sum(min(x^2, 1 - x^2)) on frac()ed rows (score = -4 * sum).  Zero padding contributes 0 in all three.
-// 3 = mode 1 on rows projected by one relation's factor c = 1 - sum(w) * w (TransH over items: every query row takes the
-// user->item relation, so one factor vector serves the whole launch; it is built once per CTA in shared memory).
-constexpr int MODE_DOT = 0, MODE_DIST = 1, MODE_TORUS = 2, MODE_PROJ = 3;
-template <int MODE, bool TOPK>
-__global__ void __launch_bounds__(TILE_THREADS) fullsort_tile_kernel(const TileArgs a) {
+// MODE: how a (query, target) pair of rows is contracted (score_common.cuh).  EPI: what the sweep does with the scores.
+// The rank epilogue asks for two CTAs per SM (128 registers): under the compiler's default budget it spills.
+template <int MODE, int EPI>
+__global__ void __launch_bounds__(TILE_THREADS, EPI == EPI_RANK ? 2 : 0) fullsort_tile_kernel(const TileArgs a) {
   constexpr bool DIST = MODE == MODE_DIST || MODE == MODE_PROJ;
+  constexpr bool TOPK = EPI == EPI_TOPK, RANK = EPI == EPI_RANK;
+  constexpr bool MASKED = EPI != EPI_DENSE;   // the trainer's masking: column 0 and the history -> -inf
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int model = a.s.m.model;
   const int parts = (model == KGE_ROTATE || model == KGE_COMPLEX) ? 2 : 1;
@@ -253,26 +266,20 @@ __global__ void __launch_bounds__(TILE_THREADS) fullsort_tile_kernel(const TileA
   uint64_t* lists = reinterpret_cast<uint64_t*>(Ts + BT * TS);  // [BU][k]
   uint64_t* cand = lists + (TOPK ? BU * k : 0);                 // [BU][BT]
   uint64_t* thr = cand + (TOPK ? BU * BT : 0);                  // [BU]
-  uint32_t* maskbits = reinterpret_cast<uint32_t*>(thr + (TOPK ? BU : 0));  // [BU][BT/32]
-  int* cnt = reinterpret_cast<int*>(maskbits + (TOPK ? BU * (BT / 32) : 0));  // [BU]
+  uint32_t* maskbits = reinterpret_cast<uint32_t*>(thr + (TOPK ? BU : 0));  // [BU][BT/32] (top-k and rank)
+  int* cnt = reinterpret_cast<int*>(maskbits + (MASKED ? BU * (BT / 32) : 0));  // [BU]
   int* llen = cnt + (TOPK ? BU : 0);                                        // [BU]
   int64_t* cursor = reinterpret_cast<int64_t*>(llen + (TOPK ? BU : 0));     // [BU] (8-byte aligned by layout)
-  int64_t* rowid = cursor + (TOPK ? BU : 0);                                // [BU] query row of each slot
+  int64_t* rowid = cursor + (MASKED ? BU : 0);                              // [BU] query row of each slot
   float* Cs = reinterpret_cast<float*>(rowid + BU);                         // [kpad] projection factor (MODE_PROJ)
-  if (MODE == MODE_PROJ) {
-    // c = 1 - sum(w) * w of the user->item relation's hyperplane vector (relation part 1), zero beyond d
-    __shared__ float s_part[TILE_THREADS / 32];
-    const float* wv = a.s.m.relation.w[1] + (int64_t)a.s.rel_row * d;
-    float part = 0.f;
-    for (int c = threadIdx.x; c < d; c += blockDim.x) part += __ldg(wv + c);
-    part = warp_sum(part);
-    if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = part;
-    __syncthreads();
-    float sw = 0.f;
-    for (int i = 0; i < TILE_THREADS / 32; ++i) sw += s_part[i];
-    for (int c = threadIdx.x; c < kpad; c += blockDim.x) Cs[c] = c < d ? 1.f - sw * __ldg(wv + c) : 0.f;
-    __syncthreads();
-  }
+  // rank only (kpad is a multiple of 32: rbase stays 8-byte aligned)
+  int64_t* rbase = reinterpret_cast<int64_t*>(Cs + (MODE == MODE_PROJ ? kpad : 0));  // [BU] pos_off of the row
+  float* rthr = reinterpret_cast<float*>(rbase + (RANK ? BU : 0));         // [BU][RANK_SM] sorted thresholds
+  uint32_t* rcnt = reinterpret_cast<uint32_t*>(rthr + (RANK ? BU * RANK_SM : 0));  // [BU][2 * RANK_SM] bins
+  float* rlo = reinterpret_cast<float*>(rcnt + (RANK ? BU * 2 * RANK_SM : 0));    // [BU] lowest finite threshold
+  int* rm = reinterpret_cast<int*>(rlo + (RANK ? BU : 0));                        // [BU] thresholds of the row
+  if (RANK && a.pos_off[a.s.n] > a.rank_cap) return;   // (the workspace was sized for fewer positives)
+  if (MODE == MODE_PROJ) proj_factor<TILE_THREADS>(a.s, kpad, Cs);
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int tu = warp;  // users 4*tu .. 4*tu+3
@@ -289,11 +296,33 @@ __global__ void __launch_bounds__(TILE_THREADS) fullsort_tile_kernel(const TileA
     rowid[u] = u < nrows ? (a.row_map ? (int64_t)__ldg(a.row_map + row0 + u) : row0 + u) : 0;
   __syncthreads();
   build_queries(a.s, rowid, nrows, kpad, Qs, MODE == MODE_PROJ ? Cs : nullptr);
-  if (TOPK) {
+  if (RANK) {
     for (int u = threadIdx.x; u < BU; u += blockDim.x) {
-      thr[u] = 0ull;
-      llen[u] = 0;
-      cnt[u] = 0;
+      int64_t base = 0, m = 0;
+      float lo = INFINITY;
+      if (u < nrows) {
+        base = a.pos_off[rowid[u]];
+        m = a.pos_off[rowid[u] + 1] - base;
+        lo = a.rank_lo[rowid[u]];
+      }
+      rbase[u] = base;
+      rm[u] = (int)min(m, (int64_t)0x7fffffff);
+      rlo[u] = lo;
+      if (m <= RANK_SM) {
+        for (int i = 0; i < m; ++i) rthr[u * RANK_SM + i] = a.rank_thr[base + i];
+        for (int i = 0; i < 2 * RANK_SM; ++i) rcnt[u * 2 * RANK_SM + i] = 0u;
+      }
+    }
+  }
+  // unmasked targets and targets scoring -inf of the thread's four rows (rank epilogue)
+  uint32_t n_unm[4] = {0u, 0u, 0u, 0u}, n_ninf[4] = {0u, 0u, 0u, 0u};
+  if (MASKED) {
+    for (int u = threadIdx.x; u < BU; u += blockDim.x) {
+      if (TOPK) {
+        thr[u] = 0ull;
+        llen[u] = 0;
+        cnt[u] = 0;
+      }
       int64_t cur = 0;
       if (u < nrows && a.hist_off) {
         // first history entry >= tile_lo * BT (history sorted ascending per row)
@@ -318,7 +347,7 @@ __global__ void __launch_bounds__(TILE_THREADS) fullsort_tile_kernel(const TileA
 #pragma unroll
       for (int y = 0; y < 4; ++y) acc[x][y] = 0.f;
 
-    if (TOPK) {
+    if (MASKED) {
       // history bits of this tile
       for (int i = threadIdx.x; i < BU * (BT / 32); i += blockDim.x) maskbits[i] = 0u;
       __syncthreads();
@@ -401,15 +430,48 @@ __global__ void __launch_bounds__(TILE_THREADS) fullsort_tile_kernel(const TileA
         const int64_t j = t0 + jo;
         if (j >= a.n_targets) continue;
         float sc = DIST ? (margin - sqrtf(acc[x][y])) : (MODE == MODE_TORUS ? -(4.f * acc[x][y]) : acc[x][y]);
-        if (!TOPK) {
+        if (!MASKED) {
           a.out[rowid[u] * a.n_targets + j] = sc;
-        } else {
-          const bool masked = (a.mask_first && j == 0) || ((maskbits[u * (BT / 32) + (jo >> 5)] >> (jo & 31)) & 1u);
-          if (masked) sc = -INFINITY;
+          continue;
+        }
+        const bool masked = (a.mask_first && j == 0) || ((maskbits[u * (BT / 32) + (jo >> 5)] >> (jo & 31)) & 1u);
+        if (masked) sc = -INFINITY;
+        if (TOPK) {
           const uint64_t key = make_key(sc, (uint32_t)j);
           if (key > thr[u]) {
             const int slot = atomicAdd(&cnt[u], 1);
             cand[u * BT + slot] = key;
+          }
+        } else {
+          n_unm[x] += masked ? 0u : 1u;
+          if (sc == -INFINITY) {
+            ++n_ninf[x];
+          } else if (sc >= rlo[u]) {
+            // Most targets score below the row's lowest positive and stop at the compare above.  The others are
+            // binned against the sorted thresholds w[0, m): with L = #{w < sc}, bin 2L counts scores equal to w[L]
+            // and bin 2L - 1 the scores strictly between w[L - 1] and w[L] (or above w[m - 1] when L = m).
+            const int m = rm[u];
+            if (m <= RANK_SM) {
+              const float* w = rthr + u * RANK_SM;
+              int lo = 0, hi = m;
+              while (lo < hi) {
+                const int mid = (lo + hi) >> 1;
+                if (w[mid] < sc) lo = mid + 1; else hi = mid;
+              }
+              atomicAdd(&rcnt[u * 2 * RANK_SM + ((lo < m && w[lo] == sc) ? 2 * lo : 2 * lo - 1)], 1u);
+            } else {
+              const int64_t base = rbase[u];
+              const int64_t mm = a.pos_off[rowid[u] + 1] - base;
+              const float* w = a.rank_thr + base;
+              int64_t lo = 0, hi = mm;
+              while (lo < hi) {
+                const int64_t mid = (lo + hi) >> 1;
+                if (w[mid] < sc) lo = mid + 1; else hi = mid;
+              }
+              atomicAdd(reinterpret_cast<unsigned long long*>(a.rank_bins + 2 * base +
+                                                              ((lo < mm && w[lo] == sc) ? 2 * lo : 2 * lo - 1)),
+                        1ull);
+            }
           }
         }
       }
@@ -430,6 +492,7 @@ __global__ void __launch_bounds__(TILE_THREADS) fullsort_tile_kernel(const TileA
       }
       // the next tile's first __syncthreads orders these writes before its reads
     }
+    if (RANK) __syncthreads();   // every warp is done with this tile's history bits before they are cleared
   }
 
   if (TOPK) {
@@ -438,6 +501,26 @@ __global__ void __launch_bounds__(TILE_THREADS) fullsort_tile_kernel(const TileA
       const int u = idx / k, i = idx - u * k;
       const uint64_t key = (i < llen[u]) ? lists[u * k + i] : 0ull;
       a.part_keys[((row0 - a.row_begin + u) * a.n_splits + blockIdx.y) * k + i] = key;
+    }
+  }
+  if (RANK) {
+    // this split's counts, added exactly (integer atomics: the result does not depend on the order)
+#pragma unroll
+    for (int x = 0; x < 4; ++x) {
+      const int u = 4 * tu + x;
+      const unsigned unm = __reduce_add_sync(0xffffffffu, n_unm[x]);
+      const unsigned ninf = __reduce_add_sync(0xffffffffu, n_ninf[x]);
+      if (lane == 0 && u < nrows) {
+        atomicAdd(reinterpret_cast<unsigned long long*>(a.rank_unmasked + rowid[u]), (unsigned long long)unm);
+        if (ninf) atomicAdd(reinterpret_cast<unsigned long long*>(a.rank_ninf + rowid[u]), (unsigned long long)ninf);
+      }
+    }
+    __syncthreads();
+    for (int idx = threadIdx.x; idx < nrows * 2 * RANK_SM; idx += blockDim.x) {
+      const int u = idx / (2 * RANK_SM), s = idx - u * (2 * RANK_SM);
+      const uint32_t c = rcnt[idx];
+      if (rm[u] <= RANK_SM && s < 2 * rm[u] && c)
+        atomicAdd(reinterpret_cast<unsigned long long*>(a.rank_bins + 2 * rbase[u] + s), (unsigned long long)c);
     }
   }
   if (!a.row_map) break;   // direct rows: the grid covers every row block
@@ -573,6 +656,171 @@ __global__ void __launch_bounds__(256) topk_metric_sums_kernel(const int32_t* __
   }
 }
 
+// ---- rank counts of listed targets (collector.py's rec.meanrank without the sorted [n, I] matrix) -------------------
+// Three launches: rank_thresholds_kernel scores every (row, positive) pair and sorts those scores per row, the tile
+// kernel's rank epilogue counts the targets against them during the sweep, rank_finalize_kernel turns the counts into
+// (greater, equal) per positive.
+struct RankPrep {
+  ScoreArgs s;
+  int64_t n_targets;
+  int kpad;
+  const int64_t* hist_off;
+  const int64_t* hist_items;
+  int mask_first;
+  const int64_t* pos_off;
+  const int64_t* pos_items;
+  int64_t cap;      // entries the workspace holds
+  float* score;     // [n_pos] the positive's masked score
+  float* sorted;    // [n_pos] the row's scores, ascending
+  int64_t* first;   // [n_pos] #{entries of the row scoring below this one} = first sorted position of its value
+  float* lo;        // [n] lowest finite score among the row's positives (+inf: none)
+};
+
+// One warp per row.  The positives are scored with exact_chain, the tile kernel's own sequence of fp32 operations, so
+// that every unmasked positive ties with itself in the sweep.  A masked positive (column 0 with mask_first, an id in
+// the row's history, or an id outside [0, n_targets), which is not a target) scores -inf.  The row's scores are then
+// placed by counting: position = #{smaller} + #{equal and listed earlier}.  That is quadratic in the row's positives,
+// which is cheap for evaluation's few positives per user and stays correct for any number.
+template <int MODE>
+__global__ void __launch_bounds__(TILE_THREADS) rank_thresholds_kernel(const RankPrep a) {
+  constexpr bool DIST = MODE == MODE_DIST || MODE == MODE_PROJ;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int parts = (a.s.m.model == KGE_ROTATE || a.s.m.model == KGE_COMPLEX) ? 2 : 1;
+  const int d = a.s.m.d;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = TILE_THREADS / 32;
+  float* Cs = reinterpret_cast<float*>(smem_raw);   // [kpad] projection factor (MODE_PROJ)
+  float* q = Cs + a.kpad + warp * parts * d;         // [parts * d] this warp's query row
+  if (a.pos_off[a.s.n] > a.cap) return;              // (the workspace was sized for fewer positives)
+  if (MODE == MODE_PROJ) proj_factor<TILE_THREADS>(a.s, a.kpad, Cs);
+  const float margin = (a.s.m.model == KGE_ROTATE) ? a.s.m.margin : 0.f;
+  for (int64_t row = (int64_t)blockIdx.x * warps + warp; row < a.s.n; row += (int64_t)gridDim.x * warps) {
+    for (int c = lane; c < d; c += 32) {
+      float q0, q1;
+      query_value(a.s, row, c, q0, q1, Cs);
+      q[c] = q0;
+      if (parts == 2) q[d + c] = q1;
+    }
+    __syncwarp();
+    const int64_t p0 = a.pos_off[row], p1 = a.pos_off[row + 1];
+    const int64_t h0 = a.hist_off ? a.hist_off[row] : 0, h1 = a.hist_off ? a.hist_off[row + 1] : 0;
+    float lo = INFINITY;
+    for (int64_t i = p0 + lane; i < p1; i += 32) {
+      const int64_t j = a.pos_items[i];
+      bool masked = j < 0 || j >= a.n_targets || (a.mask_first && j == 0);
+      if (!masked && h1 > h0) {
+        int64_t l = h0, h = h1;
+        while (l < h) {
+          const int64_t mid = (l + h) >> 1;
+          if (a.hist_items[mid] < j) l = mid + 1; else h = mid;
+        }
+        masked = l < h1 && a.hist_items[l] == j;
+      }
+      float sc = -INFINITY;
+      if (!masked) {
+        float acc = 0.f;
+        for (int p = 0; p < parts; ++p) acc = exact_chain<MODE>(q + p * d, a.s.m.entity.w[p] + j * d, d, acc, Cs);
+        sc = DIST ? (margin - sqrtf(acc)) : (MODE == MODE_TORUS ? -(4.f * acc) : acc);
+        lo = fminf(lo, sc);
+      }
+      a.score[i] = sc;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+    __syncwarp();   // the row's scores are visible to the whole warp
+    for (int64_t i = p0 + lane; i < p1; i += 32) {
+      const float s = a.score[i];
+      int64_t less = 0, before = 0;
+      for (int64_t x = p0; x < p1; ++x) {
+        const float v = a.score[x];
+        less += v < s;
+        before += (v == s) && (x < i);
+      }
+      a.sorted[p0 + less + before] = s;
+      a.first[i] = less;
+    }
+    if (lane == 0) a.lo[row] = lo;
+    __syncwarp();   // q is rewritten for the next row
+  }
+}
+
+// One warp per row: suffix sums over the row's 2m bins (in place), then per positive
+//   greater = #{targets scoring above} = the bins above its value's equal bin, equal = that bin;
+// a positive scoring -inf ties with every target scoring -inf (masked ones included) and trails all the others.
+__global__ void __launch_bounds__(256) rank_finalize_kernel(int64_t n, int64_t n_targets, int64_t cap,
+                                                            const int64_t* __restrict__ pos_off,
+                                                            const float* __restrict__ score,
+                                                            const int64_t* __restrict__ first, uint64_t* bins,
+                                                            const uint64_t* __restrict__ ninf,
+                                                            int64_t* __restrict__ greater_out,
+                                                            int64_t* __restrict__ equal_out,
+                                                            int64_t* __restrict__ n_unmasked_out) {
+  const int lane = threadIdx.x & 31, warps = blockDim.x >> 5;
+  const bool overflow = pos_off[n] > cap;
+  for (int64_t row = (int64_t)blockIdx.x * warps + (threadIdx.x >> 5); row < n; row += (int64_t)gridDim.x * warps) {
+    if (overflow) {   // nothing was counted: say so in every row instead of returning counts of nothing
+      if (lane == 0) n_unmasked_out[row] = -1;
+      continue;
+    }
+    const int64_t p0 = pos_off[row], p1 = pos_off[row + 1];
+    const int64_t slots = 2 * (p1 - p0);
+    uint64_t* b = bins + 2 * p0;
+    uint64_t carry = 0;
+    for (int64_t top = slots; top > 0; top -= 32) {   // lane 0 takes the highest slot of each round
+      const int64_t s = top - 1 - lane;
+      uint64_t v = s >= 0 ? b[s] : 0ull;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const uint64_t y = __shfl_up_sync(0xffffffffu, v, o);
+        if (lane >= o) v += y;
+      }
+      v += carry;
+      if (s >= 0) b[s] = v;
+      carry = __shfl_sync(0xffffffffu, v, 31);
+    }
+    __syncwarp();
+    const int64_t nf = (int64_t)ninf[row];
+    for (int64_t i = p0 + lane; i < p1; i += 32) {
+      int64_t gt, eq;
+      if (score[i] == -INFINITY) {
+        eq = nf;
+        gt = n_targets - nf;
+      } else {
+        const int64_t e = 2 * first[i];
+        const uint64_t above = e + 1 < slots ? b[e + 1] : 0ull;
+        gt = (int64_t)above;
+        eq = (int64_t)(b[e] - above);
+      }
+      greater_out[i] = gt;
+      equal_out[i] = eq;
+    }
+    __syncwarp();
+  }
+}
+
+struct RankLayout {
+  size_t lo, ninf, score, sorted, first, bins, total;
+};
+
+RankLayout rank_layout(int64_t n, int64_t n_pos) {
+  auto a16 = [](size_t x) { return (x + 15) / 16 * 16; };
+  RankLayout l;
+  size_t o = 0;
+  l.lo = o;
+  o += a16((size_t)n * 4);
+  l.ninf = o;
+  o += a16((size_t)n * 8);
+  l.score = o;
+  o += a16((size_t)n_pos * 4);
+  l.sorted = o;
+  o += a16((size_t)n_pos * 4);
+  l.first = o;
+  o += a16((size_t)n_pos * 8);
+  l.bins = o;
+  o += a16((size_t)n_pos * 16);
+  l.total = o;
+  return l;
+}
+
 int check_score_model(const kge_model_t* m) {
   KGE_REQUIRE(m, KGE_E_ARG, "model is NULL");
   KGE_REQUIRE(m->model >= KGE_TRANSE && m->model <= KGE_TRANSH, KGE_E_ARG, "unknown model kind %d", m->model);
@@ -590,11 +838,13 @@ struct TilePlan {
   int64_t n_blocks;
 };
 
-int plan_tiles(const kge_model_t* m, int64_t n, int64_t n_targets, int k, bool topk, TilePlan& pl) {
+int plan_tiles(const kge_model_t* m, int64_t n, int64_t n_targets, int k, int epi, TilePlan& pl) {
   const int parts = (m->model == KGE_ROTATE || m->model == KGE_COMPLEX) ? 2 : 1;
   pl.kpad = (m->d + KC - 1) / KC * KC;
   size_t smem = (size_t)BU * parts * pl.kpad * 4 + (size_t)BT * TS * 4;
-  if (topk) smem += (size_t)BU * k * 8 + (size_t)BU * BT * 8 + BU * 8 + BU * (BT / 32) * 4 + BU * 4 * 2 + BU * 8;
+  if (epi == EPI_TOPK) smem += (size_t)BU * k * 8 + (size_t)BU * BT * 8 + BU * 8 + BU * (BT / 32) * 4 + BU * 4 * 2 + BU * 8;
+  if (epi == EPI_RANK)   // maskbits, cursor | rbase, rthr, rcnt, rlo, rm
+    smem += BU * (BT / 32) * 4 + BU * 8 + BU * 8 + (size_t)BU * RANK_SM * 4 * 3 + BU * 4 * 2;
   smem += BU * 8;   // rowid
   if (m->model == KGE_TRANSH) smem += (size_t)pl.kpad * 4;   // projection factor
   pl.smem = smem;
@@ -602,7 +852,7 @@ int plan_tiles(const kge_model_t* m, int64_t n, int64_t n_targets, int k, bool t
   pl.n_blocks = (n + BU - 1) / BU;
   const int64_t n_tiles = (n_targets + BT - 1) / BT;
   int splits = 1;
-  if (topk) {
+  if (epi != EPI_DENSE) {
     // enough CTAs for two waves at 2 CTAs/SM, but at least 8 tiles per split
     const int64_t want = (int64_t)kge_num_sms() * 4;
     int64_t s = (want + pl.n_blocks - 1) / pl.n_blocks;
@@ -702,9 +952,9 @@ extern "C" int kge_transh_project(const float* emb, const int64_t* ids, int64_t 
   return 0;
 }
 
-template <int MODE, bool TOPK>
+template <int MODE, int EPI>
 static int launch_tile(const TileArgs& a, const TilePlan& pl, cudaStream_t st) {
-  auto kern = fullsort_tile_kernel<MODE, TOPK>;
+  auto kern = fullsort_tile_kernel<MODE, EPI>;
   KGE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
   // blockIdx.x is limited to 2^31-1 rows/BU: fine for any table that fits the device
   dim3 grid((unsigned)pl.n_blocks, (unsigned)pl.n_splits);
@@ -722,7 +972,7 @@ extern "C" int kge_full_sort_scores(const kge_model_t* model, const int64_t* hea
   if (n == 0) return 0;
   KGE_REQUIRE(heads && out, KGE_E_ARG, "NULL heads / out");
   TilePlan pl = {};
-  if (int e = plan_tiles(model, n, n_targets, 0, false, pl)) return e;
+  if (int e = plan_tiles(model, n, n_targets, 0, EPI_DENSE, pl)) return e;
   TileArgs a = {};
   a.s.m = *model;
   a.s.heads = heads;
@@ -737,10 +987,10 @@ extern "C" int kge_full_sort_scores(const kge_model_t* model, const int64_t* hea
   a.out = out;
   a.n_splits = 1;
   switch (tile_mode(model->model)) {
-    case MODE_DIST: return launch_tile<MODE_DIST, false>(a, pl, (cudaStream_t)stream);
-    case MODE_TORUS: return launch_tile<MODE_TORUS, false>(a, pl, (cudaStream_t)stream);
-    case MODE_PROJ: return launch_tile<MODE_PROJ, false>(a, pl, (cudaStream_t)stream);
-    default: return launch_tile<MODE_DOT, false>(a, pl, (cudaStream_t)stream);
+    case MODE_DIST: return launch_tile<MODE_DIST, EPI_DENSE>(a, pl, (cudaStream_t)stream);
+    case MODE_TORUS: return launch_tile<MODE_TORUS, EPI_DENSE>(a, pl, (cudaStream_t)stream);
+    case MODE_PROJ: return launch_tile<MODE_PROJ, EPI_DENSE>(a, pl, (cudaStream_t)stream);
+    default: return launch_tile<MODE_DOT, EPI_DENSE>(a, pl, (cudaStream_t)stream);
   }
 }
 
@@ -748,7 +998,7 @@ extern "C" int64_t kge_full_sort_topk_workspace_bytes(const kge_model_t* model, 
                                                       int32_t k) {
   if (!model || n < 0 || n_targets < 1 || k < 1 || k > KMAX) return -1;
   TilePlan pl = {};
-  if (plan_tiles(model, n > 0 ? n : 1, n_targets, k, true, pl)) return -1;
+  if (plan_tiles(model, n > 0 ? n : 1, n_targets, k, EPI_TOPK, pl)) return -1;
   return (int64_t)n * pl.n_splits * k * 8;
 }
 
@@ -767,7 +1017,7 @@ extern "C" int kge_full_sort_topk(const kge_model_t* model, const int64_t* heads
   KGE_REQUIRE(heads && ids_out, KGE_E_ARG, "NULL heads / ids_out");
   KGE_REQUIRE((hist_off == nullptr) == (hist_items == nullptr) || hist_off, KGE_E_ARG, "hist_items without hist_off");
   TilePlan pl = {};
-  if (int e = plan_tiles(model, n, n_targets, k, true, pl)) return e;
+  if (int e = plan_tiles(model, n, n_targets, k, EPI_TOPK, pl)) return e;
   const int64_t need = n * pl.n_splits * k * 8;
   KGE_REQUIRE(workspace && workspace_bytes >= need, KGE_E_ARG, "workspace too small: need %lld bytes", (long long)need);
   TileArgs a = {};
@@ -789,10 +1039,10 @@ extern "C" int kge_full_sort_topk(const kge_model_t* model, const int64_t* heads
   a.n_splits = pl.n_splits;
   cudaStream_t st = (cudaStream_t)stream;
   const int mode = tile_mode(model->model);
-  if (int e = mode == MODE_DIST ? launch_tile<MODE_DIST, true>(a, pl, st)
-                                : (mode == MODE_TORUS ? launch_tile<MODE_TORUS, true>(a, pl, st)
-                                   : (mode == MODE_PROJ ? launch_tile<MODE_PROJ, true>(a, pl, st)
-                                                        : launch_tile<MODE_DOT, true>(a, pl, st))))
+  if (int e = mode == MODE_DIST ? launch_tile<MODE_DIST, EPI_TOPK>(a, pl, st)
+                                : (mode == MODE_TORUS ? launch_tile<MODE_TORUS, EPI_TOPK>(a, pl, st)
+                                   : (mode == MODE_PROJ ? launch_tile<MODE_PROJ, EPI_TOPK>(a, pl, st)
+                                                        : launch_tile<MODE_DOT, EPI_TOPK>(a, pl, st))))
     return e;
   const int warps = 8;
   const int64_t mg = (n + warps - 1) / warps;
@@ -800,6 +1050,103 @@ extern "C" int kge_full_sort_topk(const kge_model_t* model, const int64_t* heads
                                                                             scores_out, nullptr, nullptr, 0, 0);
   KGE_LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int64_t kge_full_sort_rank_workspace_bytes(const kge_model_t* model, int64_t n, int64_t n_targets,
+                                                      int64_t n_pos) {
+  if (!model || n < 0 || n_targets < 1 || n_pos < 0) return -1;
+  TilePlan pl = {};
+  if (plan_tiles(model, n > 0 ? n : 1, n_targets, 0, EPI_RANK, pl)) return -1;
+  return (int64_t)rank_layout(n, n_pos).total;
+}
+
+template <int MODE>
+static int launch_rank(const RankPrep& rp, const TileArgs& a, const TilePlan& pl, int64_t* greater_out,
+                       int64_t* equal_out, int64_t* n_unmasked_out, cudaStream_t st) {
+  const int parts = (rp.s.m.model == KGE_ROTATE || rp.s.m.model == KGE_COMPLEX) ? 2 : 1;
+  const size_t smem = ((size_t)rp.kpad + (size_t)(TILE_THREADS / 32) * parts * rp.s.m.d) * 4;
+  KGE_CUDA(cudaFuncSetAttribute(rank_thresholds_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const int64_t rows_per_cta = TILE_THREADS / 32;
+  int64_t g = (rp.s.n + rows_per_cta - 1) / rows_per_cta;
+  const int64_t cap = (int64_t)kge_num_sms() * 8;
+  rank_thresholds_kernel<MODE><<<(unsigned)(g < cap ? g : cap), TILE_THREADS, smem, st>>>(rp);
+  KGE_LAUNCH_CHECK();
+  if (int e = launch_tile<MODE, EPI_RANK>(a, pl, st)) return e;
+  rank_finalize_kernel<<<(unsigned)(g < cap ? g : cap), 256, 0, st>>>(rp.s.n, rp.n_targets, rp.cap, rp.pos_off,
+                                                                     rp.score, rp.first, a.rank_bins, a.rank_ninf,
+                                                                     greater_out, equal_out, n_unmasked_out);
+  KGE_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int kge_full_sort_rank_counts(const kge_model_t* model, const int64_t* heads, const int64_t* rels, int64_t n,
+                                         int head_is_user, int64_t n_targets, const int64_t* hist_off,
+                                         const int64_t* hist_items, int mask_first, const int64_t* pos_off,
+                                         const int64_t* pos_items, int64_t* greater_out, int64_t* equal_out,
+                                         int64_t* n_unmasked_out, void* workspace, int64_t workspace_bytes,
+                                         kge_stream_t stream) {
+  if (int e = check_score_model(model)) return e;
+  KGE_REQUIRE(model->model != KGE_TRANSH || rels == nullptr, KGE_E_UNSUPPORTED,
+              "TransH full-sort takes the user->item relation only (transh.py:125-145; no KG scoring in the reference)");
+  KGE_REQUIRE(n >= 0 && n_targets >= 1 && n_targets <= model->entity.rows, KGE_E_ARG, "bad n / n_targets");
+  if (n == 0) return 0;
+  KGE_REQUIRE(heads && pos_off && n_unmasked_out, KGE_E_ARG, "NULL heads / pos_off / n_unmasked_out");
+  KGE_REQUIRE((hist_off == nullptr) == (hist_items == nullptr) || hist_off, KGE_E_ARG, "hist_items without hist_off");
+  TilePlan pl = {};
+  if (int e = plan_tiles(model, n, n_targets, 0, EPI_RANK, pl)) return e;
+  const RankLayout l0 = rank_layout(n, 0);
+  KGE_REQUIRE(workspace && workspace_bytes >= (int64_t)l0.total, KGE_E_ARG, "workspace too small: need %lld bytes",
+              (long long)l0.total);
+  // the number of positives lives on the device: the workspace size says how many it holds (the kernels check it)
+  int64_t cap = (workspace_bytes - (int64_t)l0.total) / 32;
+  while (cap > 0 && (int64_t)rank_layout(n, cap).total > workspace_bytes) --cap;
+  const RankLayout l = rank_layout(n, cap);
+  unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
+  cudaStream_t st = (cudaStream_t)stream;
+  KGE_CUDA(cudaMemsetAsync(ws + l.ninf, 0, (size_t)n * 8, st));
+  KGE_CUDA(cudaMemsetAsync(ws + l.bins, 0, (size_t)cap * 16, st));
+  KGE_CUDA(cudaMemsetAsync(n_unmasked_out, 0, (size_t)n * 8, st));
+  RankPrep rp = {};
+  rp.s.m = *model;
+  rp.s.heads = heads;
+  rp.s.rels = rels;
+  rp.s.n = n;
+  rp.s.head_is_user = head_is_user;
+  rp.s.rel_row = model->ui_relation_fullsort;
+  rp.n_targets = n_targets;
+  rp.kpad = pl.kpad;
+  rp.hist_off = hist_off;
+  rp.hist_items = hist_items;
+  rp.mask_first = mask_first;
+  rp.pos_off = pos_off;
+  rp.pos_items = pos_items;
+  rp.cap = cap;
+  rp.score = reinterpret_cast<float*>(ws + l.score);
+  rp.sorted = reinterpret_cast<float*>(ws + l.sorted);
+  rp.first = reinterpret_cast<int64_t*>(ws + l.first);
+  rp.lo = reinterpret_cast<float*>(ws + l.lo);
+  TileArgs a = {};
+  a.s = rp.s;
+  a.n_targets = n_targets;
+  a.kpad = pl.kpad;
+  a.tiles_per_split = pl.tiles_per_split;
+  a.hist_off = hist_off;
+  a.hist_items = hist_items;
+  a.mask_first = mask_first;
+  a.n_splits = pl.n_splits;
+  a.pos_off = pos_off;
+  a.rank_thr = rp.sorted;
+  a.rank_lo = rp.lo;
+  a.rank_bins = reinterpret_cast<uint64_t*>(ws + l.bins);
+  a.rank_unmasked = reinterpret_cast<uint64_t*>(n_unmasked_out);
+  a.rank_ninf = reinterpret_cast<uint64_t*>(ws + l.ninf);
+  a.rank_cap = cap;
+  switch (tile_mode(model->model)) {
+    case MODE_DIST: return launch_rank<MODE_DIST>(rp, a, pl, greater_out, equal_out, n_unmasked_out, st);
+    case MODE_TORUS: return launch_rank<MODE_TORUS>(rp, a, pl, greater_out, equal_out, n_unmasked_out, st);
+    case MODE_PROJ: return launch_rank<MODE_PROJ>(rp, a, pl, greater_out, equal_out, n_unmasked_out, st);
+    default: return launch_rank<MODE_DOT>(rp, a, pl, greater_out, equal_out, n_unmasked_out, st);
+  }
 }
 
 // ---- device-gated exact top-k for a row list that only exists on the device ------------------------------
@@ -817,7 +1164,7 @@ struct FallbackPlan {
   int64_t keys_a, keys_b;   // part_keys elements of the two regions
 };
 int plan_fallback(const kge_model_t* m, int64_t n, int64_t n_targets, int k, FallbackPlan& fp) {
-  if (int e = plan_tiles(m, n > 0 ? n : 1, n_targets, k, true, fp.tp)) return e;
+  if (int e = plan_tiles(m, n > 0 ? n : 1, n_targets, k, EPI_TOPK, fp.tp)) return e;
   const int64_t n_tiles = (n_targets + BT - 1) / BT;
   int64_t s = FB_SPLITS;
   if (s > (n_tiles + 7) / 8) s = (n_tiles + 7) / 8;
@@ -860,10 +1207,10 @@ int kge_topk_rows_indirect(const kge_model_t* model, const int64_t* heads, const
   a.row_map = row_map;
   a.row_count = row_count;
   const int mode = tile_mode(model->model);
-  auto kern = mode == MODE_DIST ? fullsort_tile_kernel<MODE_DIST, true>
-                                : (mode == MODE_TORUS ? fullsort_tile_kernel<MODE_TORUS, true>
-                                   : (mode == MODE_PROJ ? fullsort_tile_kernel<MODE_PROJ, true>
-                                                        : fullsort_tile_kernel<MODE_DOT, true>));
+  auto kern = mode == MODE_DIST ? fullsort_tile_kernel<MODE_DIST, EPI_TOPK>
+                                : (mode == MODE_TORUS ? fullsort_tile_kernel<MODE_TORUS, EPI_TOPK>
+                                   : (mode == MODE_PROJ ? fullsort_tile_kernel<MODE_PROJ, EPI_TOPK>
+                                                        : fullsort_tile_kernel<MODE_DOT, EPI_TOPK>));
   KGE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fp.tp.smem));
   const int warps = 8;
   const int64_t ra = n < FB_SPLIT_ROWS ? n : FB_SPLIT_ROWS;

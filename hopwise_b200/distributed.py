@@ -393,3 +393,11 @@ def reduce_metric_sums(sums: torch.Tensor, n_users: int, group=None):
                                                                        device=sums.device)])
     dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
     return buf[:-1].reshape(sums.shape), int(round(buf[-1].item()))
+
+
+def reduce_gauc_sums(sums: torch.Tensor, group=None) -> torch.Tensor:
+    """Global GAUC sums (evaluator.gauc_sums of this rank's users) with one all-reduce: every rank then holds
+    (sum of auc_u * pos_len, sum of pos_len) over all users, and GAUC = sums[0] / sums[1] exactly as on one GPU."""
+    buf = sums.reshape(-1).to(torch.float64).clone()
+    dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+    return buf

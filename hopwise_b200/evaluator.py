@@ -6,10 +6,13 @@ Host-side mirror of (paths under /root/reference/hopwise/):
   evaluator/collector.py:234-249  get_data_struct
   evaluator/base_metric.py:75-99  used_info / topk_result (mean over users, value at k-1, rounding)
   evaluator/metrics.py:44-232     Hit, MRR, Recall, NDCG, Precision
+  evaluator/collector.py          the "rec.meanrank" branch and _average_rank
+  evaluator/metrics.py            GAUC.metric_info
   evaluator/evaluator.py:27-41    Evaluator.evaluate -> OrderedDict
 
 The dense [n_users, n_items] score matrix of the reference never exists here: the kernel keeps
-the per-user top-k on chip.  Tie order is (score desc, item id asc).
+the per-user top-k on chip, and GAUC's ranks are counted during the same kind of sweep
+(kge_full_sort_rank_counts).  Tie order is (score desc, item id asc).
 """
 
 from __future__ import annotations
@@ -81,18 +84,44 @@ def metrics_from_sums(sums: torch.Tensor, n_users: int, topk, metrics=("recall",
     return out
 
 
+def gauc_sums(meanrank: torch.Tensor) -> torch.Tensor:
+    """float64 [2] = (sum of auc_u * pos_len, sum of pos_len) over the users GAUC keeps, from rec.meanrank rows
+    (pos_rank_sum, user_len, pos_len) (GAUC.metric_info): users without positives or without negatives are dropped,
+    auc_u = ((user_len + 1) pos_len - pos_len (pos_len + 1) / 2 - pos_rank_sum) / (neg_len pos_len).  Sums of
+    user blocks or ranks add up; GAUC = sums[0] / sums[1]."""
+    rank_sum, user_len, pos_len = meanrank.to(torch.float64).unbind(1)
+    neg_len = user_len - pos_len
+    keep = (pos_len != 0) & (neg_len != 0)
+    pair_num = (user_len + 1) * pos_len - pos_len * (pos_len + 1) / 2 - rank_sum
+    weighted = torch.where(keep, pair_num / torch.where(keep, neg_len * pos_len, 1.0), 0.0) * pos_len
+    return torch.stack([weighted.sum(), torch.where(keep, pos_len, 0.0).sum()])
+
+
+def gauc_from_sums(sums: torch.Tensor, decimals: int | None = 4) -> float:
+    """GAUC = sum(auc_u * pos_len) / sum(pos_len), rounded like GAUC.calculate_metric."""
+    host = sums.cpu()
+    v = float(host[0] / host[1])
+    return round(v, decimals) if decimals is not None else v
+
+
 class FusedCollector:
     """Collector twin fed by the fused top-k instead of dense scores.
 
     ``eval_batch_collect(model, user_ids, history_index, positive_u, positive_i)`` takes the same
     per-batch tuple the reference loader yields; ``get_data_struct()`` returns
-    ``{"rec.topk": int32 [n_users, max(topk)+1], "rec.items": ids, "topk": topk}``.
+    ``{"rec.topk": int32 [n_users, max(topk)+1], "rec.items": ids, "topk": topk}``, plus
+    ``"rec.meanrank"`` (float32 [n_users, 3], full_sort_meanrank) when the config's metrics include GAUC.
     """
 
     def __init__(self, config):
         self.topk = list(config["topk"])
         self.kmax = max(self.topk)
-        self._topk, self._items = [], []
+        try:
+            metrics = config["metrics"]
+        except (KeyError, TypeError):
+            metrics = None
+        self.meanrank = any(str(x).lower() == "gauc" for x in (metrics or ()))
+        self._topk, self._items, self._meanrank = [], [], []
 
     def eval_batch_collect(self, model, user_ids, history_index, positive_u, positive_i):
         device = next(model.parameters()).device
@@ -105,24 +134,31 @@ class FusedCollector:
         pos_off, pos_items = csr_from_pairs(positive_u, positive_i, n, device)
         self._topk.append(topk_hits(ids, pos_off, pos_items))
         self._items.append(ids)
+        if self.meanrank:
+            self._meanrank.append(model.full_sort_meanrank(users, pos_off, pos_items, hist_off, hist_items, mask_pad=True))
         return ids
 
     def get_data_struct(self):
         rec = torch.cat(self._topk) if self._topk else torch.zeros(0, self.kmax + 1, dtype=torch.int32)
         items = torch.cat(self._items) if self._items else torch.zeros(0, self.kmax, dtype=torch.int64)
-        self._topk, self._items = [], []
-        return {"rec.topk": rec, "rec.items": items, "topk": self.topk}
+        struct = {"rec.topk": rec, "rec.items": items, "topk": self.topk}
+        if self.meanrank:
+            struct["rec.meanrank"] = torch.cat(self._meanrank) if self._meanrank else torch.zeros(0, 3)
+        self._topk, self._items, self._meanrank = [], [], []
+        return struct
 
 
 def evaluate_full_sort(model, user_ids, hist_off, hist_items, pos_off, pos_items, topk=(10,), decimals=4,
-                       user_block: int | None = None, return_struct: bool = False):
-    """Whole-split evaluation with device-resident CSR inputs; returns the metric dictionary."""
+                       user_block: int | None = None, return_struct: bool = False, gauc: bool = False):
+    """Whole-split evaluation with device-resident CSR inputs; returns the metric dictionary (with ``gauc=True``
+    it also holds ``"gauc"``, from full_sort_meanrank)."""
     device = next(model.parameters()).device
     users = torch.as_tensor(user_ids).to(device)
     n = users.numel()
     kmax = max(topk)
     block = user_block or n
     sums = torch.zeros(5, kmax, dtype=torch.float64, device=device)
+    g_sums = torch.zeros(2, dtype=torch.float64, device=device)
     recs = []
     for s in range(0, n, block):
         e = min(n, s + block)
@@ -137,9 +173,13 @@ def evaluate_full_sort(model, user_ids, hist_off, hist_items, pos_off, pos_items
         pi = pos_items[int(pbase.item()) : int(pos_off[e].item())] if block < n else pos_items
         rec = topk_hits(ids, po, pi)
         sums += topk_metric_sums(rec)
+        if gauc:
+            g_sums += gauc_sums(model.full_sort_meanrank(users[s:e], po, pi, ho, hi, mask_pad=True))
         if return_struct:
             recs.append(rec)
     result = metrics_from_sums(sums, n, topk, decimals=decimals)
+    if gauc:
+        result["gauc"] = gauc_from_sums(g_sums, decimals)
     if return_struct:
         return result, torch.cat(recs)
     return result

@@ -878,6 +878,79 @@ class FusedKGEModel(KnowledgeRecommender):
             return ids, scores, dbg
         return ids, scores
 
+    # ------------------------------------------------------------------ fused full-sort ranks of listed targets
+    def full_sort_rank(self, query_ids, pos_off, pos_items, hist_off=None, hist_items=None, mask_pad: bool = True,
+                       relation_ids=None):
+        """Exact full-catalogue ranks of listed targets, without the score matrix (kge_full_sort_rank_counts).
+
+        The rows and the masking are full_sort_topk's (``relation_ids``: link prediction over all entities).
+        ``pos_off`` [n+1] / ``pos_items`` (sorted ascending per row) is the CSR of the targets to rank, e.g. the
+        positives.  Returns int64 ``(greater, equal, n_unmasked)``: for every entry of ``pos_items``, how many targets
+        of its row's masked scores score strictly above it and exactly equal to it (itself included), and per row
+        the number of unmasked targets.  The entry's average rank (collector.py ``_average_rank``) is
+        ``greater + (equal + 1) / 2``."""
+        device = self._check_ready()
+        self.flush()
+        users = self._ids(query_ids, device)
+        n = users.numel()
+        rels = None if relation_ids is None else self._ids(relation_ids, device)
+        if rels is not None and rels.numel() != n:
+            raise ValueError("relation_ids must have one entry per head")
+        n_targets = self.n_items if rels is None else self.n_entities
+        if hist_off is not None:
+            hist_off, hist_items = self._ids(hist_off, device), self._ids(hist_items, device)
+            if hist_off.numel() != n + 1:
+                raise ValueError("hist_off must have n_users + 1 entries")
+        pos_off, pos_items = self._ids(pos_off, device), self._ids(pos_items, device)
+        if pos_off.numel() != n + 1:
+            raise ValueError("pos_off must have n_users + 1 entries")
+        n_pos = pos_items.numel()
+        greater = torch.empty(n_pos, dtype=torch.int64, device=device)
+        equal = torch.empty(n_pos, dtype=torch.int64, device=device)
+        n_unmasked = torch.empty(n, dtype=torch.int64, device=device)
+        m = self._model_struct(False)
+        lib = _abi.lib()
+        need = lib.kge_full_sort_rank_workspace_bytes(C.byref(m), n, n_targets, n_pos)
+        if need < 0:
+            raise _abi.KgeError(f"kge_full_sort_rank_counts: unsupported shape (d={self.embedding_size})")
+        ws = torch.empty(max(need, 16), dtype=torch.uint8, device=device)
+        _abi.check(
+            lib.kge_full_sort_rank_counts(
+                C.byref(m), users.data_ptr(), _abi.ptr(rels), n, 1 if rels is None else 0, n_targets,
+                _abi.ptr(hist_off), _abi.ptr(hist_items), 1 if mask_pad else 0, pos_off.data_ptr(),
+                pos_items.data_ptr(), greater.data_ptr(), equal.data_ptr(), n_unmasked.data_ptr(), ws.data_ptr(),
+                ws.numel(), _abi.stream_ptr(),
+            ),
+            "kge_full_sort_rank_counts",
+        )
+        return greater, equal, n_unmasked
+
+    def full_sort_meanrank(self, query_ids, pos_off, pos_items, hist_off=None, hist_items=None, mask_pad: bool = True,
+                           relation_ids=None):
+        """float32 [n, 3] rows ``(pos_rank_sum, user_len, pos_len)``: the collector's ``rec.meanrank``
+        (collector.py, the ``rec.meanrank`` branch and ``_average_rank``) that GAUC reads, from full_sort_rank.
+
+        Duplicate ids of a row count once, as the reference's ``pos_matrix[u, i] = 1`` does.  The average ranks are
+        summed in float64 and rounded once.  ``user_len`` is the reference's ``argmin`` of the sorted row, which is
+        the number of unmasked targets only when the row has a masked one: ``mask_pad=True`` (what the trainer
+        does) guarantees it, so ``mask_pad=False`` without a history is refused."""
+        if not mask_pad and hist_off is None:
+            raise ValueError("full_sort_meanrank needs a masked target in every row (mask_pad=True or a history): "
+                             "user_len is the argmin of the sorted row")
+        greater, equal, n_unmasked = self.full_sort_rank(query_ids, pos_off, pos_items, hist_off, hist_items, mask_pad,
+                                                         relation_ids)
+        device = greater.device
+        pos_off, pos_items = self._ids(pos_off, device), self._ids(pos_items, device)
+        n, n_pos = n_unmasked.numel(), pos_items.numel()
+        row = torch.repeat_interleave(torch.arange(n, device=device), pos_off.diff(), output_size=n_pos)
+        first = torch.ones(n_pos, dtype=torch.bool, device=device)
+        first[1:] = (pos_items[1:] != pos_items[:-1]) | (row[1:] != row[:-1])
+        avg_rank = greater.double() + (equal.double() + 1.0) * 0.5
+        once = first.double()   # (weights rather than a boolean selection: no host synchronisation)
+        rank_sum = torch.zeros(n, dtype=torch.float64, device=device).index_add_(0, row, avg_rank * once)
+        pos_len = torch.zeros(n, dtype=torch.float64, device=device).index_add_(0, row, once)
+        return torch.stack([rank_sum, n_unmasked.double(), pos_len], dim=1).float()
+
     def forward(self, *args, **kwargs):  # the reference's forward is the scorer on gathered rows
         raise NotImplementedError("use calculate_loss / predict / full_sort_predict")
 
@@ -1013,6 +1086,15 @@ class TransH(FusedKGEModel):
         view, idx = self._rec_view(user_ids)
         return view.full_sort_topk(idx, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores)
 
+    def full_sort_rank(self, query_ids, pos_off, pos_items, hist_off=None, hist_items=None, mask_pad=True,
+                       relation_ids=None):
+        if relation_ids is not None:
+            raise NotImplementedError("the reference TransH has no KG scoring entry points (transh.py)")
+        if self.n_items < self.VIEW_MIN_ITEMS:
+            return super().full_sort_rank(query_ids, pos_off, pos_items, hist_off, hist_items, mask_pad)
+        view, idx = self._rec_view(query_ids)
+        return view.full_sort_rank(idx, pos_off, pos_items, hist_off, hist_items, mask_pad)
+
 
 class TransD(FusedKGEModel):
     """transd.py: every table has an embedding and a transfer vector; ``forward(ent, ent_vec, rel_vec) = rel_vec *
@@ -1104,6 +1186,13 @@ class TransD(FusedKGEModel):
             raise NotImplementedError("TransD scores users against items only (see full_sort_predict_kg)")
         view, idx = self._rec_view(user_ids)
         return view.full_sort_topk(idx, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores)
+
+    def full_sort_rank(self, query_ids, pos_off, pos_items, hist_off=None, hist_items=None, mask_pad=True,
+                       relation_ids=None):
+        if relation_ids is not None:
+            raise NotImplementedError("TransD scores users against items only (see full_sort_predict_kg)")
+        view, idx = self._rec_view(query_ids)
+        return view.full_sort_rank(idx, pos_off, pos_items, hist_off, hist_items, mask_pad)
 
 
 MODELS = {"TransE": TransE, "DistMult": DistMult, "RotatE": RotatE, "ComplEx": ComplEx, "TorusE": TorusE,

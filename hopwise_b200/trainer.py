@@ -26,10 +26,12 @@ checkpoints, early stopping, logging are inherited unchanged) and overrides only
                             summed on the device in float64 (the reference adds the same fp32 values in Python
                             doubles: identical result, one host sync per epoch instead of one per step);
   * ``evaluate_data_loop``  fused full-sort top-k over large user blocks straight from the loader's own per-user
-                            history / positives (built once per loader), the ``rec.topk`` rows handed to the
-                            reference ``Evaluator`` unchanged -- so the metric dictionary is the reference's own.
-                            Anything the fused kernels do not cover (sampled evaluation, sequential loaders, metrics
-                            that need full score rows, k > 128) goes through the inherited dense path.
+                            history / positives (built once per loader), the ``rec.topk`` rows -- and for GAUC the
+                            ``rec.meanrank`` rows, from the exact full-catalogue ranks of the positives -- handed to
+                            the reference ``Evaluator`` unchanged, so the metric dictionary is the reference's own.
+                            Anything the fused kernels do not cover (sampled evaluation, sequential loaders, the
+                            labelled value metrics that read ``rec.score`` / ``data.label``, k > 128) goes through
+                            the inherited dense path.
 
 ``install()`` registers the classes with hopwise's own factories, so ``run_hopwise(model="TransE", ...)`` and the
 ``hopwise train`` CLI pick them up without edits: ``get_model`` (utils/utils.py:65-98) resolves
@@ -162,8 +164,8 @@ class FusedKGTrainer(KGTrainer):
             return None
         collector = self.eval_collector if task == KnowledgeEvaluationType.REC else self.eval_collector_kg
         reg = collector.register
-        if any(reg.need(key) for key in ("rec.meanrank", "rec.score", "data.label")):
-            return None   # these need the dense score rows
+        if any(reg.need(key) for key in ("rec.score", "data.label")):
+            return None   # the labelled value metrics need the dense score rows
         if max(collector.topk) > KMAX_FUSED or torch.device(self.device).type != "cuda":
             return None
         plan = eval_data.__dict__.get("_kge_fused_plan")
@@ -221,6 +223,10 @@ class FusedKGTrainer(KGTrainer):
                 struct.update_tensor("rec.items", ids)
             if reg.need("rec.topk"):
                 struct.update_tensor("rec.topk", topk_hits(ids, po, pval[p0:p1]))
+            if reg.need("rec.meanrank"):
+                # collector.py's rec.meanrank branch without sorting the [users, n_items] score rows
+                struct.update_tensor("rec.meanrank", self.model.full_sort_meanrank(
+                    users, po, pval[p0:p1], ho, hval[h0:h1], mask_pad=True, relation_ids=rels))
         collector.model_collect(self.model)
         result = evaluator.evaluate(collector.get_data_struct())
         if not self.config["single_spec"]:

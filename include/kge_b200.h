@@ -255,6 +255,26 @@ int kge_full_sort_topk(const kge_model_t* model, const int64_t* heads, const int
                        int mask_first, int32_t k, int64_t* ids_out, float* scores_out, void* workspace,
                        int64_t workspace_bytes, kge_stream_t stream);
 
+/* kge_full_sort_rank_counts: the exact rank of listed targets over the whole masked row, without
+ * materialising [n, n_targets] -- what the collector's rec.meanrank branch (collector.py, the sort
+ * of every score row and _average_rank) and metrics.py's GAUC read.  Same query and masking
+ * arguments as kge_full_sort_topk (rels == NULL: the user->item relation; masked targets score
+ * -inf).  The listed targets are CSR over the rows: pos_off[n+1], pos_items sorted ascending per
+ * row (duplicates allowed: each copy gets the same counts).  For every entry i of pos_items, over
+ * the row's masked scores s and the entry's own masked score s_i:
+ *   greater_out[i] = #{targets with s > s_i},  equal_out[i] = #{targets with s == s_i}
+ * (the target itself included), so its average rank is greater + (equal + 1) / 2;
+ * n_unmasked_out[n] = the row's unmasked targets.  Ids outside [0, n_targets) are counted as
+ * masked.  Scores are bit-identical to kge_full_sort_scores / kge_full_sort_topk, counts are exact
+ * integers.  workspace: device scratch of kge_full_sort_rank_workspace_bytes(model, n, n_targets,
+ * n_pos) bytes with n_pos = pos_off[n]; a smaller one sets every n_unmasked_out to -1. */
+int64_t kge_full_sort_rank_workspace_bytes(const kge_model_t* model, int64_t n, int64_t n_targets, int64_t n_pos);
+int kge_full_sort_rank_counts(const kge_model_t* model, const int64_t* heads, const int64_t* rels, int64_t n,
+                              int head_is_user, int64_t n_targets, const int64_t* hist_off, const int64_t* hist_items,
+                              int mask_first, const int64_t* pos_off, const int64_t* pos_items,
+                              int64_t* greater_out, int64_t* equal_out, int64_t* n_unmasked_out,
+                              void* workspace, int64_t workspace_bytes, kge_stream_t stream);
+
 /* ---- tensor-core full-sort top-k (tcgen05) -------------------------------------------------------
  * Same contract and same results as kge_full_sort_topk (ids and scores are bit-identical: the
  * fp16 tensor-core pass only filters, under a proven error bound; every reported score comes from
