@@ -19,7 +19,8 @@
 // memory latency per triple; further negatives are prefetched one ahead).  Gradients leave as
 // RED.ADD.F32x4; a touched row is marked by a plain store of the step number.  The user->item
 // relation row is shared by every rec triple, so its gradient is accumulated in registers,
-// reduced per CTA in shared memory and flushed once per CTA.
+// reduced per CTA in shared memory and flushed once per CTA.  With two triples per warp, the KG
+// relation rows go the same way, through per-warp copies in shared memory (WARP_RACC).
 // Kernel B (adam_apply_kernel): lanes scan row_state (8 B per row, coalesced), ballot the rows
 // marked in this step and a lane group updates each: replay the zero-gradient steps the row
 // skipped (dense Adam keeps moving a row after its last gradient), apply the real step, zero g.
@@ -159,12 +160,25 @@ struct FwdBounds {
 #endif
 };
 
-template <int MODEL, int VEC, int G, int NCH>
+// Shared memory of the WARP_RACC path: every warp's private [R][PR][d] relation-gradient copy, then one flag per
+// relation row that this CTA gave a gradient.
+constexpr int kFwdWarps = 8;   // train_fwd_kernel runs 256 threads per CTA
+inline size_t warp_racc_smem_bytes(int64_t rows, int parts, int d) {
+  return (size_t)kFwdWarps * rows * parts * d * sizeof(float) + (size_t)rows * sizeof(int);
+}
+
+// WARP_RACC (two triples per warp only, G = 16): relation gradients of both halves are summed in per-warp copies in
+// shared memory with plain loads and stores and leave once per CTA, one float4 RED per 4 columns of each touched
+// row -- instead of one RED per triple onto the few lines of the ~20 KG relation rows, which every L2 slice holding
+// them has to serialise.  (A CTA-wide copy would need float atomics on shared memory: a CAS loop on sm_100a.)
+template <int MODEL, int VEC, int G, int NCH, bool WARP_RACC = false>
 __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) train_fwd_kernel(const TrainArgs a) {
   constexpr int E = VEC * NCH;
   constexpr int PH = (MODEL == KGE_ROTATE || MODEL == KGE_COMPLEX || MODEL == KGE_TRANSD) ? 2 : 1;  // head / tail parts
   constexpr int PR = (MODEL == KGE_COMPLEX || MODEL == KGE_TRANSH || MODEL == KGE_TRANSD) ? 2 : 1;   // relation parts
-  extern __shared__ float s_racc[];  // [PR][d] user->item relation gradient of this CTA
+  static_assert(!WARP_RACC || (VEC == 4 && G == 16), "per-warp relation copies pair the two half-warp groups");
+  // without WARP_RACC: [PR][d] user->item relation gradient of this CTA; with it: warp_racc_smem_bytes
+  extern __shared__ __align__(16) float s_racc[];
   __shared__ float s_loss[8];
 
   const int d = a.m.d;
@@ -178,8 +192,34 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
   // (small batches: every touched row is also appended to its table's slice of the touch list, kge_model_t)
   const TouchList tl_user = {a.m, 0, a.with_grad}, tl_entity = {a.m, 1, a.with_grad}, tl_relation = {a.m, 2, a.with_grad};
 
-  for (int i = threadIdx.x; i < PR * d; i += blockDim.x) s_racc[i] = 0.f;
+  const int n_rel = (int)RT.rows;
+  const int nv = d >> 2;
+  // WARP_RACC: this warp's copy, as float4 [R][PR][nv]; the touched flags follow the copies of all warps
+  float4* s_wrg = reinterpret_cast<float4*>(s_racc) + (size_t)(threadIdx.x >> 5) * n_rel * PR * nv;
+  int* s_rtouch = reinterpret_cast<int*>(s_racc + (size_t)kFwdWarps * n_rel * PR * d);
+  if constexpr (WARP_RACC) {
+    float4* s4 = reinterpret_cast<float4*>(s_racc);
+    for (int i = threadIdx.x; i < kFwdWarps * n_rel * PR * nv; i += blockDim.x) s4[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int i = threadIdx.x; i < n_rel; i += blockDim.x) s_rtouch[i] = 0;
+  } else {
+    for (int i = threadIdx.x; i < PR * d; i += blockDim.x) s_racc[i] = 0.f;
+  }
   __syncthreads();
+  // (adds a group's relation-gradient fragment into row `row` of its warp's copy)
+  auto warp_copy_add = [&](int row, const float (&x)[PR][E]) {
+#pragma unroll
+    for (int p = 0; p < PR; ++p)
+#pragma unroll
+      for (int j = 0; j < NCH; ++j) {
+        const int c = gl + j * G;
+        if (c < nv) {
+          float4& s = s_wrg[(row * PR + p) * nv + c];
+          float4 v = s;
+          v.x += x[p][4 * j]; v.y += x[p][4 * j + 1]; v.z += x[p][4 * j + 2]; v.w += x[p][4 * j + 3];
+          s = v;
+        }
+      }
+  };
 
   float lsum = 0.f;
   float racc[PR][E];
@@ -652,37 +692,93 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
         for (int p = 0; p < PR; ++p)
 #pragma unroll
           for (int e = 0; e < E; ++e) racc[p][e] += gr[p][e];
-      } else {
+      } else if (!WARP_RACC) {
 #pragma unroll
         for (int p = 0; p < PR; ++p) frag_atomic_add<VEC, G, NCH>(RT.g[p], r_id, d, gl, gr[p]);
         touch_row(RT, r_id, sr.y, step, gl, tl_relation);
+      }
+    }
+
+    if constexpr (WARP_RACC && !is_rec) {
+      // The two groups of the warp run triples i and i + 1 (i even).  Lane l and lane l + 16 hold the same columns:
+      // when both triples name the same relation, group 1 hands its fragment to group 0, which writes alone.
+      const bool pair = (i | 1) < n_seg;   // (group 1 has left the loop when this is false)
+      __syncwarp(pair ? 0xffffffffu : 0x0000ffffu);   // orders the other group's add of the previous iteration
+      bool write = any_grad;
+      if (pair) {
+        const int r_other = __shfl_xor_sync(0xffffffffu, (int)r_id, 16);
+        if (r_other == (int)r_id) {
+          const bool any_other = __shfl_xor_sync(0xffffffffu, any_grad ? 1 : 0, 16) != 0;
+#pragma unroll
+          for (int p = 0; p < PR; ++p)
+#pragma unroll
+            for (int e = 0; e < E; ++e) gr[p][e] += __shfl_xor_sync(0xffffffffu, gr[p][e], 16);
+          write = (threadIdx.x & 16) == 0 && (any_grad || any_other);
+        }
+      }
+      if (write) {
+        warp_copy_add((int)r_id, gr);
+        if (gl == 0) s_rtouch[r_id] = 1;
       }
     }
   }
 
   };
   run_half(std::true_type{});
-  run_half(std::false_type{});
-
-  // ---- CTA epilogue: user->item relation gradient and the loss --------------------------------
-  if (rec_seen) {
+  if constexpr (WARP_RACC) {
+    // the user->item relation gradient of this warp: both groups hold the same columns
 #pragma unroll
-    for (int p = 0; p < PR; ++p) {
+    for (int p = 0; p < PR; ++p)
 #pragma unroll
-      for (int e = 0; e < E; ++e) {
-        const int j = e / VEC;
-        const int col = (gl + j * G) * VEC + (e % VEC);
-        if (col < d) atomicAdd(&s_racc[p * d + col], racc[p][e]);
-      }
+      for (int e = 0; e < E; ++e) racc[p][e] += __shfl_xor_sync(0xffffffffu, racc[p][e], 16);
+    if (__any_sync(0xffffffffu, rec_seen) && (threadIdx.x & 16) == 0) {
+      warp_copy_add(a.m.ui_relation, racc);
+      if (gl == 0) s_rtouch[a.m.ui_relation] = 1;
     }
   }
-  const int any_rec = __syncthreads_or(rec_seen ? 1 : 0);
-  if (any_rec) {
-    for (int i = threadIdx.x; i < PR * d; i += blockDim.x) {
-      const int p = i / d, col = i - p * d;
-      atomicAdd(RT.g[p] + (int64_t)a.m.ui_relation * d + col, s_racc[i]);
+  run_half(std::false_type{});
+
+  // ---- CTA epilogue: relation gradients and the loss --------------------------------------------
+  if constexpr (WARP_RACC) {
+    // sum the warp copies of every row this CTA touched: one float4 RED per 4 columns, one mark per row
+    __syncthreads();
+    const float4* s4 = reinterpret_cast<const float4*>(s_racc);
+    const int row_len = PR * nv;
+    const int warp_stride = n_rel * row_len;
+    for (int k = threadIdx.x; k < warp_stride; k += blockDim.x) {
+      const int row = k / row_len;
+      if (!s_rtouch[row]) continue;
+      const int p = (k - row * row_len) / nv, c = k - row * row_len - p * nv;
+      float4 s = s4[k];
+#pragma unroll
+      for (int w = 1; w < kFwdWarps; ++w) {
+        const float4 v = s4[w * warp_stride + k];
+        s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+      }
+      atomicAdd(reinterpret_cast<float4*>((p == 0 ? RT.g[0] : RT.g[PR - 1]) + (int64_t)row * d) + c, s);
     }
-    if (threadIdx.x == 0) touch_row(RT, a.m.ui_relation, -1, step, 0, tl_relation);
+    for (int row = threadIdx.x; row < n_rel; row += blockDim.x)
+      if (s_rtouch[row]) touch_row(RT, row, -1, step, 0, tl_relation);
+  } else {
+    if (rec_seen) {
+#pragma unroll
+      for (int p = 0; p < PR; ++p) {
+#pragma unroll
+        for (int e = 0; e < E; ++e) {
+          const int j = e / VEC;
+          const int col = (gl + j * G) * VEC + (e % VEC);
+          if (col < d) atomicAdd(&s_racc[p * d + col], racc[p][e]);
+        }
+      }
+    }
+    const int any_rec = __syncthreads_or(rec_seen ? 1 : 0);
+    if (any_rec) {
+      for (int i = threadIdx.x; i < PR * d; i += blockDim.x) {
+        const int p = i / d, col = i - p * d;
+        atomicAdd(RT.g[p] + (int64_t)a.m.ui_relation * d + col, s_racc[i]);
+      }
+      if (threadIdx.x == 0) touch_row(RT, a.m.ui_relation, -1, step, 0, tl_relation);
+    }
   }
   lsum = warp_sum(lsum);
   if ((threadIdx.x & 31) == 0) s_loss[threadIdx.x >> 5] = lsum;
@@ -1066,9 +1162,32 @@ extern "C" int kge_train_forward(const kge_model_t* model, const kge_batch_t* b,
                             n_total >= (int64_t)kge_num_sms() * 256 &&
                             (kind == KGE_TRANSE || kind == KGE_DISTMULT);
   const int threads = 256;
-  const int grid = grid_for(n_total, threads / (two_per_warp ? 16 : c.g), 8);
-  const size_t smem = (size_t)model->relation.parts * model->d * sizeof(float);
+  int grid = grid_for(n_total, threads / (two_per_warp ? 16 : c.g), 8);
+  size_t smem = (size_t)model->relation.parts * model->d * sizeof(float);
   cudaStream_t st = (cudaStream_t)stream;
+  // Two triples per warp with gradients: relation gradients go through per-warp copies in shared memory when those
+  // fit at the residency the kernel's register budget is shaped for.  The grid is then sized to what is resident,
+  // so that every CTA zeroes and flushes its copies once.
+  bool warp_racc = false;
+  if (two_per_warp && with_grad) {
+    const size_t ws = warp_racc_smem_bytes(model->relation.rows, model->relation.parts, model->d);
+    auto kern = kind == KGE_TRANSE ? train_fwd_kernel<KGE_TRANSE, 4, 16, 2, true>
+                                   : train_fwd_kernel<KGE_DISTMULT, 4, 16, 2, true>;
+    const int min_ctas = kind == KGE_TRANSE ? FwdBounds<KGE_TRANSE, 4, 16, 2>::MIN_CTAS
+                                            : FwdBounds<KGE_DISTMULT, 4, 16, 2>::MIN_CTAS;
+    int dev = 0, optin = 0, resident = 0;
+    KGE_CUDA(cudaGetDevice(&dev));
+    KGE_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    if (ws <= (size_t)optin) {
+      KGE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ws));
+      KGE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, threads, ws));
+    }
+    if (resident >= min_ctas) {
+      warp_racc = true;
+      smem = ws;
+      grid = grid_for(n_total, threads / 16, resident);
+    }
+  }
 #define CALL(V, G, N)                                                                                   \
   switch (kind) {                                                                                       \
     case KGE_TRANSE: train_fwd_kernel<KGE_TRANSE, V, G, N><<<grid, threads, smem, st>>>(a); break;      \
@@ -1078,7 +1197,10 @@ extern "C" int kge_train_forward(const kge_model_t* model, const kge_batch_t* b,
     case KGE_TRANSD: train_fwd_kernel<KGE_TRANSD, V, G, N><<<grid, threads, smem, st>>>(a); break;      \
     default: train_fwd_kernel<KGE_COMPLEX, V, G, N><<<grid, threads, smem, st>>>(a); break;             \
   }
-  if (two_per_warp) {
+  if (warp_racc) {
+    if (kind == KGE_TRANSE) train_fwd_kernel<KGE_TRANSE, 4, 16, 2, true><<<grid, threads, smem, st>>>(a);
+    else train_fwd_kernel<KGE_DISTMULT, 4, 16, 2, true><<<grid, threads, smem, st>>>(a);
+  } else if (two_per_warp) {
     if (kind == KGE_TRANSE) train_fwd_kernel<KGE_TRANSE, 4, 16, 2><<<grid, threads, smem, st>>>(a);
     else train_fwd_kernel<KGE_DISTMULT, 4, 16, 2><<<grid, threads, smem, st>>>(a);
   } else {
