@@ -13,7 +13,7 @@ import os
 
 from . import _build
 
-KGE_ABI_VERSION = 6
+KGE_ABI_VERSION = 7
 MODEL_KINDS = {"TransE": 0, "DistMult": 1, "RotatE": 2, "ComplEx": 3, "TorusE": 4, "TransH": 5, "TransD": 6}
 
 
@@ -49,8 +49,6 @@ class kge_model_t(C.Structure):
         ("adam_table", C.c_void_p),
         ("adam_table_len", C.c_int32),
         ("_pad2", C.c_int32),
-        ("touch_list", C.c_void_p),
-        ("touch_count", C.c_void_p),
     ]
 
 

@@ -5,7 +5,7 @@
 // transe.py:112-126, rotate.py:161-190}, trainer/trainer.py:716-735, evaluator/collector.py:176-177)
 // for the scorers that are dense contractions: DistMult / ComplEx directly (score = q . t) and
 // the L2 models through  -||q - t||^2 = 2 (q . t - ||t||^2 / 2) - ||q||^2  (the per-row constant
-// does not change the order; -||t||^2/2 rides in three extra K columns as a bf16 hi/mid/lo split).
+// does not change the order; -||t||^2/2 rides in three extra K columns as an fp16 hi/mid/lo split).
 //
 // The tensor cores only FILTER; the answer is exact:
 //   1. fp16 GEMM  a^_ij ~ S_i (q_i . t_j)  with fp32 accumulation in TMEM.  Operands are scaled by powers of two
@@ -16,13 +16,14 @@
 //      (two roundings per product, the subnormal floor, fp32 accumulation; see row_eps()).  Round 1 used bf16
 //      with 1.02 * 2^-8: too small by 2x (two roundings of 2^-8 each) -- fp16 is 8x tighter than the valid bf16
 //      bound at the same tensor-core rate.
-//   2. sweep epilogue, one thread per query row: maxima of groups of 8 adjacent targets are compared
-//      with a running threshold thr_i = tau_i - 2 eps_i, where tau_i is the k-th largest group
-//      maximum among groups without masked targets seen so far (a lower bound of the k-th largest
-//      unmasked approximate score).  Every member of the exact top-k has a^ >= tau_final - 2 eps,
-//      so its group survives.  Surviving groups are appended to a list of CAND entries per row in
-//      global memory (L2); when a list fills, its warp compacts it (radix select of tau, keep the
-//      entries >= tau - 2 eps); a list that cannot be compacted flags the row.
+//   2. sweep epilogue, one thread per query row: the maximum of each chunk of 32 adjacent targets is compared
+//      with a running threshold thr_i = tau_i - 2 eps_i, where tau_i is the k-th largest chunk maximum
+//      among chunks without masked targets seen so far (a lower bound of the k-th largest unmasked
+//      approximate score).  Every member of the exact top-k has a^ >= tau_final - 2 eps, so its chunk
+//      survives.  A surviving chunk is appended, with the mask of its groups of GRP targets that clear the
+//      threshold, to a list of CAND entries per (row, split, column slice) in global memory (L2); when a list
+//      fills, its warp compacts it (radix select of tau, keep the entries >= tau - 2 eps); a list that cannot
+//      be compacted flags the row.
 //   3. rescore kernel (one warp per row): final tau over the row's lists, then only the targets of
 //      the groups >= tau - 2 eps are scored in fp32 with the same sequential FMA chain as the
 //      CUDA-core kernel (bit-identical scores), masked, pre-filtered by score >= tau - eps (the k
@@ -30,17 +31,15 @@
 //      Flagged rows and rows with fewer than k valid candidates are reported to the caller, which
 //      runs them through kge_full_sort_topk.
 //
-// Sweep kernel shape: CTA = 256 query rows = two M=128 accumulators against target tiles of TN rows
-// (every B tile feeds two MMAs); the accumulators are double-buffered in TMEM (4 x TN columns) and
-// the epilogue releases a buffer as soon as its values sit in registers, so the MMAs of tile i+1
-// run under the epilogue of tile i.  TN = 64 keeps the CTA at 256 TMEM columns and <= 113 KB of
-// shared memory so that two CTAs share an SM: 16 epilogue warps hide the TMEM-load and issue
-// latencies of each other.  Warp 0 streams pre-tiled bf16 target images with cp.async.bulk into a
-// ring of shared-memory stages (mbarrier expect_tx), warp 1 issues tcgen05.mma (one thread), warps
-// 2..9 are the epilogue (warp % 4 = the TMEM lane quadrant a warp may read).  A grid of
-// (row blocks) x (target splits) fills the GPU when few users are evaluated; every (row, split)
-// owns a list.  Operands use the no-swizzle K-major canonical layout [K/8][rows][8 bf16]:
-// 8x16-byte core matrices, SBO = 128 B, LBO = rows * 16 B.
+// Sweep kernel (fullsort_mma_kernel): a CTA keeps NH row halves of 128 query rows in shared memory and sweeps
+// target tiles of TN rows; every B tile feeds one M = 128 MMA per half.  Each half has NBUF accumulators in TMEM:
+// one in shape (a) (256 columns, so that two CTAs share an SM), two in shapes (f), (c) and (k), where the MMAs of
+// tile i+1 run under the epilogue of tile i.  plan_mma picks the shape (DESIGN 3.4(b) item 2).  Warp roles, in warp
+// order (sweep_threads): the epilogue warps, one thread per query row; one producer warp that streams the pre-tiled
+// fp16 target image with cp.async.bulk into a ring of shared-memory stages (mbarrier expect_tx); NMMA issuer warps
+// whose elected lane issues tcgen05.mma.  A grid of (row blocks) x (target splits) fills the GPU when few users are
+// evaluated; every (row, split, column slice) owns a list.  Operands use the no-swizzle K-major canonical layout
+// [K/8][rows][8 fp16]: 8x16-byte core matrices, SBO = 128 B, LBO = rows * 16 B.
 #include <cuda_fp16.h>
 #include <math.h>
 
@@ -51,23 +50,16 @@ namespace {
 
 constexpr int MH = 128;    // query rows per row half (one M = 128 accumulator); a CTA sweeps NH = 1 or 2 halves
 constexpr int GRP = 4;     // targets per candidate group (what the rescore kernel reads per mask bit)
-#ifndef KGE_MMA_CAND
-#define KGE_MMA_CAND 128
-#endif
-constexpr int CAND = KGE_MMA_CAND;  // candidate chunks kept per (row, split)
+constexpr int CAND = 128;  // candidate chunks kept per (row, split)
 constexpr int MAX_SPLITS = 4;
-// Warp roles of the sweep: 8 * NCOL epilogue warps (warp % 4 = TMEM lane quadrant, (warp / 4) % 2 = row half,
-// warp / 8 = column slice of the tile), then the producer warp, then one MMA issuer warp per row half (the issue
-// arbiter favours high warp ids, and an MMA issuer must never starve; one warp cannot issue fast enough for both
-// halves: a free-running issuer needs ~125 cycles per tcgen05.mma).
-// Warps of a sweep CTA: 4 * NH * NCOL epilogue warps, one producer warp, NMMA issuer warps.
+// Warps of a sweep CTA, in this order: 4 * NH * NCOL epilogue warps (warp % 4 = TMEM lane quadrant, (warp / 4) % NH =
+// row half, warp / (4 * NH) = column slice of the tile), one producer warp, NMMA issuer warps.  The issuers come last:
+// the issue arbiter favours high warp ids, and an MMA issuer must never starve.  (A CTA that has the SM to itself
+// takes one issuer per row half: a free-running issuer needs ~125 cycles per tcgen05.mma.)
 constexpr int PRODUCER_WARPS = 1;
 __host__ __device__ constexpr int sweep_threads(int nh, int ncol, int nmma) {
   return (4 * nh * ncol + PRODUCER_WARPS + nmma) * 32;
 }
-#ifndef KGE_MMA_A_NMMA
-#define KGE_MMA_A_NMMA 1   // MMA issuer warps of shape (a): 1 = one warp for both halves, 2 = one per half (experiment)
-#endif
 constexpr int IMG_HEADER = 128;  // bytes before the first tile image: {max |t|, max |t_c|, max |t|^2} (floats)
 constexpr uint32_t SPIN_LIMIT = 1u << 26;
 
@@ -158,9 +150,7 @@ __device__ __forceinline__ void umma_commit(uint32_t bar) {
       : "memory")
 // 32 consecutive accumulator columns of this thread's TMEM lane, issued without waiting ...
 __device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t (&r)[32]) {
-#ifndef KGE_EXP_NOLD
   KGE_TMEM_LD32_ASM(r, taddr);
-#endif
 }
 // ... and the wait; naming the registers keeps every use of them behind it.
 __device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[32]) {
@@ -496,10 +486,7 @@ struct EpiState {
   float thr;       // +inf: the row collects nothing (inactive, not representable, or its list overflowed)
   uint32_t widx;
 };
-#ifndef KGE_MMA_TRIG
-#define KGE_MMA_TRIG (CAND - 5)
-#endif
-constexpr int TRIG = KGE_MMA_TRIG;   // a list is compacted when it holds more than TRIG entries at the end of a tile
+constexpr int TRIG = CAND - 5;   // a list is compacted when it holds more than TRIG entries at the end of a tile
 
 // One chunk (32 columns = 8 groups of 4) of one row, in two steps so that the registers of the chunk are free for
 // the next tcgen05.ld as early as possible: the group maxima and the chunk maximum ...
@@ -551,6 +538,7 @@ __global__ void __launch_bounds__(sweep_threads(NH, NCOL, NMMA), (NBUF == 1 && N
   constexpr uint32_t TMEM_COLS = NH * TN * NBUF;
   static_assert(NMMA <= NH, "one issuer warp per row half at most");
   static_assert(NCH % 2 == 0 && (NBUF == 1 || NBUF == 2), "the chunk pipeline alternates two register sets");
+  static_assert(TRIG + NCH < CAND, "a list below the trigger takes one more tile's appends without reaching CAND");
   constexpr uint32_t IDESC = make_idesc(TN);
   extern __shared__ __align__(128) unsigned char smem[];
   const int kp = a.kp;
@@ -711,9 +699,7 @@ __global__ void __launch_bounds__(sweep_threads(NH, NCOL, NMMA), (NBUF == 1 && N
             for (int ks = 0; ks < ksteps; ++ks) {
               const uint64_t adesc = ((uint64_t)desc_hi << 32) | (a_lo + (uint32_t)ks * a_kstep);
               const uint64_t bdesc = ((uint64_t)desc_hi << 32) | (b_lo + (uint32_t)ks * b_kstep);
-#ifndef KGE_EXP_NOMMA   // timing experiments only (scripts/gpu_exp_sweep.sh); results are wrong with a knob set
               umma_f16(dcol, adesc, bdesc, IDESC, (ks0 + ks) > 0 ? 1u : 0u);
-#endif
             }
             if (j == a.nkc - 1) umma_commit(tfull0 + 8 * (buf * 2 + h));   // this half's accumulator is ready
             if (h == h_hi - 1) umma_commit(empty0 + 8 * s);                // stage reusable once its MMAs have read it
@@ -780,10 +766,7 @@ __global__ void __launch_bounds__(sweep_threads(NH, NCOL, NMMA), (NBUF == 1 && N
     float gm[8], gm2[8];
 
     {
-      // ---- one warp = (row half, lane quadrant, column slice); two accumulators per half -------------------
-      // Software pipeline over chunks: the load of the next chunk is in flight while the current one is filtered,
-      // and an accumulator goes back to the tensor core as soon as its last chunk sits in registers (the MMAs of
-      // the next tile already run in the other buffer).
+      // ---- one warp = (row half, lane quadrant, column slice) -------------------------------------------------
       const int h = NH == 2 ? (warp >> 2) & 1 : 0;
       const int cs = warp / (4 * NH);                   // column slice of the tile
       const int64_t lsplit = (int64_t)split * NCOL + cs;   // list index of this (target split, column slice)
@@ -794,15 +777,13 @@ __global__ void __launch_bounds__(sweep_threads(NH, NCOL, NMMA), (NBUF == 1 && N
       const uint32_t tlane = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(h * TN + cs * NCH * CH);
       const uint32_t my_tfull = tfull0 + 8 * h, my_tempty = tempty0 + 8 * h;   // + 16 * buf
       auto process = [&](const uint32_t (&r)[32], uint32_t cid) {
-#ifndef KGE_EXP_NOFILTER
         dump(r, u, cid);
         const float tm = chunk_reduce(r, gm);
         chunk_push(gm, tm, st, cid << CID_SHIFT, a.cand);   // (targets beyond the table: zero rows, chunks marked unsafe)
-#endif
       };
       uint32_t cid = (uint32_t)(t0 * (TN / CH) + cs * NCH);
-#ifndef KGE_MMA_CHUNKED_A
-      if constexpr (NBUF == 1 && NCH == 4) {
+      if constexpr (NBUF == 1) {
+        static_assert(NCH == 4, "one accumulator per half: a tile is read as two batches of two chunks");
         // One accumulator per half: what bounds the sweep is how long an accumulator stays away from the tensor
         // core, i.e. the number of TMEM round trips between "tile ready" and "tile in registers".  Chunk by chunk
         // that is four latencies per tile (measured: MMAs alone 1.21 ms, filter alone 0.98 ms, together 2.23 ms --
@@ -817,27 +798,21 @@ __global__ void __launch_bounds__(sweep_threads(NH, NCOL, NMMA), (NBUF == 1 && N
           // While the accumulator is held only what frees the registers runs (the two max trees: 40 ALU-pipe
           // instructions); the appends of the first batch wait until the accumulator is back with the tensor core.
           tmem_ld_wait2(va, vb);
-#ifndef KGE_EXP_NOFILTER
           dump(va, u, cid);
           const float tma = chunk_reduce(va, gm);
-#endif
           tmem_ld32_issue(tlane + 2 * CH, va);
-#ifndef KGE_EXP_NOFILTER
           dump(vb, u, cid + 1);
           const float tmb = chunk_reduce(vb, gm2);
-#endif
           tmem_ld32_issue(tlane + 3 * CH, vb);
           tmem_ld_wait2(va, vb);
           tc_fence_before();   // every chunk of the tile is in registers: release the accumulator
           __syncwarp();
           if (lane == 0) mbar_arrive(my_tempty);
-#ifndef KGE_EXP_NOFILTER
           chunk_push(gm, tma, st, cid << CID_SHIFT, a.cand);
           chunk_push(gm2, tmb, st, (cid + 1) << CID_SHIFT, a.cand);
-#endif
           process(va, cid + 2);
           process(vb, cid + 3);
-          compact_full(st, u, lsplit, TRIG < CAND - (NCH + 1) ? TRIG : CAND - (NCH + 1));
+          compact_full(st, u, lsplit, TRIG);
           if (i + 1 < nti) {   // computed while the second batch was filtered
             mbar_wait(my_tfull, (uint32_t)((i + 1) & 1));
             tc_fence_after();
@@ -845,46 +820,46 @@ __global__ void __launch_bounds__(sweep_threads(NH, NCOL, NMMA), (NBUF == 1 && N
             tmem_ld32_issue(tlane + CH, vb);
           }
         }
-        store_state(st, u, lsplit);
-        goto epilogue_done;
-      }
-#endif
-      mbar_wait(my_tfull, 0u);
-      tc_fence_after();
-      tmem_ld32_issue(tlane, va);
-      tmem_ld_wait(va);
-      for (int i = 0; i < nti; ++i, cid += TN / CH) {
-        const uint32_t buf = NBUF == 1 ? 0u : (uint32_t)(i & 1);
-        const uint32_t tbase = tlane + buf * NH * TN;
+      } else {
+        static_assert(NBUF == 2, "the chunk pipeline alternates two accumulators");
+        // Two accumulators per half, software pipeline over chunks: the load of the next chunk is in flight while the
+        // current one is filtered, and an accumulator goes back to the tensor core as soon as its last chunk sits in
+        // registers (the MMAs of the next tile already run in the other buffer).
+        mbar_wait(my_tfull, 0u);
+        tc_fence_after();
+        tmem_ld32_issue(tlane, va);
+        tmem_ld_wait(va);
+        for (int i = 0; i < nti; ++i, cid += TN / CH) {
+          const uint32_t buf = (uint32_t)(i & 1);
+          const uint32_t tbase = tlane + buf * NH * TN;
 #pragma unroll
-        for (int c = 0; c < NCH; ++c) {
-          uint32_t(&cur)[32] = (c & 1) ? vb : va;
-          uint32_t(&nxt)[32] = (c & 1) ? va : vb;
-          if (c + 1 < NCH) {
-            tmem_ld32_issue(tbase + (uint32_t)((c + 1) * CH), nxt);
-            process(cur, cid + c);
-            tmem_ld_wait(nxt);
-            if (c + 1 == NCH - 1) {   // every chunk of the tile is in registers: release the accumulator
-              tc_fence_before();
-              __syncwarp();
-              if (lane == 0) mbar_arrive(my_tempty + 16 * buf);
+          for (int c = 0; c < NCH; ++c) {
+            uint32_t(&cur)[32] = (c & 1) ? vb : va;
+            uint32_t(&nxt)[32] = (c & 1) ? va : vb;
+            if (c + 1 < NCH) {
+              tmem_ld32_issue(tbase + (uint32_t)((c + 1) * CH), nxt);
+              process(cur, cid + c);
+              tmem_ld_wait(nxt);
+              if (c + 1 == NCH - 1) {   // every chunk of the tile is in registers: release the accumulator
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive(my_tempty + 16 * buf);
+              }
+            } else {
+              if (i + 1 < nti) {
+                const uint32_t nbuf = buf ^ 1u;
+                mbar_wait(my_tfull + 16 * nbuf, (uint32_t)(((i + 1) / 2) & 1));
+                tc_fence_after();
+                tmem_ld32_issue(tlane + nbuf * NH * TN, nxt);
+              }
+              process(cur, cid + c);
+              if (i + 1 < nti) tmem_ld_wait(nxt);
             }
-          } else {
-            if (NBUF == 1) process(cur, cid + c);
-            if (i + 1 < nti) {
-              const uint32_t nbuf = NBUF == 1 ? 0u : (buf ^ 1u);
-              mbar_wait(my_tfull + 16 * nbuf, (uint32_t)(((i + 1) / NBUF) & 1));
-              tc_fence_after();
-              tmem_ld32_issue(tlane + nbuf * NH * TN, nxt);
-            }
-            if (NBUF != 1) process(cur, cid + c);
-            if (i + 1 < nti) tmem_ld_wait(nxt);
           }
+          compact_full(st, u, lsplit, TRIG);
         }
-        compact_full(st, u, lsplit, TRIG < CAND - (NCH + 1) ? TRIG : CAND - (NCH + 1));
       }
       store_state(st, u, lsplit);
-    epilogue_done:;
     }
   }
 
@@ -946,11 +921,8 @@ __device__ __forceinline__ uint64_t warp_sort_desc(uint64_t key, int lane) {
   return key;
 }
 
-#ifndef KGE_RS_MINB
-#define KGE_RS_MINB 2
-#endif
 template <bool DIST>
-__global__ void __launch_bounds__(RS_WARPS * 32, KGE_RS_MINB) rescore_topk_kernel(const RescoreArgs a) {
+__global__ void __launch_bounds__(RS_WARPS * 32, 2) rescore_topk_kernel(const RescoreArgs a) {
   extern __shared__ __align__(128) unsigned char smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int d = a.s.m.d;
@@ -1422,7 +1394,7 @@ extern "C" int kge_full_sort_topk_mma(const kge_model_t* model, const int64_t* h
         <<<grid, sweep_threads(NH_, NC_, NM_), pl.smem, st>>>(a);                                                 \
   } while (0)
   if (pl.cfg == 'a') {
-    if (debug_scores) KGE_SWEEP(2, 128, 1, 1, KGE_MMA_A_NMMA, true); else KGE_SWEEP(2, 128, 1, 1, KGE_MMA_A_NMMA, false);
+    if (debug_scores) KGE_SWEEP(2, 128, 1, 1, 1, true); else KGE_SWEEP(2, 128, 1, 1, 1, false);
   } else if (pl.cfg == 'f') {
     if (debug_scores) KGE_SWEEP(2, 128, 2, 2, 2, true); else KGE_SWEEP(2, 128, 2, 2, 2, false);
   } else if (pl.cfg == 'c') {

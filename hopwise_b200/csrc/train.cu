@@ -93,47 +93,28 @@ __device__ __forceinline__ int2 row_state(const kge_table_t& T, int64_t row) {
   return *(reinterpret_cast<const int2*>(T.row_state) + row);
 }
 
+// Mark a row as touched in `step` (an idempotent plain store); skipped when the loaded state shows it.
+__device__ __forceinline__ void touch_row(const kge_table_t& T, int64_t row, int seen_touch, int step, int gl) {
+  // (tables without row states -- dense Adam on every element, owner-sharded over the switch -- keep no marks)
+  if (gl != 0 || seen_touch == step || !T.row_state) return;
+  T.row_state[2 * row + 1] = step;
+}
+
 // Bring a fragment that was loaded from w up to step-1 when the row lags behind (rare path).
 // With `mark` (a training pass) the lagging row is also marked as touched, even if it will receive no gradient:
 // the Adam kernel then brings it up to date with a zero-gradient step (exactly what dense Adam does to it), so
 // the lag of a row that keeps being referenced by inactive triples stays bounded -- without this every forward
 // pass would replay the same (growing, up to the cap) run of skipped steps for it again.
-// Where the rows a training pass touches are recorded besides their mark: the table's slice of
-// kge_model_t.touch_list (which: 0 user, 1 entity, 2 relation) when the model carries one and the pass trains.
-// (The model is passed by reference and the slice is formed on the marking path only: held in registers across the
-// loop body the three slices cost the 64-register shapes another 200 bytes of spills.)
-struct TouchList {
-  const kge_model_t& m;
-  int which;
-  int on;
-};
-
-// Mark a row as touched in `step`; skipped when the loaded state shows it.  Without a list the mark is an idempotent
-// plain store.  With one, an exchange decides which group saw the row first, and that group appends it -- once.
-__device__ __forceinline__ void touch_row(const kge_table_t& T, int64_t row, int seen_touch, int step, int gl,
-                                          const TouchList& tl) {
-  // (tables without row states -- dense Adam on every element, owner-sharded over the switch -- keep no marks)
-  if (gl != 0 || seen_touch == step || !T.row_state) return;
-  if (tl.on && tl.m.touch_list) {
-    if (atomicExch(&T.row_state[2 * row + 1], step) != step) {
-      const int64_t base = tl.which == 0 ? 0 : (tl.which == 1 ? tl.m.user.rows : tl.m.user.rows + tl.m.entity.rows);
-      tl.m.touch_list[base + atomicAdd(tl.m.touch_count + 3 * (step & 1) + tl.which, 1)] = (int32_t)row;
-    }
-  } else {
-    T.row_state[2 * row + 1] = step;
-  }
-}
-
 template <int VEC, int G, int NCH>
 __device__ __forceinline__ void catch_up(const kge_table_t& T, int part, int64_t row, int2 st, int d, int gl,
-                                         const AdamDev& A, float (&x)[VEC * NCH], int mark, const TouchList& tl) {
+                                         const AdamDev& A, float (&x)[VEC * NCH], int mark) {
   const int last = st.x;
   if (last >= 0 && last < A.step - 1 && A.opt == KGE_OPT_ADAM) {   // (only Adam moves a row that has no gradient)
     float m[VEC * NCH], v[VEC * NCH];
     frag_load<VEC, G, NCH>(T.m[part], row, d, gl, m);
     frag_load<VEC, G, NCH>(T.v[part], row, d, gl, v);
     adam_replay<VEC * NCH>(x, m, v, last, A.step - 1, A);
-    if (mark && part == 0) touch_row(T, row, st.y, A.step, gl, tl);   // (last >= 0: the table has states)
+    if (mark && part == 0) touch_row(T, row, st.y, A.step, gl);   // (last >= 0: the table has states)
   }
 }
 
@@ -141,23 +122,15 @@ __device__ __forceinline__ void catch_up(const kge_table_t& T, int part, int64_t
 __device__ __forceinline__ float softplusf(float z) { return fmaxf(z, 0.f) + log1pf(expf(-fabsf(z))); }
 __device__ __forceinline__ float sigmoidf(float z) { return 1.f / (1.f + expf(-z)); }
 
-#ifndef KGE_FWD_TWO_PER_WARP
-#define KGE_FWD_TWO_PER_WARP 1   // see kge_train_forward (0: always one triple per warp for rows of 17..32 float4)
-#endif
-
 template <int MODEL, int VEC, int G, int NCH>
 struct FwdBounds {
   static constexpr int E = VEC * NCH;
   static constexpr int PH = (MODEL == KGE_ROTATE || MODEL == KGE_COMPLEX || MODEL == KGE_TRANSD) ? 2 : 1;
   // resident CTAs per SM the register budget is shaped for (more warps = more loads in flight)
-#ifdef KGE_FWD_MIN_CTAS
-  static constexpr int MIN_CTAS = KGE_FWD_MIN_CTAS;   // experiment knob (scripts/build_variant.sh)
-#else
   // (the two-triples-per-warp shape, G = 16 with two fragments per lane, wants its 8-element fragments of h, r, both
   // tails and three gradients in registers: measured 0.320 ms at two CTAs per SM vs 0.381 ms at three, cfg2)
   static constexpr int MIN_CTAS = (VEC == 4 && G == 16 && NCH == 2) ? 2
                                   : (E * PH <= 4) ? 4 : (E * PH <= 8 ? 3 : (E * PH <= 16 ? 2 : 1));
-#endif
 };
 
 // Shared memory of the WARP_RACC path: every warp's private [R][PR][d] relation-gradient copy, then one flag per
@@ -189,8 +162,6 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
   const float margin = a.m.margin;
   const kge_table_t& ET = a.m.entity;
   const kge_table_t& RT = a.m.relation;
-  // (small batches: every touched row is also appended to its table's slice of the touch list, kge_model_t)
-  const TouchList tl_user = {a.m, 0, a.with_grad}, tl_entity = {a.m, 1, a.with_grad}, tl_relation = {a.m, 2, a.with_grad};
 
   const int n_rel = (int)RT.rows;
   const int nv = d >> 2;
@@ -260,11 +231,11 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
 #pragma unroll
     for (int p = 0; p < PH; ++p) frag_load<VEC, G, NCH>(ET.w[p], tn_id, d, gl, tnx[p]);
 #pragma unroll
-    for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH>(HT, p, h_id, sh, d, gl, a.adam, h[p], a.with_grad, is_rec ? tl_user : tl_entity);
+    for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH>(HT, p, h_id, sh, d, gl, a.adam, h[p], a.with_grad);
 #pragma unroll
-    for (int p = 0; p < PR; ++p) catch_up<VEC, G, NCH>(RT, p, r_id, sr, d, gl, a.adam, r[p], a.with_grad, tl_relation);
+    for (int p = 0; p < PR; ++p) catch_up<VEC, G, NCH>(RT, p, r_id, sr, d, gl, a.adam, r[p], a.with_grad);
 #pragma unroll
-    for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH>(ET, p, tp_id, stp, d, gl, a.adam, tp[p], a.with_grad, tl_entity);
+    for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH>(ET, p, tp_id, stp, d, gl, a.adam, tp[p], a.with_grad);
 
     // gradient fragments of the anchor, relation and positive tail
     float gh[PH][E], gr[PR][E], gtp[PH][E];
@@ -409,7 +380,7 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
           for (int p = 0; p < PH; ++p) frag_load<VEC, G, NCH>(ET.w[p], tn_id, d, gl, tnx[p]);
         }
 #pragma unroll
-        for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH>(ET, p, t_id, st, d, gl, a.adam, t[p], a.with_grad, tl_entity);
+        for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH>(ET, p, t_id, st, d, gl, a.adam, t[p], a.with_grad);
       }
 
       if (MODEL == KGE_TRANSD) {
@@ -450,7 +421,7 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
             }
             frag_atomic_add<VEC, G, NCH>(ET.g[0], t_id, d, gl, dnv);
             frag_atomic_add<VEC, G, NCH>(ET.g[PH - 1], t_id, d, gl, gv);
-            touch_row(ET, t_id, st.y, step, gl, tl_entity);
+            touch_row(ET, t_id, st.y, step, gl);
           }
         }
       } else if (MODEL == KGE_TRANSH) {
@@ -477,7 +448,7 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
               t[0][e] = gneg * c2[e];                                      // back through the projection
             }
             frag_atomic_add<VEC, G, NCH>(ET.g[0], t_id, d, gl, t[0]);
-            touch_row(ET, t_id, st.y, step, gl, tl_entity);
+            touch_row(ET, t_id, st.y, step, gl);
           }
         }
       } else if (MODEL == KGE_TRANSE) {
@@ -502,7 +473,7 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
               gtp[0][e] -= c1[e];
             }
             frag_atomic_add<VEC, G, NCH>(ET.g[0], t_id, d, gl, t[0]);
-            touch_row(ET, t_id, st.y, step, gl, tl_entity);
+            touch_row(ET, t_id, st.y, step, gl);
           }
         }
       } else if (MODEL == KGE_DISTMULT) {
@@ -522,7 +493,7 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
               gtn[e] = w * c0[e];
             }
             frag_atomic_add<VEC, G, NCH>(ET.g[0], t_id, d, gl, gtn);
-            touch_row(ET, t_id, st.y, step, gl, tl_entity);
+            touch_row(ET, t_id, st.y, step, gl);
           }
         }
       } else if (MODEL == KGE_ROTATE) {
@@ -559,7 +530,7 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
           } else {
 #pragma unroll
             for (int p = 0; p < PH; ++p) frag_atomic_add<VEC, G, NCH>(ET.g[p], t_id, d, gl, t[p]);
-            touch_row(ET, t_id, st.y, step, gl, tl_entity);
+            touch_row(ET, t_id, st.y, step, gl);
           }
         }
       } else {
@@ -588,7 +559,7 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
           } else {
 #pragma unroll
             for (int p = 0; p < PH; ++p) frag_atomic_add<VEC, G, NCH>(ET.g[p], t_id, d, gl, t[p]);
-            touch_row(ET, t_id, st.y, step, gl, tl_entity);
+            touch_row(ET, t_id, st.y, step, gl);
           }
         }
       }
@@ -684,8 +655,8 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
         frag_atomic_add<VEC, G, NCH>(HT.g[p], h_id, d, gl, gh[p]);
         frag_atomic_add<VEC, G, NCH>(ET.g[p], tp_id, d, gl, gtp[p]);
       }
-      touch_row(HT, h_id, sh.y, step, gl, is_rec ? tl_user : tl_entity);
-      touch_row(ET, tp_id, stp.y, step, gl, tl_entity);
+      touch_row(HT, h_id, sh.y, step, gl);
+      touch_row(ET, tp_id, stp.y, step, gl);
       if (is_rec) {
         rec_seen = true;
 #pragma unroll
@@ -695,7 +666,7 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
       } else if (!WARP_RACC) {
 #pragma unroll
         for (int p = 0; p < PR; ++p) frag_atomic_add<VEC, G, NCH>(RT.g[p], r_id, d, gl, gr[p]);
-        touch_row(RT, r_id, sr.y, step, gl, tl_relation);
+        touch_row(RT, r_id, sr.y, step, gl);
       }
     }
 
@@ -758,7 +729,7 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
       atomicAdd(reinterpret_cast<float4*>((p == 0 ? RT.g[0] : RT.g[PR - 1]) + (int64_t)row * d) + c, s);
     }
     for (int row = threadIdx.x; row < n_rel; row += blockDim.x)
-      if (s_rtouch[row]) touch_row(RT, row, -1, step, 0, tl_relation);
+      if (s_rtouch[row]) touch_row(RT, row, -1, step, 0);
   } else {
     if (rec_seen) {
 #pragma unroll
@@ -777,7 +748,7 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
         const int p = i / d, col = i - p * d;
         atomicAdd(RT.g[p] + (int64_t)a.m.ui_relation * d + col, s_racc[i]);
       }
-      if (threadIdx.x == 0) touch_row(RT, a.m.ui_relation, -1, step, 0, tl_relation);
+      if (threadIdx.x == 0) touch_row(RT, a.m.ui_relation, -1, step, 0);
     }
   }
   lsum = warp_sum(lsum);
@@ -882,32 +853,6 @@ __global__ void __launch_bounds__(256) adam_apply_kernel(const ApplyArgs a) {
   const int gl = (threadIdx.x & 31) % G;
   const int step = a.adam.step;
   const float scale = a.scale_dev ? a.scale * __ldg(a.scale_dev) : a.scale;
-  if (a.m.touch_list) {
-    // Small batch: the forward pass listed the touched rows; one row per lane group, no scan, no imbalance.
-    const int64_t group = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G;
-    const int64_t n_groups = (int64_t)gridDim.x * blockDim.x / G;
-    const int32_t* ul = a.m.touch_list;
-    const int32_t* el = ul + a.m.user.rows;
-    const int32_t* rl = el + a.m.entity.rows;
-    // (two sets of counters, by step parity: this kernel zeroes the set the NEXT forward pass will count into --
-    // nobody reads or writes it while this kernel runs -- which saves a memset node in front of every forward pass)
-    const int32_t* cnt = a.m.touch_count + 3 * (step & 1);
-    const int nu = cnt[0], ne = cnt[1], nr = cnt[2];
-    if (blockIdx.x == 0 && threadIdx.x < 3) a.m.touch_count[3 * ((step + 1) & 1) + threadIdx.x] = 0;
-    for (int64_t i = group; i < nu; i += n_groups) {
-      const int64_t row = __ldg(ul + i);
-      adam_row<VEC, G, NCH>(a.m.user, row, a.m.user.row_state[2 * row], a.m.d, gl, a.adam, scale);
-    }
-    for (int64_t i = group; i < ne; i += n_groups) {
-      const int64_t row = __ldg(el + i);
-      adam_row<VEC, G, NCH>(a.m.entity, row, a.m.entity.row_state[2 * row], a.m.d, gl, a.adam, scale);
-    }
-    for (int64_t i = group; i < nr; i += n_groups) {
-      const int64_t row = __ldg(rl + i);
-      adam_row<VEC, G, NCH>(a.m.relation, row, a.m.relation.row_state[2 * row], a.m.d, gl, a.adam, scale);
-    }
-    return;
-  }
   auto marked = [step](int2 st) { return st.y == step; };
   // (the tables are kernel parameters: index them by name, a pointer array would copy them to local memory)
   for_selected_rows<G>(a.m.user, a.win[0], marked, [&](int64_t row, int last) {
@@ -1117,8 +1062,6 @@ extern "C" int kge_train_forward(const kge_model_t* model, const kge_batch_t* b,
   KGE_REQUIRE(adam->step >= 1, KGE_E_ARG, "adam.step is 1-based");
   KGE_REQUIRE(adam->optimizer >= KGE_OPT_ADAM && adam->optimizer <= KGE_OPT_RMSPROP, KGE_E_ARG, "unknown optimizer %d",
               adam->optimizer);
-  KGE_REQUIRE((model->touch_list == nullptr) == (model->touch_count == nullptr), KGE_E_ARG,
-              "touch_list and touch_count go together");
   const int64_t n_total = b->n_rec + b->n_kg;
   if (n_total == 0) return 0;
   KGE_REQUIRE(b->n_rec == 0 || (b->user && b->item && b->neg_item), KGE_E_ARG, "NULL rec id array");
@@ -1158,7 +1101,7 @@ extern "C" int kge_train_forward(const kge_model_t* model, const kge_batch_t* b,
   const double table_bytes = ((double)model->user.rows + (double)model->entity.rows) * model->d * 16.0;
   // (a batch that does not fill the resident warps even once -- the reference's 2048 + 2048 -- is bound by the
   // length of one warp's dependent instruction chain: one triple per warp halves it and doubles the warps)
-  const bool two_per_warp = c.vec == 4 && c.g == 32 && c.nch == 1 && KGE_FWD_TWO_PER_WARP && table_bytes < 96e6 &&
+  const bool two_per_warp = c.vec == 4 && c.g == 32 && c.nch == 1 && table_bytes < 96e6 &&
                             n_total >= (int64_t)kge_num_sms() * 256 &&
                             (kind == KGE_TRANSE || kind == KGE_DISTMULT);
   const int threads = 256;

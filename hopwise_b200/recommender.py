@@ -275,9 +275,6 @@ class FusedKGEModel(KnowledgeRecommender):
         alloc = self.__dict__.get("_g_alloc")
         st["g_flat"] = alloc(g_numel, device) if alloc is not None else torch.zeros(g_numel, device=device)
         st["row_state_flat"] = torch.full((sum(rows for _, _, rows in fams), 2), -1, dtype=torch.int32, device=device)
-        # small batches: the rows a step touches, listed by the forward pass for the optimiser kernel (kge_model_t)
-        st["touch_list"] = torch.empty(sum(rows for _, _, rows in fams), dtype=torch.int32, device=device)
-        st["touch_count"] = torch.zeros(6, dtype=torch.int32, device=device)   # two sets, by step parity
         # the moments share the gradient buffer's flat layout (an owner-sharded optimiser step walks the three
         # buffers -- and the weights, below -- element for element)
         flat_len = (g_numel + 3) // 4 * 4
@@ -334,28 +331,19 @@ class FusedKGEModel(KnowledgeRecommender):
         self._struct_cache = {}
         return st
 
-    def _model_struct(self, with_state: bool, listed: bool = False) -> _abi.kge_model_t:
+    def _model_struct(self, with_state: bool) -> _abi.kge_model_t:
         # the struct only holds pointers and shapes: rebuilt when a table or the optimiser state moves
         with_state = bool(with_state) and self._state is not None
-        slot = 2 if (listed and with_state) else int(with_state)
-        ckey = (slot, self._ready_key, id(self._state))
-        hit = self._struct_cache.get(slot)
+        ckey = (with_state, self._ready_key, id(self._state))
+        hit = self._struct_cache.get(with_state)
         if hit is not None and hit[0] == ckey:
             return hit[1]
-        m = self._build_model_struct(with_state, slot == 2)
+        m = self._build_model_struct(with_state)
         if self._ready_key is not None:
-            self._struct_cache[slot] = (ckey, m)
+            self._struct_cache[with_state] = (ckey, m)
         return m
 
-    # A step that can touch at most this many rows hands the optimiser kernel a list of them (no scan of the row
-    # states, no imbalance between the scanning warps).  Off by default (0).  Measured at the reference batch
-    # (2048 + 2048, cfg2): the optimiser kernel 21 -> 16 us and the back-to-back step 32.6 -> 29.6 us of device time,
-    # but every first touch now costs the forward pass two dependent atomic round trips (exchange the mark, then take
-    # a list slot), and with a cold L2 -- how bench.py times its legs -- the step goes 43.7 -> 58.6 us.  Set it to
-    # e.g. 65536 for long runs of small batches over tables that stay in L2.
-    LIST_ROWS_MAX = 0
-
-    def _build_model_struct(self, with_state: bool, listed: bool = False) -> _abi.kge_model_t:
+    def _build_model_struct(self, with_state: bool) -> _abi.kge_model_t:
         m = _abi.kge_model_t()
         m.model = _abi.MODEL_KINDS[self.KIND]
         m.d = self.embedding_size
@@ -383,9 +371,6 @@ class FusedKGEModel(KnowledgeRecommender):
         if st is not None:
             m.adam_table = st["adam_table"].data_ptr()
             m.adam_table_len = st["adam_table_len"]
-            if listed:
-                m.touch_list = st["touch_list"].data_ptr()
-                m.touch_count = st["touch_count"].data_ptr()
         return m
 
     def _adam_struct(self, step: int) -> _abi.kge_adam_t:
@@ -458,9 +443,7 @@ class FusedKGEModel(KnowledgeRecommender):
         if self._pending:  # a loss whose backward never ran: drop its gradient
             self._discard_pending(lib, stream)
         b, keep = self._batch_struct(interaction, device)
-        listed = with_grad and self._lists_touched_rows(b)
-        _plain_set(self, "_listed", listed)
-        m = self._model_struct(lazy, listed)
+        m = self._model_struct(lazy)
         a = self._adam_struct(self._step + 1)
         loss = torch.zeros(1, device=device)
         _abi.check(
@@ -478,23 +461,7 @@ class FusedKGEModel(KnowledgeRecommender):
             _plain_set(self, "_pending", True)
         return loss.reshape(())
 
-    def _lists_touched_rows(self, b) -> bool:
-        """Whether this step lists its touched rows for the optimiser kernel (LIST_ROWS_MAX): single replica only --
-        an exchange marks rows itself -- and small enough that one atomic per first touch is cheap."""
-        listed = False
-        if self._grad_sync is None and not self._owner_adam and self._state is not None:
-            refs = int(b.n_rec) * (2 + int(b.k_rec)) + int(b.n_kg) * (3 + int(b.k_kg))
-            listed = 0 < refs <= self.LIST_ROWS_MAX
-        # the optimiser kernel of a listed step zeroes the counters of the next one; after a step that was not listed
-        # (or never applied) they are stale
-        if listed and not self.__dict__.get("_listed_last", False):
-            self._state["touch_count"].zero_()
-        _plain_set(self, "_listed_last", listed)
-        return listed
-
     def _discard_pending(self, lib, stream):
-        self._state["touch_count"].zero_()   # (the dropped step's rows were counted; the optimiser kernel never ran)
-        _plain_set(self, "_listed_last", False)
         if self._owner_adam:
             self._state["g_flat"].zero_()
         else:
@@ -519,7 +486,7 @@ class FusedKGEModel(KnowledgeRecommender):
             g = grad_out
             if g is not None and (g.dtype != torch.float32 or g.numel() != 1 or g.requires_grad):
                 g = g.detach().to(torch.float32).reshape(1).contiguous()
-            m = self._model_struct(True, self.__dict__.get("_listed", False))
+            m = self._model_struct(True)
             a = self._adam_struct(self._step + 1)
             _abi.check(
                 lib.kge_adam_apply(C.byref(m), C.byref(a), float(self._grad_scale), _abi.ptr(g), _abi.stream_ptr()),
@@ -572,7 +539,7 @@ class FusedKGEModel(KnowledgeRecommender):
         pos = ring[2]
         ring[2] = pos + 1
         b, keep = self._batch_struct(interaction, device)
-        m = self._model_struct(True, self._lists_touched_rows(b))
+        m = self._model_struct(True)
         a = self._adam_struct(self._step + 1)
         _abi.check(
             lib.kge_train_step(C.byref(m), C.byref(b), C.byref(a), float(self._grad_scale), ring[3] + 4 * pos, stream),

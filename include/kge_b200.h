@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define KGE_ABI_VERSION 6
+#define KGE_ABI_VERSION 7
 
 typedef void* kge_stream_t; /* cudaStream_t */
 
@@ -83,14 +83,6 @@ typedef struct {
   const float* adam_table;      /* [2*adam_table_len]: {lr/(1-b1^j), 1/sqrt(1-b2^j)} for j = 0..len-1 */
   int32_t adam_table_len;
   int32_t _pad2;
-  /* Optional (both or neither; small batches): the training pass appends every row it touches, once, to
-   * touch_list -- user rows at [0, user.rows), entity rows from user.rows, relation rows behind them -- and counts
-   * them per table in touch_count[6] (two sets of three, by step parity; zero before the first step);
-   * kge_adam_apply walks the three lists instead of scanning every row state and zeroes the other parity's set for
-   * the next step.  A gradient that is dropped instead of applied leaves its set to be zeroed by the caller.  Leave
-   * both NULL when anything else marks rows (the data-parallel exchange). */
-  int32_t* touch_list;
-  int32_t* touch_count;
 } kge_model_t;
 
 /* One training batch, the fields Interaction carries into calculate_loss

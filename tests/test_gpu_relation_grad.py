@@ -128,14 +128,12 @@ def test_forward_without_gradient_touches_nothing():
     assert not bool((st["row_state"][:, 1] == m._step + 1).any())
 
 
-@pytest.mark.parametrize("listed", [False, True])
-def test_marked_relation_rows_follow_the_rule(listed):
+def test_marked_relation_rows_follow_the_rule():
     """Marked = every row with an active triple, plus every lagging row a triple references (brought up to date by a
-    zero-gradient step), with and without the touch list."""
+    zero-gradient step)."""
     R = 22
     margin = 0.0   # about half of the pairs are inactive
     m = make_product_model("TransE", U, I, E, R, D, margin=margin)
-    m.LIST_ROWS_MAX = (1 << 24) if listed else 0
     rng = np.random.default_rng(14)
     # step 1 references every relation, steps 2-3 only relation 1: the others lag behind at step 4
     for step in range(3):
@@ -149,9 +147,6 @@ def test_marked_relation_rows_follow_the_rule(listed):
     b["relation_id"][np.isin(b["relation_id"], single)] = 2
     b["relation_id"][: len(single)] = single
     got, marked = _forward(m, b)
-    if listed:
-        assert m._listed
-        assert int(m._state["touch_count"][2]) == int(marked.sum())
     _, active = _closed_form(m, "TransE", b, R, margin)   # (state_dict brings the lagging rows to step 3)
     lagging = np.ones(R, dtype=bool)
     lagging[[1, R - 1]] = False
