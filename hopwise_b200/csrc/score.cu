@@ -179,7 +179,7 @@ struct TileArgs {
   const int64_t* hist_items;
   int mask_first;
   int k;
-  uint64_t* part_keys;  // [n, n_splits, k]
+  uint64_t* part_keys;  // [n, n_splits, k]; large k: [n, n_splits, buf_cap]
   int n_splits;
   // Indirect rows (the tensor-core path's device-side fallback): the CTA works on entries [row_begin, min(*row_count,
   // row_end)) of row_map instead of rows [0, n); the row count is only known on the device, so the grid is sized for
@@ -196,11 +196,115 @@ struct TileArgs {
   uint64_t* rank_unmasked;     // [n]
   uint64_t* rank_ninf;         // [n]
   int64_t rank_cap;            // positives the workspace holds
+  // large-k epilogue: keys one (row, split) buffer of part_keys holds (>= k + BT)
+  int64_t buf_cap;
 };
 
 // Epilogue of the tile kernel: the dense scores, the per-row top-k, or the rank counts of listed targets.
-constexpr int EPI_DENSE = 0, EPI_TOPK = 1, EPI_RANK = 2;
+// EPI_TOPK_LARGE is the top-k for k > KMAX (see large_k_cap).
+constexpr int EPI_DENSE = 0, EPI_TOPK = 1, EPI_RANK = 2, EPI_TOPK_LARGE = 3;
 constexpr int RANK_SM = 16;   // thresholds a row keeps in shared memory; rows with more count in global memory
+
+// ---- large-k top-k (k > KMAX) -----------------------------------------------------------------------------------
+// A sorted list of k keys per row no longer fits shared memory, so each (row, split) appends the keys that beat the
+// row's threshold to a buffer of buf_cap = large_k_cap(k) keys in the workspace.  When a tile's keys would overflow
+// it, the buffer is compacted to exactly its top k (keys are unique: the id is part of the key) and the threshold
+// rises to the k-th key.  A merge kernel then selects each row's top k over its splits and sorts them.
+__host__ __device__ __forceinline__ int64_t large_k_cap(int64_t k) { return (2 * k + 31) / 32 * 32; }   // >= k + BT
+
+__device__ __forceinline__ uint64_t warp_min_u64(uint64_t x) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) x = min(x, (uint64_t)__shfl_xor_sync(0xffffffffu, x, o));
+  return x;
+}
+__device__ __forceinline__ int64_t warp_sum_i64(int64_t x) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+  return x;
+}
+
+// The k-th largest non-zero key among keys[s * stride + i] (s < nseg, i < len), or 0 when fewer than k are non-zero;
+// every lane of the warp returns it.  mma_topk.cu's warp_kth_largest on 64-bit keys in memory: the radix descent
+// starts at the highest bit in which the keys differ and stops as soon as exactly k keys remain above the prefix.
+__device__ __forceinline__ uint64_t warp_kth_largest_mem(const uint64_t* keys, int64_t nseg, int64_t len, int64_t stride,
+                                                      int64_t k) {
+  const int lane = threadIdx.x & 31;
+  int64_t n_t = 0;
+  uint64_t k_or = 0ull, k_and = ~0ull;
+  for (int64_t s = 0; s < nseg; ++s)
+    for (int64_t i = lane; i < len; i += 32) {
+      const uint64_t x = keys[s * stride + i];
+      if (x) {
+        ++n_t;
+        k_or |= x;
+        k_and &= x;
+      }
+    }
+  n_t = warp_sum_i64(n_t);
+  if (n_t < k) return 0ull;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    k_or |= (uint64_t)__shfl_xor_sync(0xffffffffu, k_or, o);
+    k_and &= (uint64_t)__shfl_xor_sync(0xffffffffu, k_and, o);
+  }
+  const uint64_t diff = k_or ^ k_and;
+  if (diff == 0ull) return k_or;   // one key
+  const int top = 63 - __clzll((long long)diff);
+  uint64_t P = top == 63 ? 0ull : (k_and & ~((2ull << top) - 1ull));   // invariant: #(key >= max(P, 1)) = n_t >= k
+  for (int bit = top; bit >= 0 && n_t > k; --bit) {
+    const uint64_t c = P | (1ull << bit);
+    int64_t n = 0;
+    for (int64_t s = 0; s < nseg; ++s)
+      for (int64_t i = lane; i < len; i += 32) n += keys[s * stride + i] >= c;
+    n = warp_sum_i64(n);
+    if (n >= k) {
+      P = c;
+      n_t = n;
+    }
+  }
+  const uint64_t T = P ? P : 1ull;
+  uint64_t mn = ~0ull;
+  for (int64_t s = 0; s < nseg; ++s)
+    for (int64_t i = lane; i < len; i += 32) {
+      const uint64_t x = keys[s * stride + i];
+      if (x >= T) mn = min(mn, x);
+    }
+  return warp_min_u64(mn);
+}
+
+// Keep the keys >= T (T > 0) of buf[0, len), in order, in place; returns the new length (lane-uniform).  Writes never
+// overtake reads: a key moves to a position at or below its own, and the ballot orders a round's reads before its
+// writes.
+__device__ __forceinline__ int warp_keep_at_least(uint64_t* buf, int len, uint64_t T) {
+  const int lane = threadIdx.x & 31;
+  int w = 0;
+  for (int base = 0; base < len; base += 32) {
+    const int i = base + lane;
+    const uint64_t x = i < len ? buf[i] : 0ull;
+    const bool keep = x >= T;
+    const unsigned b = __ballot_sync(0xffffffffu, keep);
+    if (keep) buf[w + __popc(b & ((1u << lane) - 1u))] = x;
+    w += __popc(b);
+  }
+  __syncwarp();
+  return w;
+}
+
+// Sort buf[0, P) descending with the whole block (bitonic network; P a power of two).
+__device__ __forceinline__ void block_bitonic_sort_desc(uint64_t* buf, int64_t P) {
+  for (int64_t size = 2; size <= P; size <<= 1)
+    for (int64_t stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int64_t i = threadIdx.x; i < P / 2; i += blockDim.x) {
+        const int64_t lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
+        const uint64_t x = buf[lo], y = buf[hi];
+        if ((lo & size) == 0 ? x < y : x > y) {
+          buf[lo] = y;
+          buf[hi] = x;
+        }
+      }
+      __syncthreads();
+    }
+}
 
 __device__ __forceinline__ void build_queries(const ScoreArgs& a, const int64_t* rowid, int nrows, int kpad, float* Qs,
                                               const float* proj = nullptr) {
@@ -248,9 +352,10 @@ __device__ __forceinline__ void load_target_chunk(const float* __restrict__ W, i
 // MODE: how a (query, target) pair of rows is contracted (score_common.cuh).  EPI: what the sweep does with the scores.
 // The rank epilogue asks for two CTAs per SM (128 registers): under the compiler's default budget it spills.
 template <int MODE, int EPI>
-__global__ void __launch_bounds__(TILE_THREADS, EPI == EPI_RANK ? 2 : 0) fullsort_tile_kernel(const TileArgs a) {
+__global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_TOPK_LARGE) ? 2 : 0) fullsort_tile_kernel(const TileArgs a) {
   constexpr bool DIST = MODE == MODE_DIST || MODE == MODE_PROJ;
-  constexpr bool TOPK = EPI == EPI_TOPK, RANK = EPI == EPI_RANK;
+  constexpr bool TOPK = EPI == EPI_TOPK, RANK = EPI == EPI_RANK, LARGE = EPI == EPI_TOPK_LARGE;
+  constexpr bool SEL = TOPK || LARGE;         // a top-k epilogue: candidate keys staged per tile
   constexpr bool MASKED = EPI != EPI_DENSE;   // the trainer's masking: column 0 and the history -> -inf
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int model = a.s.m.model;
@@ -265,11 +370,11 @@ __global__ void __launch_bounds__(TILE_THREADS, EPI == EPI_RANK ? 2 : 0) fullsor
   // top-k only
   uint64_t* lists = reinterpret_cast<uint64_t*>(Ts + BT * TS);  // [BU][k]
   uint64_t* cand = lists + (TOPK ? BU * k : 0);                 // [BU][BT]
-  uint64_t* thr = cand + (TOPK ? BU * BT : 0);                  // [BU]
-  uint32_t* maskbits = reinterpret_cast<uint32_t*>(thr + (TOPK ? BU : 0));  // [BU][BT/32] (top-k and rank)
+  uint64_t* thr = cand + (SEL ? BU * BT : 0);                   // [BU]
+  uint32_t* maskbits = reinterpret_cast<uint32_t*>(thr + (SEL ? BU : 0));  // [BU][BT/32] (top-k and rank)
   int* cnt = reinterpret_cast<int*>(maskbits + (MASKED ? BU * (BT / 32) : 0));  // [BU]
-  int* llen = cnt + (TOPK ? BU : 0);                                        // [BU]
-  int64_t* cursor = reinterpret_cast<int64_t*>(llen + (TOPK ? BU : 0));     // [BU] (8-byte aligned by layout)
+  int* llen = cnt + (SEL ? BU : 0);                                         // [BU] list / buffer length
+  int64_t* cursor = reinterpret_cast<int64_t*>(llen + (SEL ? BU : 0));      // [BU] (8-byte aligned by layout)
   int64_t* rowid = cursor + (MASKED ? BU : 0);                              // [BU] query row of each slot
   float* Cs = reinterpret_cast<float*>(rowid + BU);                         // [kpad] projection factor (MODE_PROJ)
   // rank only (kpad is a multiple of 32: rbase stays 8-byte aligned)
@@ -318,7 +423,7 @@ __global__ void __launch_bounds__(TILE_THREADS, EPI == EPI_RANK ? 2 : 0) fullsor
   uint32_t n_unm[4] = {0u, 0u, 0u, 0u}, n_ninf[4] = {0u, 0u, 0u, 0u};
   if (MASKED) {
     for (int u = threadIdx.x; u < BU; u += blockDim.x) {
-      if (TOPK) {
+      if (SEL) {
         thr[u] = 0ull;
         llen[u] = 0;
         cnt[u] = 0;
@@ -436,7 +541,7 @@ __global__ void __launch_bounds__(TILE_THREADS, EPI == EPI_RANK ? 2 : 0) fullsor
         }
         const bool masked = (a.mask_first && j == 0) || ((maskbits[u * (BT / 32) + (jo >> 5)] >> (jo & 31)) & 1u);
         if (masked) sc = -INFINITY;
-        if (TOPK) {
+        if (SEL) {
           const uint64_t key = make_key(sc, (uint32_t)j);
           if (key > thr[u]) {
             const int slot = atomicAdd(&cnt[u], 1);
@@ -492,6 +597,33 @@ __global__ void __launch_bounds__(TILE_THREADS, EPI == EPI_RANK ? 2 : 0) fullsor
       }
       // the next tile's first __syncthreads orders these writes before its reads
     }
+    if (LARGE) {
+      __syncthreads();
+      for (int u = warp; u < nrows; u += TILE_THREADS / 32) {
+        const int c = cnt[u];
+        if (c == 0) continue;
+        int len = llen[u];
+        uint64_t t = thr[u];
+        uint64_t* buf = a.part_keys + ((row0 + u) * a.n_splits + blockIdx.y) * a.buf_cap;
+        if (len + c > a.buf_cap) {   // len > k: keep exactly the top k, whose last key becomes the threshold
+          t = warp_kth_largest_mem(buf, 1, len, 0, k);
+          len = warp_keep_at_least(buf, len, t);
+        }
+        for (int base = 0; base < c; base += 32) {
+          const uint64_t key = base + lane < c ? cand[u * BT + base + lane] : 0ull;
+          const bool keep = key > t;
+          const unsigned b = __ballot_sync(0xffffffffu, keep);
+          if (keep) buf[len + __popc(b & ((1u << lane) - 1u))] = key;
+          len += __popc(b);
+        }
+        __syncwarp();
+        if (lane == 0) {
+          llen[u] = len;
+          cnt[u] = 0;
+          thr[u] = t;
+        }
+      }
+    }
     if (RANK) __syncthreads();   // every warp is done with this tile's history bits before they are cleared
   }
 
@@ -501,6 +633,16 @@ __global__ void __launch_bounds__(TILE_THREADS, EPI == EPI_RANK ? 2 : 0) fullsor
       const int u = idx / k, i = idx - u * k;
       const uint64_t key = (i < llen[u]) ? lists[u * k + i] : 0ull;
       a.part_keys[((row0 - a.row_begin + u) * a.n_splits + blockIdx.y) * k + i] = key;
+    }
+  }
+  if (LARGE) {
+    // each split leaves its top min(k, len) keys in the first k slots of its buffer, zero-padded
+    __syncthreads();
+    for (int u = warp; u < nrows; u += TILE_THREADS / 32) {
+      int len = llen[u];
+      uint64_t* buf = a.part_keys + ((row0 + u) * a.n_splits + blockIdx.y) * a.buf_cap;
+      if (len > k) len = warp_keep_at_least(buf, len, warp_kth_largest_mem(buf, 1, len, 0, k));
+      for (int i = len + lane; i < k; i += 32) buf[i] = 0ull;
     }
   }
   if (RANK) {
@@ -564,6 +706,54 @@ __global__ void __launch_bounds__(256) topk_merge_kernel(const uint64_t* __restr
     if (scores_out) scores_out[row * k + i] = key ? key_score(key) : -INFINITY;
   }
   __syncwarp();
+  }
+}
+
+// Large-k merge, one CTA per row: warp 0 selects the k-th key T over the row's n_splits zero-padded lists of k keys
+// (the row has at least k keys: every split keeps min(k, its targets)), the block gathers the k keys >= T, sorts
+// them and decodes.  Up to SORT_SM keys the sort runs in shared memory; above, it runs in the row's own workspace
+// (buf_cap >= P keys), with the ids_out row as the staging area of the gather.
+constexpr int64_t SORT_SM = 8192;
+
+__global__ void __launch_bounds__(256) topk_merge_large_kernel(uint64_t* __restrict__ part_keys, int n_splits, int k,
+                                                               int64_t buf_cap, int64_t P, int64_t* __restrict__ ids_out,
+                                                               float* __restrict__ scores_out) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ uint64_t s_T;
+  __shared__ int s_n;
+  const int64_t row = blockIdx.x;
+  uint64_t* region = part_keys + row * n_splits * buf_cap;
+  if (threadIdx.x < 32) {
+    const uint64_t T = warp_kth_largest_mem(region, n_splits, k, buf_cap, k);
+    if (threadIdx.x == 0) {
+      s_T = T;
+      s_n = 0;
+    }
+  }
+  __syncthreads();
+  const uint64_t T = s_T;
+  const bool in_sm = P <= SORT_SM;
+  uint64_t* stage = in_sm ? reinterpret_cast<uint64_t*>(smem_raw) : reinterpret_cast<uint64_t*>(ids_out + row * k);
+  for (int s = 0; s < n_splits; ++s)
+    for (int i = threadIdx.x; i < k; i += blockDim.x) {
+      const uint64_t x = region[s * buf_cap + i];
+      if (x != 0ull && x >= T) {
+        const int slot = atomicAdd(&s_n, 1);
+        if (slot < k) stage[slot] = x;
+      }
+    }
+  __syncthreads();
+  const int64_t m = min(s_n, k);
+  uint64_t* buf = in_sm ? stage : region;
+  if (!in_sm)
+    for (int64_t i = threadIdx.x; i < m; i += blockDim.x) buf[i] = stage[i];
+  for (int64_t i = m + threadIdx.x; i < P; i += blockDim.x) buf[i] = 0ull;
+  __syncthreads();
+  block_bitonic_sort_desc(buf, P);
+  for (int64_t i = threadIdx.x; i < k; i += blockDim.x) {
+    const uint64_t key = buf[i];
+    ids_out[row * k + i] = key ? key_id(key) : -1;
+    if (scores_out) scores_out[row * k + i] = key ? key_score(key) : -INFINITY;
   }
 }
 
@@ -653,6 +843,81 @@ __global__ void __launch_bounds__(256) topk_metric_sums_kernel(const int32_t* __
     double t = 0.0;
     for (int w = 0; w < warps; ++w) t += acc[w * 5 * k + i];
     atomicAdd(&sums[i], t);
+  }
+}
+
+// The same sums for k > KMAX, whose per-warp [5][k] accumulators would not fit shared memory: blockIdx.y strides over
+// windows of MW cutoffs.  A lane first rebuilds its user's running state (hits, first hit, dcg, idcg) over the columns
+// before the window, adding in the same order as the loop above, then accumulates the window as above.
+constexpr int MW = 128;
+
+__global__ void __launch_bounds__(256) topk_metric_sums_window_kernel(const int32_t* __restrict__ rec, int64_t n, int k,
+                                                                      double* __restrict__ sums) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  double* acc = reinterpret_cast<double*>(smem_raw);  // [warps][5*MW]
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = blockDim.x >> 5;
+  double* mine = acc + warp * 5 * MW;
+  const int n_win = (k + MW - 1) / MW;
+  for (int win = blockIdx.y; win < n_win; win += gridDim.y) {
+    const int j0 = win * MW, j1 = min(k, j0 + MW);
+    __syncthreads();   // (the previous window's flush is done)
+    for (int i = threadIdx.x; i < warps * 5 * MW; i += blockDim.x) acc[i] = 0.0;
+    __syncthreads();
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t base = (int64_t)blockIdx.x * blockDim.x + warp * 32; base < n; base += stride) {
+      const int64_t u = base + lane;
+      const bool valid = u < n;
+      const int32_t* row = rec + (valid ? u : 0) * (int64_t)(k + 1);
+      const int pos_len = row[k];
+      const int ilen = pos_len < k ? pos_len : k;
+      int cum = 0, first = -1;
+      double dcg = 0.0, idcg = 0.0;
+      for (int j = 0; j < j0; ++j) {
+        if (row[j] != 0) {
+          if (first < 0) first = j;
+          dcg += 1.0 / log2((double)(j + 2));
+          ++cum;
+        }
+      }
+      for (int j = 0; j < min(ilen, j0); ++j) idcg += 1.0 / log2((double)(j + 2));
+      for (int j = j0; j < j1; ++j) {
+        const int hit = row[j] != 0;
+        const double disc = 1.0 / log2((double)(j + 2));
+        if (hit) {
+          if (first < 0) first = j;
+          dcg += disc;
+        }
+        cum += hit;
+        if (j < ilen) idcg += disc;
+        double v0 = (double)cum / (double)pos_len;
+        double v1 = first >= 0 ? 1.0 / (double)(first + 1) : 0.0;
+        double v2 = dcg / idcg;
+        double v3 = cum > 0 ? 1.0 : 0.0;
+        double v4 = (double)cum / (double)(j + 1);
+        if (!valid) v0 = v1 = v2 = v3 = v4 = 0.0;
+        v0 = warp_sum_f64(v0);
+        v1 = warp_sum_f64(v1);
+        v2 = warp_sum_f64(v2);
+        v3 = warp_sum_f64(v3);
+        v4 = warp_sum_f64(v4);
+        if (lane == 0) {
+          const int jj = j - j0;
+          mine[0 * MW + jj] += v0;
+          mine[1 * MW + jj] += v1;
+          mine[2 * MW + jj] += v2;
+          mine[3 * MW + jj] += v3;
+          mine[4 * MW + jj] += v4;
+        }
+      }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < 5 * MW; i += blockDim.x) {
+      const int c = i / MW, jj = i - c * MW;
+      if (j0 + jj >= j1) continue;
+      double t = 0.0;
+      for (int w = 0; w < warps; ++w) t += acc[w * 5 * MW + i];
+      atomicAdd(&sums[(int64_t)c * k + j0 + jj], t);
+    }
   }
 }
 
@@ -843,6 +1108,8 @@ int plan_tiles(const kge_model_t* m, int64_t n, int64_t n_targets, int k, int ep
   pl.kpad = (m->d + KC - 1) / KC * KC;
   size_t smem = (size_t)BU * parts * pl.kpad * 4 + (size_t)BT * TS * 4;
   if (epi == EPI_TOPK) smem += (size_t)BU * k * 8 + (size_t)BU * BT * 8 + BU * 8 + BU * (BT / 32) * 4 + BU * 4 * 2 + BU * 8;
+  if (epi == EPI_TOPK_LARGE)   // the same without the lists: cand, thr, maskbits, cnt, llen, cursor
+    smem += (size_t)BU * BT * 8 + BU * 8 + BU * (BT / 32) * 4 + BU * 4 * 2 + BU * 8;
   if (epi == EPI_RANK)   // maskbits, cursor | rbase, rthr, rcnt, rlo, rm
     smem += BU * (BT / 32) * 4 + BU * 8 + BU * 8 + (size_t)BU * RANK_SM * 4 * 3 + BU * 4 * 2;
   smem += BU * 8;   // rowid
@@ -853,10 +1120,13 @@ int plan_tiles(const kge_model_t* m, int64_t n, int64_t n_targets, int k, int ep
   const int64_t n_tiles = (n_targets + BT - 1) / BT;
   int splits = 1;
   if (epi != EPI_DENSE) {
-    // enough CTAs for two waves at 2 CTAs/SM, but at least 8 tiles per split
+    // enough CTAs for two waves at 2 CTAs/SM, but at least 8 tiles per split (large k: and at least k targets, so
+    // that the merge does not read many nearly empty lists)
     const int64_t want = (int64_t)kge_num_sms() * 4;
     int64_t s = (want + pl.n_blocks - 1) / pl.n_blocks;
-    const int64_t max_s = (n_tiles + 7) / 8;
+    const int64_t k_tiles = ((int64_t)k + BT - 1) / BT;
+    const int64_t min_tiles = (epi == EPI_TOPK_LARGE && k_tiles > 8) ? k_tiles : 8;
+    const int64_t max_s = (n_tiles + min_tiles - 1) / min_tiles;
     if (s > max_s) s = max_s;
     if (s < 1) s = 1;
     if (s > 65535) s = 65535;
@@ -996,8 +1266,12 @@ extern "C" int kge_full_sort_scores(const kge_model_t* model, const int64_t* hea
 
 extern "C" int64_t kge_full_sort_topk_workspace_bytes(const kge_model_t* model, int64_t n, int64_t n_targets,
                                                       int32_t k) {
-  if (!model || n < 0 || n_targets < 1 || k < 1 || k > KMAX) return -1;
+  if (!model || n < 0 || n_targets < 1 || k < 1) return -1;
   TilePlan pl = {};
+  if (k > KMAX) {
+    if (large_k_cap(k) > 0x7fffffff || plan_tiles(model, n > 0 ? n : 1, n_targets, k, EPI_TOPK_LARGE, pl)) return -1;
+    return (int64_t)n * pl.n_splits * large_k_cap(k) * 8;
+  }
   if (plan_tiles(model, n > 0 ? n : 1, n_targets, k, EPI_TOPK, pl)) return -1;
   return (int64_t)n * pl.n_splits * k * 8;
 }
@@ -1010,15 +1284,17 @@ extern "C" int kge_full_sort_topk(const kge_model_t* model, const int64_t* heads
   KGE_REQUIRE(model->model != KGE_TRANSH || rels == nullptr, KGE_E_UNSUPPORTED,
               "TransH full-sort takes the user->item relation only (transh.py:125-145; no KG scoring in the reference)");
   KGE_REQUIRE(n >= 0 && n_targets >= 1 && n_targets <= model->entity.rows, KGE_E_ARG, "bad n / n_targets");
-  KGE_REQUIRE(k >= 1 && k <= KMAX, KGE_E_UNSUPPORTED, "k=%d outside [1, %d]", k, KMAX);
+  KGE_REQUIRE(k >= 1, KGE_E_UNSUPPORTED, "k=%d below 1", k);
   KGE_REQUIRE(k <= n_targets, KGE_E_ARG, "k=%d larger than the number of targets", k);
   KGE_REQUIRE(n_targets < 0xFFFFFFFFll, KGE_E_UNSUPPORTED, "more than 2^32-2 targets");
   if (n == 0) return 0;
   KGE_REQUIRE(heads && ids_out, KGE_E_ARG, "NULL heads / ids_out");
   KGE_REQUIRE((hist_off == nullptr) == (hist_items == nullptr) || hist_off, KGE_E_ARG, "hist_items without hist_off");
+  const bool large = k > KMAX;
+  KGE_REQUIRE(!large || large_k_cap(k) <= 0x7fffffff, KGE_E_UNSUPPORTED, "k=%d: buffers above 2^31 keys", k);
   TilePlan pl = {};
-  if (int e = plan_tiles(model, n, n_targets, k, EPI_TOPK, pl)) return e;
-  const int64_t need = n * pl.n_splits * k * 8;
+  if (int e = plan_tiles(model, n, n_targets, k, large ? EPI_TOPK_LARGE : EPI_TOPK, pl)) return e;
+  const int64_t need = n * pl.n_splits * (large ? large_k_cap(k) : k) * 8;
   KGE_REQUIRE(workspace && workspace_bytes >= need, KGE_E_ARG, "workspace too small: need %lld bytes", (long long)need);
   TileArgs a = {};
   a.s.m = *model;
@@ -1039,6 +1315,23 @@ extern "C" int kge_full_sort_topk(const kge_model_t* model, const int64_t* heads
   a.n_splits = pl.n_splits;
   cudaStream_t st = (cudaStream_t)stream;
   const int mode = tile_mode(model->model);
+  if (large) {
+    a.buf_cap = large_k_cap(k);
+    if (int e = mode == MODE_DIST ? launch_tile<MODE_DIST, EPI_TOPK_LARGE>(a, pl, st)
+                                  : (mode == MODE_TORUS ? launch_tile<MODE_TORUS, EPI_TOPK_LARGE>(a, pl, st)
+                                     : (mode == MODE_PROJ ? launch_tile<MODE_PROJ, EPI_TOPK_LARGE>(a, pl, st)
+                                                          : launch_tile<MODE_DOT, EPI_TOPK_LARGE>(a, pl, st))))
+      return e;
+    int64_t P = 1;
+    while (P < k) P <<= 1;
+    const size_t smem = P <= SORT_SM ? (size_t)P * 8 : 0;
+    KGE_CUDA(cudaFuncSetAttribute(topk_merge_large_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)(SORT_SM * 8)));
+    topk_merge_large_kernel<<<(unsigned)n, 256, smem, st>>>(a.part_keys, pl.n_splits, k, a.buf_cap, P, ids_out,
+                                                            scores_out);
+    KGE_LAUNCH_CHECK();
+    return 0;
+  }
   if (int e = mode == MODE_DIST ? launch_tile<MODE_DIST, EPI_TOPK>(a, pl, st)
                                 : (mode == MODE_TORUS ? launch_tile<MODE_TORUS, EPI_TOPK>(a, pl, st)
                                    : (mode == MODE_PROJ ? launch_tile<MODE_PROJ, EPI_TOPK>(a, pl, st)
@@ -1258,11 +1551,21 @@ extern "C" int kge_topk_hits(const int64_t* ids, int64_t n, int32_t k, const int
 }
 
 extern "C" int kge_topk_metric_sums(const int32_t* rec_topk, int64_t n, int32_t k, double* sums, kge_stream_t stream) {
-  KGE_REQUIRE(n >= 0 && k >= 1 && k <= 128, KGE_E_ARG, "bad n / k");
+  KGE_REQUIRE(n >= 0 && k >= 1, KGE_E_ARG, "bad n / k");
   if (n == 0) return 0;
   KGE_REQUIRE(rec_topk && sums, KGE_E_ARG, "NULL argument");
   int64_t g = (n + 255) / 256;
   const int64_t cap = (int64_t)kge_num_sms() * 4;
+  if (k > KMAX) {
+    const int64_t n_win = (k + MW - 1) / MW;
+    // about as many CTAs in all as the k <= KMAX launch (each one takes a window)
+    int64_t gx = (g < cap ? g : cap) / n_win;
+    if (gx < 1) gx = 1;
+    const dim3 grid((unsigned)gx, (unsigned)(n_win < 65535 ? n_win : 65535));
+    topk_metric_sums_window_kernel<<<grid, 256, (size_t)8 * 5 * MW * 8, (cudaStream_t)stream>>>(rec_topk, n, k, sums);
+    KGE_LAUNCH_CHECK();
+    return 0;
+  }
   topk_metric_sums_kernel<<<(unsigned)(g < cap ? g : cap), 256, (size_t)8 * 5 * k * 8, (cudaStream_t)stream>>>(rec_topk, n, k,
                                                                                                          sums);
   KGE_LAUNCH_CHECK();

@@ -7,7 +7,7 @@
 
 namespace {
 
-constexpr int KMAX = 128;  // largest supported k
+constexpr int KMAX = 128;  // largest k of the sorted-list epilogue (warp_insert); larger k take score.cu's buffers
 
 __device__ __forceinline__ uint64_t make_key(float score, uint32_t id) {
   uint32_t b = __float_as_uint(score);

@@ -55,6 +55,10 @@ except Exception:  # pragma: no cover - exercised on boxes without hopwise
         LISTWISE = 3
 
 
+TOPK_LIST_MAX = 128                 # largest k of the sorted-list top-k epilogue; larger k take per-row buffers
+TOPK_WORKSPACE_BUDGET = 2 << 30     # default workspace bound of a k > TOPK_LIST_MAX full_sort_topk call (bytes)
+
+
 def _cfg_get(config, key, default=None):
     try:
         if key in config:
@@ -695,23 +699,37 @@ class FusedKGEModel(KnowledgeRecommender):
         return view
 
     # ------------------------------------------------------------------ fused full-sort top-k
-    def _topk_exact(self, m, users, k, hist_off, hist_items, mask_pad, ids, scores, rels=None, n_targets=None):
+    def _topk_exact(self, m, users, k, hist_off, hist_items, mask_pad, ids, scores, rels=None, n_targets=None,
+                    workspace_budget=TOPK_WORKSPACE_BUDGET):
         lib = _abi.lib()
         n = users.numel()
         n_targets = self.n_items if n_targets is None else n_targets
         head_is_user = 1 if rels is None else 0
-        need = lib.kge_full_sort_topk_workspace_bytes(C.byref(m), n, n_targets, k)
-        if need < 0:
-            raise _abi.KgeError(f"kge_full_sort_topk: unsupported shape (k={k}, d={self.embedding_size})")
-        ws = torch.empty(max(need, 8), dtype=torch.uint8, device=users.device)
-        _abi.check(
-            lib.kge_full_sort_topk(
-                C.byref(m), users.data_ptr(), _abi.ptr(rels), n, head_is_user, n_targets, _abi.ptr(hist_off),
-                _abi.ptr(hist_items), 1 if mask_pad else 0, k, ids.data_ptr(), _abi.ptr(scores), ws.data_ptr(), ws.numel(),
-                _abi.stream_ptr(),
-            ),
-            "kge_full_sort_topk",
-        )
+
+        def need(rows):
+            b = lib.kge_full_sort_topk_workspace_bytes(C.byref(m), rows, n_targets, k)
+            if b < 0:
+                raise _abi.KgeError(f"kge_full_sort_topk: unsupported shape (k={k}, d={self.embedding_size})")
+            return b
+
+        # k > TOPK_LIST_MAX keeps a buffer of about 2k keys per row and target split in the workspace: the rows go
+        # in chunks that keep it under the budget (the result does not depend on the chunking)
+        chunk = max(n, 1)
+        if k > TOPK_LIST_MAX:
+            while chunk > 1 and need(chunk) > workspace_budget:
+                chunk = (chunk + 1) // 2
+        bounds = [(s, min(n, s + chunk)) for s in range(0, n, chunk)] or [(0, 0)]
+        ws = torch.empty(max(max(need(e - s) for s, e in bounds), 8), dtype=torch.uint8, device=users.device)
+        for s, e in bounds:
+            _abi.check(
+                lib.kge_full_sort_topk(
+                    C.byref(m), _abi.ptr(users[s:e]), _abi.ptr(None if rels is None else rels[s:e]), e - s,
+                    head_is_user, n_targets, _abi.ptr(None if hist_off is None else hist_off[s : e + 1]),
+                    _abi.ptr(hist_items), 1 if mask_pad else 0, k, _abi.ptr(ids[s:e]),
+                    _abi.ptr(None if scores is None else scores[s:e]), ws.data_ptr(), ws.numel(), _abi.stream_ptr(),
+                ),
+                "kge_full_sort_topk",
+            )
 
     @staticmethod
     def _mma_shape() -> int:
@@ -766,15 +784,16 @@ class FusedKGEModel(KnowledgeRecommender):
         return self._mma_total + self._mma_last_fallback_rows
 
     def full_sort_topk_kg(self, head_ids, relation_ids, k: int, hist_off=None, hist_items=None, mask_pad: bool = True,
-                          return_scores: bool = True, path: str = "auto"):
+                          return_scores: bool = True, path: str = "auto", workspace_budget: int = TOPK_WORKSPACE_BUDGET):
         """Link-prediction twin of full_sort_topk: full_sort_predict_kg (transe.py:139-154, distmult.py:135-146,
         rotate.py:192-220, complex.py:192-219) over all entities with a relation per row, the same masking
         (trainer.py:731-734: entity 0 and the known tails in `hist`) and top-k (Collector_KG, collector.py:252-261)."""
         return self.full_sort_topk(head_ids, k, hist_off, hist_items, mask_pad, return_scores, path,
-                                   relation_ids=relation_ids)
+                                   relation_ids=relation_ids, workspace_budget=workspace_budget)
 
     def full_sort_topk(self, user_ids, k: int, hist_off=None, hist_items=None, mask_pad: bool = True,
-                       return_scores: bool = True, path: str = "auto", _debug_scores: bool = False, relation_ids=None):
+                       return_scores: bool = True, path: str = "auto", _debug_scores: bool = False, relation_ids=None,
+                       workspace_budget: int = TOPK_WORKSPACE_BUDGET):
         """Fused full_sort_predict + trainer masking + top-k (trainer.py:716-735, collector.py:176-177).
 
         With ``relation_ids`` the rows are (head entity, relation) queries scored against every entity
@@ -785,6 +804,10 @@ class FusedKGEModel(KnowledgeRecommender):
         ordered by (score desc, id asc).  ``path``: "cuda" = fp32 CUDA-core kernel, "mma" = tcgen05
         filter + exact fp32 re-score (same results), "auto" = "mma" where it is supported and the
         item set is large enough to pay for the operand image.
+
+        Any ``1 <= k <= n_targets`` is taken; the tensor cores serve k <= 32 only.  Above k = 128 the kernel keeps
+        a buffer of about 2k keys per row and target split in a workspace, and the rows are processed in chunks
+        that keep it under ``workspace_budget`` bytes (the result does not depend on the chunking).
         """
         device = self._check_ready()
         self.flush()
@@ -806,7 +829,8 @@ class FusedKGEModel(KnowledgeRecommender):
             raise ValueError(path)
         use_mma = path == "mma" or (path == "auto" and n_targets >= 8192 and n >= 64 and self._mma_supported(k, n_targets))
         if not use_mma or n == 0:
-            self._topk_exact(m, users, k, hist_off, hist_items, mask_pad, ids, scores, rels, n_targets)
+            self._topk_exact(m, users, k, hist_off, hist_items, mask_pad, ids, scores, rels, n_targets,
+                             workspace_budget)
             return ids, scores
         lib = _abi.lib()
         shape = self._mma_shape()
@@ -1045,13 +1069,15 @@ class TransH(FusedKGEModel):
         return view.full_sort_predict({self.USER_ID: idx})
 
     def full_sort_topk(self, user_ids, k, hist_off=None, hist_items=None, mask_pad=True, return_scores=True,
-                       path="auto", _debug_scores=False, relation_ids=None):
+                       path="auto", _debug_scores=False, relation_ids=None, workspace_budget=TOPK_WORKSPACE_BUDGET):
         if relation_ids is not None:
             raise NotImplementedError("the reference TransH has no KG scoring entry points (transh.py)")
         if self.n_items < self.VIEW_MIN_ITEMS:
-            return super().full_sort_topk(user_ids, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores)
+            return super().full_sort_topk(user_ids, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores,
+                                          workspace_budget=workspace_budget)
         view, idx = self._rec_view(user_ids)
-        return view.full_sort_topk(idx, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores)
+        return view.full_sort_topk(idx, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores,
+                                   workspace_budget=workspace_budget)
 
     def full_sort_rank(self, query_ids, pos_off, pos_items, hist_off=None, hist_items=None, mask_pad=True,
                        relation_ids=None):
@@ -1148,11 +1174,12 @@ class TransD(FusedKGEModel):
                                   "relation per row over all tails (transd.py:192-217); not built")
 
     def full_sort_topk(self, user_ids, k, hist_off=None, hist_items=None, mask_pad=True, return_scores=True,
-                       path="auto", _debug_scores=False, relation_ids=None):
+                       path="auto", _debug_scores=False, relation_ids=None, workspace_budget=TOPK_WORKSPACE_BUDGET):
         if relation_ids is not None:
             raise NotImplementedError("TransD scores users against items only (see full_sort_predict_kg)")
         view, idx = self._rec_view(user_ids)
-        return view.full_sort_topk(idx, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores)
+        return view.full_sort_topk(idx, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores,
+                                   workspace_budget=workspace_budget)
 
     def full_sort_rank(self, query_ids, pos_off, pos_items, hist_off=None, hist_items=None, mask_pad=True,
                        relation_ids=None):

@@ -30,8 +30,9 @@ checkpoints, early stopping, logging are inherited unchanged) and overrides only
                             ``rec.meanrank`` rows, from the exact full-catalogue ranks of the positives -- handed to
                             the reference ``Evaluator`` unchanged, so the metric dictionary is the reference's own.
                             Anything the fused kernels do not cover (sampled evaluation, sequential loaders, the
-                            labelled value metrics that read ``rec.score`` / ``data.label``, k > 128) goes through
-                            the inherited dense path.
+                            labelled value metrics that read ``rec.score`` / ``data.label``) goes through the
+                            inherited dense path.  Any cutoff is covered: above k = 128 the fused top-k keeps
+                            per-row buffers in a workspace instead of sorted lists in shared memory.
 
 ``install()`` registers the classes with hopwise's own factories, so ``run_hopwise(model="TransE", ...)`` and the
 ``hopwise train`` CLI pick them up without edits: ``get_model`` (utils/utils.py:65-98) resolves
@@ -71,7 +72,6 @@ from hopwise.utils import InputType as _InputType, ModelType as _ModelType  # no
 _rec.KnowledgeRecommender.type = _ModelType.KNOWLEDGE
 _rec.FusedKGEModel.input_type = _InputType.PAIRWISE
 
-KMAX_FUSED = 128                 # largest k of kge_full_sort_topk
 DEFAULT_USER_BLOCK = 148 * 512   # users per fused call: one full wave of the tensor-core sweep
 
 
@@ -166,7 +166,7 @@ class FusedKGTrainer(KGTrainer):
         reg = collector.register
         if any(reg.need(key) for key in ("rec.score", "data.label")):
             return None   # the labelled value metrics need the dense score rows
-        if max(collector.topk) > KMAX_FUSED or torch.device(self.device).type != "cuda":
+        if torch.device(self.device).type != "cuda":
             return None
         plan = eval_data.__dict__.get("_kge_fused_plan")
         if plan is not None and plan["task"] == task and plan["device"] == str(self.device):

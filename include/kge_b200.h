@@ -239,8 +239,11 @@ int kge_full_sort_scores(const kge_model_t* model, const int64_t* heads, const i
  * hist_items sorted ascending per row; both NULL = no history).  mask_first != 0 masks target 0
  * (the [PAD] item).  Order: score descending, id ascending (masked targets, score -inf, rank
  * last and enter only when a row has fewer than k unmasked targets).
+ * Any 1 <= k <= n_targets (k > n_targets: KGE_E_ARG).  Up to k = 128 each row keeps a sorted
+ * list in shared memory; above, a buffer of about 2k keys per row and target split in the
+ * workspace, so the workspace grows with n * k.
  * Outputs ids_out[n,k] (int64), scores_out[n,k] (fp32, may be NULL).  workspace: device
- * scratch of kge_full_sort_topk_workspace_bytes(model, n, n_targets, k) bytes. */
+ * scratch of kge_full_sort_topk_workspace_bytes(model, n, n_targets, k) bytes (-1: unsupported). */
 int64_t kge_full_sort_topk_workspace_bytes(const kge_model_t* model, int64_t n, int64_t n_targets, int32_t k);
 int kge_full_sort_topk(const kge_model_t* model, const int64_t* heads, const int64_t* rels, int64_t n,
                        int head_is_user, int64_t n_targets, const int64_t* hist_off, const int64_t* hist_items,
@@ -294,12 +297,14 @@ int kge_full_sort_topk_mma(const kge_model_t* model, const int64_t* heads, const
                            float* debug_scores, int32_t shape, kge_stream_t stream);
 
 /* kge_topk_hits: collector.py:178-183 without the [n, I] pos_matrix: out[n, k+1] int32 =
- * hit flags of ids[n,k] against the positives CSR (pos_off[n+1], pos_items sorted) then pos_len. */
+ * hit flags of ids[n,k] against the positives CSR (pos_off[n+1], pos_items sorted) then pos_len.
+ * Any k >= 1. */
 int kge_topk_hits(const int64_t* ids, int64_t n, int32_t k, const int64_t* pos_off, const int64_t* pos_items,
                   int32_t* out, kge_stream_t stream);
 
 /* kge_topk_metric_sums: metrics.py:67-69,93-101,164-165,191-207,231-232 summed over users:
- * sums[5*k] float64 = per-cutoff sums of recall, mrr, ndcg, hit, precision (caller zeroes). */
+ * sums[5*k] float64 = per-cutoff sums of recall, mrr, ndcg, hit, precision (caller zeroes).
+ * Any k >= 1. */
 int kge_topk_metric_sums(const int32_t* rec_topk, int64_t n, int32_t k, double* sums, kge_stream_t stream);
 
 /* ---- batch assembly ------------------------------------------------------------------------
