@@ -7,12 +7,13 @@
 //   trainer/trainer.py:716-735                     (scores[:, 0] = -inf; scores[history] = -inf)
 //   evaluator/collector.py:176-177                 (torch.topk over [n, I])
 //
-// All four scorers are "transform the (head, relation) pair into one query vector q of
+// All five scorers are "transform the (head, relation) pair into one query vector q of
 // Kdim = parts*d floats, then reduce against the target row t":
 //   TransE   q = h + r                      score = -||q - t||
 //   RotatE   q = rot(h, theta) (re | im)    score = margin - ||q - t||   (one L2 norm, rotate.py:61-69)
 //   DistMult q = h * r                      score = q . t
 //   ComplEx  q = (hr*rr | hi*rr + hr*ri - hi*ri)   score = q . t        (complex.py:53-62 as written)
+//   TorusE   q = frac(h) + frac(r)          score = -4 * sum(min(x^2, 1 - x^2)), x = q - frac(t)
 // so one tile kernel serves them all: a CTA owns BU=32 query rows (q kept in shared memory for
 // the whole sweep) and streams target tiles of BT=128 rows through shared memory in K-chunks
 // of 32 floats; each thread accumulates a 4x4 register block.  The epilogue either stores
@@ -21,6 +22,8 @@
 // matrix never exists (800 GB at 1M x 200k).  Order: score descending, id ascending.  A third
 // epilogue counts, for listed targets (the positives), the targets scoring above and equal to
 // them over the whole masked row: the exact ranks GAUC reads (collector.py's rec.meanrank).
+// TransH and TransD have no scorer here: transh_project_kernel / transd_project_kernel write projected rows, which
+// the caller scores as TransE (check_score_model refuses both model kinds).
 #include <math.h>
 
 #include "common.cuh"
@@ -39,7 +42,7 @@ template <int MODEL, int VEC, int G, int NCH>
 __global__ void __launch_bounds__(256) predict_kernel(const ScoreArgs a, float* __restrict__ out) {
   constexpr int E = VEC * NCH;
   constexpr int PH = (MODEL == KGE_ROTATE || MODEL == KGE_COMPLEX) ? 2 : 1;
-  constexpr int PR = (MODEL == KGE_COMPLEX || MODEL == KGE_TRANSH) ? 2 : 1;
+  constexpr int PR = MODEL == KGE_COMPLEX ? 2 : 1;
   const int d = a.m.d;
   const int gl = (threadIdx.x & 31) % G;
   const int groups_per_cta = blockDim.x / G;
@@ -62,18 +65,6 @@ __global__ void __launch_bounds__(256) predict_kernel(const ScoreArgs a, float* 
 #pragma unroll
       for (int e = 0; e < E; ++e) {
         const float x = h[0][e] + r[0][e] - t[0][e];
-        s += x * x;
-      }
-      s = -sqrtf(group_sum<G>(s));
-    } else if (MODEL == KGE_TRANSH) {   // transh.py:53-58, 73-74: project head and tail, then TransE's norm
-      float sw = 0.f;
-#pragma unroll
-      for (int e = 0; e < E; ++e) sw += r[1][e];
-      sw = group_sum<G>(sw);
-#pragma unroll
-      for (int e = 0; e < E; ++e) {
-        const float c = 1.f - sw * r[1][e];
-        const float x = (h[0][e] * c + r[0][e]) - t[0][e] * c;
         s += x * x;
       }
       s = -sqrtf(group_sum<G>(s));
@@ -306,24 +297,23 @@ __device__ __forceinline__ void block_bitonic_sort_desc(uint64_t* buf, int64_t P
     }
 }
 
-__device__ __forceinline__ void build_queries(const ScoreArgs& a, const int64_t* rowid, int nrows, int kpad, float* Qs,
-                                              const float* proj = nullptr) {
+__device__ __forceinline__ void build_queries(const ScoreArgs& a, const int64_t* rowid, int nrows, int kpad, float* Qs) {
   const int d = a.m.d;
   const int parts = (a.m.model == KGE_ROTATE || a.m.model == KGE_COMPLEX) ? 2 : 1;
   const int qstride = parts * kpad;
   for (int idx = threadIdx.x; idx < BU * kpad; idx += blockDim.x) {
     const int u = idx / kpad, c = idx - u * kpad;
     float q0 = 0.f, q1 = 0.f;
-    if (u < nrows && c < d) query_value(a, rowid[u], c, q0, q1, proj);
+    if (u < nrows && c < d) query_value(a, rowid[u], c, q0, q1);
     Qs[u * qstride + c] = q0;
     if (parts == 2) Qs[u * qstride + kpad + c] = q1;
   }
 }
 
 // Stage target rows [t0, t0+BT) x columns [c0, c0+KC) of one part into Ts (zero padded).
-template <bool FRAC, bool PROJ>
+template <bool FRAC>
 __device__ __forceinline__ void load_target_chunk(const float* __restrict__ W, int d, int64_t n_targets, int64_t t0,
-                                                  int c0, float* Ts, const float* Cs) {
+                                                  int c0, float* Ts) {
   if ((d & 3) == 0) {
     // 8 float4 per row chunk; consecutive lanes take consecutive rows -> conflict-free STS.128
     for (int idx = threadIdx.x; idx < BT * (KC / 4); idx += blockDim.x) {
@@ -333,9 +323,6 @@ __device__ __forceinline__ void load_target_chunk(const float* __restrict__ W, i
       const int64_t t = t0 + j;
       if (t < n_targets && c < d) v = __ldg(reinterpret_cast<const float4*>(W + t * d + c));
       if (FRAC) v = make_float4(fracf_signed(v.x), fracf_signed(v.y), fracf_signed(v.z), fracf_signed(v.w));
-      if (PROJ) {   // (c < kpad always; Cs is zero beyond d like v)
-        v = make_float4(v.x * Cs[c], v.y * Cs[c + 1], v.z * Cs[c + 2], v.w * Cs[c + 3]);
-      }
       *reinterpret_cast<float4*>(Ts + j * TS + q * 4) = v;
     }
   } else {
@@ -344,7 +331,7 @@ __device__ __forceinline__ void load_target_chunk(const float* __restrict__ W, i
       const int c = c0 + q;
       const int64_t t = t0 + j;
       const float v = (t < n_targets && c < d) ? __ldg(W + t * d + c) : 0.f;
-      Ts[j * TS + q] = FRAC ? fracf_signed(v) : (PROJ ? v * Cs[c] : v);
+      Ts[j * TS + q] = FRAC ? fracf_signed(v) : v;
     }
   }
 }
@@ -353,7 +340,7 @@ __device__ __forceinline__ void load_target_chunk(const float* __restrict__ W, i
 // The rank epilogue asks for two CTAs per SM (128 registers): under the compiler's default budget it spills.
 template <int MODE, int EPI>
 __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_TOPK_LARGE) ? 2 : 0) fullsort_tile_kernel(const TileArgs a) {
-  constexpr bool DIST = MODE == MODE_DIST || MODE == MODE_PROJ;
+  constexpr bool DIST = MODE == MODE_DIST;
   constexpr bool TOPK = EPI == EPI_TOPK, RANK = EPI == EPI_RANK, LARGE = EPI == EPI_TOPK_LARGE;
   constexpr bool SEL = TOPK || LARGE;         // a top-k epilogue: candidate keys staged per tile
   constexpr bool MASKED = EPI != EPI_DENSE;   // the trainer's masking: column 0 and the history -> -inf
@@ -376,15 +363,13 @@ __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_T
   int* llen = cnt + (SEL ? BU : 0);                                         // [BU] list / buffer length
   int64_t* cursor = reinterpret_cast<int64_t*>(llen + (SEL ? BU : 0));      // [BU] (8-byte aligned by layout)
   int64_t* rowid = cursor + (MASKED ? BU : 0);                              // [BU] query row of each slot
-  float* Cs = reinterpret_cast<float*>(rowid + BU);                         // [kpad] projection factor (MODE_PROJ)
-  // rank only (kpad is a multiple of 32: rbase stays 8-byte aligned)
-  int64_t* rbase = reinterpret_cast<int64_t*>(Cs + (MODE == MODE_PROJ ? kpad : 0));  // [BU] pos_off of the row
+  // rank only
+  int64_t* rbase = rowid + BU;                                              // [BU] pos_off of the row
   float* rthr = reinterpret_cast<float*>(rbase + (RANK ? BU : 0));         // [BU][RANK_SM] sorted thresholds
   uint32_t* rcnt = reinterpret_cast<uint32_t*>(rthr + (RANK ? BU * RANK_SM : 0));  // [BU][2 * RANK_SM] bins
   float* rlo = reinterpret_cast<float*>(rcnt + (RANK ? BU * 2 * RANK_SM : 0));    // [BU] lowest finite threshold
   int* rm = reinterpret_cast<int*>(rlo + (RANK ? BU : 0));                        // [BU] thresholds of the row
   if (RANK && a.pos_off[a.s.n] > a.rank_cap) return;   // (the workspace was sized for fewer positives)
-  if (MODE == MODE_PROJ) proj_factor<TILE_THREADS>(a.s, kpad, Cs);
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int tu = warp;  // users 4*tu .. 4*tu+3
@@ -400,7 +385,7 @@ __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_T
   for (int u = threadIdx.x; u < BU; u += blockDim.x)
     rowid[u] = u < nrows ? (a.row_map ? (int64_t)__ldg(a.row_map + row0 + u) : row0 + u) : 0;
   __syncthreads();
-  build_queries(a.s, rowid, nrows, kpad, Qs, MODE == MODE_PROJ ? Cs : nullptr);
+  build_queries(a.s, rowid, nrows, kpad, Qs);
   if (RANK) {
     for (int u = threadIdx.x; u < BU; u += blockDim.x) {
       int64_t base = 0, m = 0;
@@ -483,7 +468,7 @@ __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_T
       const float* W = a.s.m.entity.w[p];
       for (int c0 = 0; c0 < kpad; c0 += KC) {
         __syncthreads();  // previous chunk consumed
-        load_target_chunk<MODE == MODE_TORUS, MODE == MODE_PROJ>(W, d, a.n_targets, t0, c0, Ts, Cs);
+        load_target_chunk<MODE == MODE_TORUS>(W, d, a.n_targets, t0, c0, Ts);
         __syncthreads();
         const float* qbase = Qs + (4 * tu) * qstride + p * kpad + c0;
 #pragma unroll
@@ -928,7 +913,6 @@ __global__ void __launch_bounds__(256) topk_metric_sums_window_kernel(const int3
 struct RankPrep {
   ScoreArgs s;
   int64_t n_targets;
-  int kpad;
   const int64_t* hist_off;
   const int64_t* hist_items;
   int mask_first;
@@ -948,20 +932,18 @@ struct RankPrep {
 // which is cheap for evaluation's few positives per user and stays correct for any number.
 template <int MODE>
 __global__ void __launch_bounds__(TILE_THREADS) rank_thresholds_kernel(const RankPrep a) {
-  constexpr bool DIST = MODE == MODE_DIST || MODE == MODE_PROJ;
+  constexpr bool DIST = MODE == MODE_DIST;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int parts = (a.s.m.model == KGE_ROTATE || a.s.m.model == KGE_COMPLEX) ? 2 : 1;
   const int d = a.s.m.d;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = TILE_THREADS / 32;
-  float* Cs = reinterpret_cast<float*>(smem_raw);   // [kpad] projection factor (MODE_PROJ)
-  float* q = Cs + a.kpad + warp * parts * d;         // [parts * d] this warp's query row
-  if (a.pos_off[a.s.n] > a.cap) return;              // (the workspace was sized for fewer positives)
-  if (MODE == MODE_PROJ) proj_factor<TILE_THREADS>(a.s, a.kpad, Cs);
+  float* q = reinterpret_cast<float*>(smem_raw) + warp * parts * d;   // [parts * d] this warp's query row
+  if (a.pos_off[a.s.n] > a.cap) return;                                // (the workspace was sized for fewer positives)
   const float margin = (a.s.m.model == KGE_ROTATE) ? a.s.m.margin : 0.f;
   for (int64_t row = (int64_t)blockIdx.x * warps + warp; row < a.s.n; row += (int64_t)gridDim.x * warps) {
     for (int c = lane; c < d; c += 32) {
       float q0, q1;
-      query_value(a.s, row, c, q0, q1, Cs);
+      query_value(a.s, row, c, q0, q1);
       q[c] = q0;
       if (parts == 2) q[d + c] = q1;
     }
@@ -983,7 +965,7 @@ __global__ void __launch_bounds__(TILE_THREADS) rank_thresholds_kernel(const Ran
       float sc = -INFINITY;
       if (!masked) {
         float acc = 0.f;
-        for (int p = 0; p < parts; ++p) acc = exact_chain<MODE>(q + p * d, a.s.m.entity.w[p] + j * d, d, acc, Cs);
+        for (int p = 0; p < parts; ++p) acc = exact_chain<MODE>(q + p * d, a.s.m.entity.w[p] + j * d, d, acc);
         sc = DIST ? (margin - sqrtf(acc)) : (MODE == MODE_TORUS ? -(4.f * acc) : acc);
         lo = fminf(lo, sc);
       }
@@ -1088,9 +1070,13 @@ RankLayout rank_layout(int64_t n, int64_t n_pos) {
 
 int check_score_model(const kge_model_t* m) {
   KGE_REQUIRE(m, KGE_E_ARG, "model is NULL");
-  KGE_REQUIRE(m->model >= KGE_TRANSE && m->model <= KGE_TRANSH, KGE_E_ARG, "unknown model kind %d", m->model);
+  KGE_REQUIRE(m->model != KGE_TRANSH, KGE_E_UNSUPPORTED,
+              "TransH scores through kge_transh_project and the KGE_TRANSE scoring entry points");
+  KGE_REQUIRE(m->model != KGE_TRANSD, KGE_E_UNSUPPORTED,
+              "TransD scores through kge_transd_project and the KGE_TRANSE scoring entry points");
+  KGE_REQUIRE(m->model >= KGE_TRANSE && m->model <= KGE_TORUSE, KGE_E_ARG, "unknown model kind %d", m->model);
   const int ph = (m->model == KGE_ROTATE || m->model == KGE_COMPLEX) ? 2 : 1;
-  const int pr = (m->model == KGE_COMPLEX || m->model == KGE_TRANSH) ? 2 : 1;
+  const int pr = m->model == KGE_COMPLEX ? 2 : 1;
   for (int p = 0; p < ph; ++p) KGE_REQUIRE(m->user.w[p] && m->entity.w[p], KGE_E_ARG, "NULL weight table");
   for (int p = 0; p < pr; ++p) KGE_REQUIRE(m->relation.w[p], KGE_E_ARG, "NULL relation table");
   KGE_REQUIRE(m->d >= 1, KGE_E_UNSUPPORTED, "embedding_size %d unsupported", m->d);
@@ -1113,7 +1099,6 @@ int plan_tiles(const kge_model_t* m, int64_t n, int64_t n_targets, int k, int ep
   if (epi == EPI_RANK)   // maskbits, cursor | rbase, rthr, rcnt, rlo, rm
     smem += BU * (BT / 32) * 4 + BU * 8 + BU * 8 + (size_t)BU * RANK_SM * 4 * 3 + BU * 4 * 2;
   smem += BU * 8;   // rowid
-  if (m->model == KGE_TRANSH) smem += (size_t)pl.kpad * 4;   // projection factor
   pl.smem = smem;
   KGE_REQUIRE(smem <= 220 * 1024, KGE_E_UNSUPPORTED, "embedding_size %d needs %zu bytes of shared memory", m->d, smem);
   pl.n_blocks = (n + BU - 1) / BU;
@@ -1140,7 +1125,6 @@ int plan_tiles(const kge_model_t* m, int64_t n, int64_t n_targets, int k, int ep
 
 int tile_mode(int model) {
   if (model == KGE_TORUSE) return MODE_TORUS;
-  if (model == KGE_TRANSH) return MODE_PROJ;
   return (model == KGE_TRANSE || model == KGE_ROTATE) ? MODE_DIST : MODE_DOT;
 }
 
@@ -1173,7 +1157,6 @@ extern "C" int kge_predict(const kge_model_t* model, const int64_t* heads, const
     case KGE_DISTMULT: predict_kernel<KGE_DISTMULT, V, G, N><<<grid, threads, 0, st>>>(a, out); break; \
     case KGE_ROTATE: predict_kernel<KGE_ROTATE, V, G, N><<<grid, threads, 0, st>>>(a, out); break;     \
     case KGE_TORUSE: predict_kernel<KGE_TORUSE, V, G, N><<<grid, threads, 0, st>>>(a, out); break;     \
-    case KGE_TRANSH: predict_kernel<KGE_TRANSH, V, G, N><<<grid, threads, 0, st>>>(a, out); break;     \
     default: predict_kernel<KGE_COMPLEX, V, G, N><<<grid, threads, 0, st>>>(a, out); break;            \
   }
   KGE_DISPATCH_ROWCFG(c, CALL);
@@ -1236,8 +1219,6 @@ static int launch_tile(const TileArgs& a, const TilePlan& pl, cudaStream_t st) {
 extern "C" int kge_full_sort_scores(const kge_model_t* model, const int64_t* heads, const int64_t* rels, int64_t n,
                                     int head_is_user, int64_t n_targets, float* out, kge_stream_t stream) {
   if (int e = check_score_model(model)) return e;
-  KGE_REQUIRE(model->model != KGE_TRANSH || rels == nullptr, KGE_E_UNSUPPORTED,
-              "TransH full-sort takes the user->item relation only (transh.py:125-145; no KG scoring in the reference)");
   KGE_REQUIRE(n >= 0 && n_targets >= 1 && n_targets <= model->entity.rows, KGE_E_ARG, "bad n / n_targets");
   if (n == 0) return 0;
   KGE_REQUIRE(heads && out, KGE_E_ARG, "NULL heads / out");
@@ -1259,7 +1240,6 @@ extern "C" int kge_full_sort_scores(const kge_model_t* model, const int64_t* hea
   switch (tile_mode(model->model)) {
     case MODE_DIST: return launch_tile<MODE_DIST, EPI_DENSE>(a, pl, (cudaStream_t)stream);
     case MODE_TORUS: return launch_tile<MODE_TORUS, EPI_DENSE>(a, pl, (cudaStream_t)stream);
-    case MODE_PROJ: return launch_tile<MODE_PROJ, EPI_DENSE>(a, pl, (cudaStream_t)stream);
     default: return launch_tile<MODE_DOT, EPI_DENSE>(a, pl, (cudaStream_t)stream);
   }
 }
@@ -1281,8 +1261,6 @@ extern "C" int kge_full_sort_topk(const kge_model_t* model, const int64_t* heads
                                   const int64_t* hist_items, int mask_first, int32_t k, int64_t* ids_out,
                                   float* scores_out, void* workspace, int64_t workspace_bytes, kge_stream_t stream) {
   if (int e = check_score_model(model)) return e;
-  KGE_REQUIRE(model->model != KGE_TRANSH || rels == nullptr, KGE_E_UNSUPPORTED,
-              "TransH full-sort takes the user->item relation only (transh.py:125-145; no KG scoring in the reference)");
   KGE_REQUIRE(n >= 0 && n_targets >= 1 && n_targets <= model->entity.rows, KGE_E_ARG, "bad n / n_targets");
   KGE_REQUIRE(k >= 1, KGE_E_UNSUPPORTED, "k=%d below 1", k);
   KGE_REQUIRE(k <= n_targets, KGE_E_ARG, "k=%d larger than the number of targets", k);
@@ -1319,8 +1297,7 @@ extern "C" int kge_full_sort_topk(const kge_model_t* model, const int64_t* heads
     a.buf_cap = large_k_cap(k);
     if (int e = mode == MODE_DIST ? launch_tile<MODE_DIST, EPI_TOPK_LARGE>(a, pl, st)
                                   : (mode == MODE_TORUS ? launch_tile<MODE_TORUS, EPI_TOPK_LARGE>(a, pl, st)
-                                     : (mode == MODE_PROJ ? launch_tile<MODE_PROJ, EPI_TOPK_LARGE>(a, pl, st)
-                                                          : launch_tile<MODE_DOT, EPI_TOPK_LARGE>(a, pl, st))))
+                                                        : launch_tile<MODE_DOT, EPI_TOPK_LARGE>(a, pl, st)))
       return e;
     int64_t P = 1;
     while (P < k) P <<= 1;
@@ -1334,8 +1311,7 @@ extern "C" int kge_full_sort_topk(const kge_model_t* model, const int64_t* heads
   }
   if (int e = mode == MODE_DIST ? launch_tile<MODE_DIST, EPI_TOPK>(a, pl, st)
                                 : (mode == MODE_TORUS ? launch_tile<MODE_TORUS, EPI_TOPK>(a, pl, st)
-                                   : (mode == MODE_PROJ ? launch_tile<MODE_PROJ, EPI_TOPK>(a, pl, st)
-                                                        : launch_tile<MODE_DOT, EPI_TOPK>(a, pl, st))))
+                                                      : launch_tile<MODE_DOT, EPI_TOPK>(a, pl, st)))
     return e;
   const int warps = 8;
   const int64_t mg = (n + warps - 1) / warps;
@@ -1357,7 +1333,7 @@ template <int MODE>
 static int launch_rank(const RankPrep& rp, const TileArgs& a, const TilePlan& pl, int64_t* greater_out,
                        int64_t* equal_out, int64_t* n_unmasked_out, cudaStream_t st) {
   const int parts = (rp.s.m.model == KGE_ROTATE || rp.s.m.model == KGE_COMPLEX) ? 2 : 1;
-  const size_t smem = ((size_t)rp.kpad + (size_t)(TILE_THREADS / 32) * parts * rp.s.m.d) * 4;
+  const size_t smem = (size_t)(TILE_THREADS / 32) * parts * rp.s.m.d * 4;
   KGE_CUDA(cudaFuncSetAttribute(rank_thresholds_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int64_t rows_per_cta = TILE_THREADS / 32;
   int64_t g = (rp.s.n + rows_per_cta - 1) / rows_per_cta;
@@ -1379,8 +1355,6 @@ extern "C" int kge_full_sort_rank_counts(const kge_model_t* model, const int64_t
                                          int64_t* n_unmasked_out, void* workspace, int64_t workspace_bytes,
                                          kge_stream_t stream) {
   if (int e = check_score_model(model)) return e;
-  KGE_REQUIRE(model->model != KGE_TRANSH || rels == nullptr, KGE_E_UNSUPPORTED,
-              "TransH full-sort takes the user->item relation only (transh.py:125-145; no KG scoring in the reference)");
   KGE_REQUIRE(n >= 0 && n_targets >= 1 && n_targets <= model->entity.rows, KGE_E_ARG, "bad n / n_targets");
   if (n == 0) return 0;
   KGE_REQUIRE(heads && pos_off && n_unmasked_out, KGE_E_ARG, "NULL heads / pos_off / n_unmasked_out");
@@ -1407,7 +1381,6 @@ extern "C" int kge_full_sort_rank_counts(const kge_model_t* model, const int64_t
   rp.s.head_is_user = head_is_user;
   rp.s.rel_row = model->ui_relation_fullsort;
   rp.n_targets = n_targets;
-  rp.kpad = pl.kpad;
   rp.hist_off = hist_off;
   rp.hist_items = hist_items;
   rp.mask_first = mask_first;
@@ -1437,7 +1410,6 @@ extern "C" int kge_full_sort_rank_counts(const kge_model_t* model, const int64_t
   switch (tile_mode(model->model)) {
     case MODE_DIST: return launch_rank<MODE_DIST>(rp, a, pl, greater_out, equal_out, n_unmasked_out, st);
     case MODE_TORUS: return launch_rank<MODE_TORUS>(rp, a, pl, greater_out, equal_out, n_unmasked_out, st);
-    case MODE_PROJ: return launch_rank<MODE_PROJ>(rp, a, pl, greater_out, equal_out, n_unmasked_out, st);
     default: return launch_rank<MODE_DOT>(rp, a, pl, greater_out, equal_out, n_unmasked_out, st);
   }
 }
@@ -1502,8 +1474,7 @@ int kge_topk_rows_indirect(const kge_model_t* model, const int64_t* heads, const
   const int mode = tile_mode(model->model);
   auto kern = mode == MODE_DIST ? fullsort_tile_kernel<MODE_DIST, EPI_TOPK>
                                 : (mode == MODE_TORUS ? fullsort_tile_kernel<MODE_TORUS, EPI_TOPK>
-                                   : (mode == MODE_PROJ ? fullsort_tile_kernel<MODE_PROJ, EPI_TOPK>
-                                                        : fullsort_tile_kernel<MODE_DOT, EPI_TOPK>));
+                                                      : fullsort_tile_kernel<MODE_DOT, EPI_TOPK>);
   KGE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fp.tp.smem));
   const int warps = 8;
   const int64_t ra = n < FB_SPLIT_ROWS ? n : FB_SPLIT_ROWS;

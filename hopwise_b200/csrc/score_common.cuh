@@ -1,6 +1,7 @@
 // Pieces shared by the CUDA-core scoring kernels (score.cu) and the tcgen05 full-sort path
 // (mma_topk.cu): the 64-bit top-k key, the warp-cooperative sorted-list insertion and the query
-// transform q(head, relation) of the four scorers.
+// transform q(head, relation) of the five scorers.  TransH and TransD have no scorer of their own:
+// they score as TransE on rows projected by kge_transh_project / kge_transd_project.
 #pragma once
 
 #include "common.cuh"
@@ -67,10 +68,7 @@ struct ScoreArgs {
 //   RotatE   q = rot(h, theta) = (re | im) (rotate.py:61-66)
 //   ComplEx  q = (hr*rr | hi*rr + hr*ri - hi*ri)   (complex.py:53-62 regrouped by tail part)
 //   TorusE   q = frac(h) + frac(r)         (toruse.py:66-76; torch.frac keeps the sign: x - trunc(x))
-//   TransH   q = h * (1 - sum(w) * w) + r  (transh.py:53-58, 73-74; `proj` = the factor vector of the relation, built
-//                                           by the caller -- every query row shares the user->item relation)
-__device__ __forceinline__ void query_value(const ScoreArgs& a, int64_t qrow, int c, float& q0, float& q1,
-                                            const float* proj = nullptr) {
+__device__ __forceinline__ void query_value(const ScoreArgs& a, int64_t qrow, int c, float& q0, float& q1) {
   const int d = a.m.d;
   const int model = a.m.model;
   const kge_table_t& HT = a.head_is_user ? a.m.user : a.m.entity;
@@ -83,8 +81,6 @@ __device__ __forceinline__ void query_value(const ScoreArgs& a, int64_t qrow, in
     q0 = h0 + r0;
   } else if (model == KGE_TORUSE) {
     q0 = fracf_signed(h0) + fracf_signed(r0);
-  } else if (model == KGE_TRANSH) {
-    q0 = h0 * proj[c] + r0;
   } else if (model == KGE_DISTMULT) {
     q0 = h0 * r0;
   } else if (model == KGE_ROTATE) {
@@ -103,37 +99,15 @@ __device__ __forceinline__ void query_value(const ScoreArgs& a, int64_t qrow, in
 
 // How a (query, target) pair of rows is contracted -- 0 dot product, 1 squared distance (score = margin - sqrt),
 // 2 torus distance sum(min(x^2, 1 - x^2)) on frac()ed rows (score = -4 * sum).  Zero padding contributes 0 in all three.
-// 3 = mode 1 on rows projected by one relation's factor c = 1 - sum(w) * w (TransH over items: every query row takes the
-// user->item relation, so one factor vector serves the whole launch; it is built once per CTA in shared memory).
-constexpr int MODE_DOT = 0, MODE_DIST = 1, MODE_TORUS = 2, MODE_PROJ = 3;
-
-// The projection factor c = 1 - sum(w) * w of the user->item relation's hyperplane vector (relation part 1), zero
-// beyond d, into Cs[kpad].  Every thread of the block (THREADS of them) calls it; the sum's order depends on THREADS,
-// so every kernel whose scores must agree bit for bit uses the same block size.
-template <int THREADS>
-__device__ __forceinline__ void proj_factor(const ScoreArgs& a, int kpad, float* Cs) {
-  __shared__ float s_part[THREADS / 32];
-  const int d = a.m.d;
-  const float* wv = a.m.relation.w[1] + (int64_t)a.rel_row * d;
-  float part = 0.f;
-  for (int c = threadIdx.x; c < d; c += blockDim.x) part += __ldg(wv + c);
-  part = warp_sum(part);
-  if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = part;
-  __syncthreads();
-  float sw = 0.f;
-  for (int i = 0; i < THREADS / 32; ++i) sw += s_part[i];
-  for (int c = threadIdx.x; c < kpad; c += blockDim.x) Cs[c] = c < d ? 1.f - sw * __ldg(wv + c) : 0.f;
-  __syncthreads();
-}
+constexpr int MODE_DOT = 0, MODE_DIST = 1, MODE_TORUS = 2;
 
 // The sequential fp32 chain of score.cu's tile kernel over one part of one (query, target) pair: columns ascending,
 // one accumulation per column, continuing from `acc`.  `qp` = the part's d query values, `t` = the target's row of
-// that part (raw: the torus frac() and the TransH factor `Cs` are applied here as the tile kernel applies them when
-// it stages targets).  Scores built on it are bit-identical to the tile kernel's.  The loads of a 64-column block
-// are all issued before the chain consumes them.
+// that part (raw: the torus frac() is applied here as the tile kernel applies it when it stages targets).  Scores
+// built on it are bit-identical to the tile kernel's.  The loads of a 64-column block are all issued before the chain
+// consumes them.
 template <int MODE>
-__device__ __forceinline__ float exact_chain(const float* qp, const float* __restrict__ t, int d, float acc,
-                                             const float* Cs = nullptr) {
+__device__ __forceinline__ float exact_chain(const float* qp, const float* __restrict__ t, int d, float acc) {
   if ((d & 3) == 0) {
     for (int c0 = 0; c0 < d; c0 += 64) {
       float4 tv[16];
@@ -147,9 +121,6 @@ __device__ __forceinline__ float exact_chain(const float* qp, const float* __res
           const float4 qv = *reinterpret_cast<const float4*>(qp + c);
           float4 v = tv[x];
           if (MODE == MODE_TORUS) v = make_float4(fracf_signed(v.x), fracf_signed(v.y), fracf_signed(v.z), fracf_signed(v.w));
-          if (MODE == MODE_PROJ)
-            v = make_float4(__fmul_rn(v.x, Cs[c]), __fmul_rn(v.y, Cs[c + 1]), __fmul_rn(v.z, Cs[c + 2]),
-                            __fmul_rn(v.w, Cs[c + 3]));
           if (MODE == MODE_TORUS) {
             const float e0 = qv.x - v.x, e1 = qv.y - v.y, e2 = qv.z - v.z, e3 = qv.w - v.w;
             const float s0 = e0 * e0, s1 = e1 * e1, s2 = e2 * e2, s3 = e3 * e3;
@@ -157,7 +128,7 @@ __device__ __forceinline__ float exact_chain(const float* qp, const float* __res
             acc += fminf(s1, 1.f - s1);
             acc += fminf(s2, 1.f - s2);
             acc += fminf(s3, 1.f - s3);
-          } else if (MODE == MODE_DIST || MODE == MODE_PROJ) {
+          } else if (MODE == MODE_DIST) {
             const float e0 = qv.x - v.x, e1 = qv.y - v.y, e2 = qv.z - v.z, e3 = qv.w - v.w;
             acc = fmaf(e0, e0, acc);
             acc = fmaf(e1, e1, acc);
@@ -177,12 +148,11 @@ __device__ __forceinline__ float exact_chain(const float* qp, const float* __res
     for (int c = 0; c < d; ++c) {
       float v = __ldg(t + c);
       if (MODE == MODE_TORUS) v = fracf_signed(v);
-      if (MODE == MODE_PROJ) v = __fmul_rn(v, Cs[c]);
       const float e0 = qp[c] - v;
       if (MODE == MODE_TORUS) {
         const float s0 = e0 * e0;
         acc += fminf(s0, 1.f - s0);
-      } else if (MODE == MODE_DIST || MODE == MODE_PROJ) {
+      } else if (MODE == MODE_DIST) {
         acc = fmaf(e0, e0, acc);
       } else {
         acc = fmaf(qp[c], v, acc);

@@ -671,33 +671,6 @@ class FusedKGEModel(KnowledgeRecommender):
     def full_sort_predict_kg(self, interaction):
         return self._full_sort(interaction[self.HEAD_ENTITY_ID], interaction[self.RELATION_ID], False, self.n_entities)
 
-    # ------------------------------------------------------------------ projected-table scoring (TransD, TransH)
-    def _transe_view(self, users, entities):
-        """The private TransE model over projected tables: `users` [n, d] rows, `entities` [m, d] rows, the
-        relation table shared with this model."""
-        view = self.__dict__.get("_view")
-        if view is None:
-            cfg = {"USER_ID_FIELD": self.USER_ID, "ITEM_ID_FIELD": self.ITEM_ID,
-                   "NEG_PREFIX": self.NEG_ITEM_ID[: -len(self.ITEM_ID)],
-                   "ENTITY_ID_FIELD": self.ENTITY_ID, "RELATION_ID_FIELD": self.RELATION_ID,
-                   "HEAD_ENTITY_ID_FIELD": self.HEAD_ENTITY_ID, "TAIL_ENTITY_ID_FIELD": self.TAIL_ENTITY_ID,
-                   "device": self.device, "embedding_size": self.embedding_size, "margin": self.margin}
-
-            class _Shape:
-                def num(_, field):
-                    return {self.RELATION_ID: self.n_relations}.get(field, 1)
-
-            view = TransE(cfg, _Shape())
-            view.eval()
-            self.__dict__["_view"] = view   # (not a submodule: its tables are scratch, not parameters of this model)
-        with torch.no_grad():
-            view.user_embedding.weight.data = users
-            view.entity_embedding.weight.data = entities
-            view.relation_embedding.weight.data = self.relation_embedding.weight.data
-        view.n_users, view.n_items, view.n_entities = users.shape[0], entities.shape[0], entities.shape[0]
-        view.__dict__.pop("_table_params", None)
-        return view
-
     # ------------------------------------------------------------------ fused full-sort top-k
     def _topk_exact(self, m, users, k, hist_off, hist_items, mask_pad, ids, scores, rels=None, n_targets=None,
                     workspace_budget=TOPK_WORKSPACE_BUDGET):
@@ -996,18 +969,108 @@ class TorusE(FusedKGEModel):
     RELATION_TABLES = ("relation_embedding",)
 
 
-class TransH(FusedKGEModel):
+class _ProjectedKGEModel(FusedKGEModel):
+    """TransE on rows projected per relation (TransH, TransD).  Scoring composes two library calls: the subclass's
+    ``_project(family, ids)`` writes rows projected with the user->item relation, and since the projection of an
+    item does not depend on the user, the rest IS TransE on projected tables -- a private TransE view of those
+    buffers runs predict, dense full-sort, the fused top-k (tensor-core path included) and the rank counts.  The
+    projected items are cached per weight version.  Users are scored against items only: the dense and fused KG
+    full-sort entry points refuse, with the subclass's ``KG_REFUSAL`` as the reason."""
+
+    KG_REFUSAL: str = ""
+
+    def _transe_view(self, users, entities):
+        """The private TransE model over projected tables: `users` [n, d] rows, `entities` [m, d] rows, the
+        relation table shared with this model."""
+        view = self.__dict__.get("_view")
+        if view is None:
+            cfg = {"USER_ID_FIELD": self.USER_ID, "ITEM_ID_FIELD": self.ITEM_ID,
+                   "NEG_PREFIX": self.NEG_ITEM_ID[: -len(self.ITEM_ID)],
+                   "ENTITY_ID_FIELD": self.ENTITY_ID, "RELATION_ID_FIELD": self.RELATION_ID,
+                   "HEAD_ENTITY_ID_FIELD": self.HEAD_ENTITY_ID, "TAIL_ENTITY_ID_FIELD": self.TAIL_ENTITY_ID,
+                   "device": self.device, "embedding_size": self.embedding_size, "margin": self.margin}
+
+            class _Shape:
+                def num(_, field):
+                    return {self.RELATION_ID: self.n_relations}.get(field, 1)
+
+            view = TransE(cfg, _Shape())
+            view.eval()
+            self.__dict__["_view"] = view   # (not a submodule: its tables are scratch, not parameters of this model)
+        with torch.no_grad():
+            view.user_embedding.weight.data = users
+            view.entity_embedding.weight.data = entities
+            view.relation_embedding.weight.data = self.relation_embedding.weight.data
+        view.n_users, view.n_items, view.n_entities = users.shape[0], entities.shape[0], entities.shape[0]
+        view.__dict__.pop("_table_params", None)
+        return view
+
+    def _projected_items(self):
+        """Rows [0, n_items) of the entity table projected with the user->item relation, cached per weight version."""
+        tabs = self._tables(self.ENTITY_TABLES + self.RELATION_TABLES[1:])
+        key = (self._step, tuple(t.data_ptr() for t in tabs), tuple(t._version for t in tabs))
+        hit = self.__dict__.get("_items_cache")
+        if hit is None or hit[0] != key:
+            ids = torch.arange(self.n_items, device=tabs[0].device)
+            hit = (key, self._project("entity", ids))
+            self.__dict__["_items_cache"] = hit
+            view = self.__dict__.get("_view")
+            if view is not None:
+                view.invalidate_target_image()
+        return hit[1]
+
+    def invalidate_target_image(self):
+        super().invalidate_target_image()
+        self.__dict__.pop("_items_cache", None)
+
+    def _rec_view(self, user_ids):
+        view = self._transe_view(self._project("user", user_ids), self._projected_items())
+        return view, torch.arange(view.n_users, device=view.user_embedding.weight.device)
+
+    def predict(self, interaction):
+        users, items = interaction[self.USER_ID], interaction[self.ITEM_ID]
+        view = self._transe_view(self._project("user", users), self._project("entity", items))
+        view.invalidate_target_image()
+        idx = torch.arange(view.n_users, device=view.user_embedding.weight.device)
+        return view.predict({self.USER_ID: idx, self.ITEM_ID: idx})
+
+    def full_sort_predict(self, interaction):
+        view, idx = self._rec_view(interaction[self.USER_ID])
+        return view.full_sort_predict({self.USER_ID: idx})
+
+    def full_sort_predict_kg(self, interaction):
+        raise NotImplementedError(self.KG_REFUSAL)
+
+    def full_sort_topk(self, user_ids, k, hist_off=None, hist_items=None, mask_pad=True, return_scores=True,
+                       path="auto", _debug_scores=False, relation_ids=None, workspace_budget=TOPK_WORKSPACE_BUDGET):
+        if relation_ids is not None:
+            raise NotImplementedError(self.KG_REFUSAL)
+        view, idx = self._rec_view(user_ids)
+        return view.full_sort_topk(idx, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores,
+                                   workspace_budget=workspace_budget)
+
+    def full_sort_rank(self, query_ids, pos_off, pos_items, hist_off=None, hist_items=None, mask_pad=True,
+                       relation_ids=None):
+        if relation_ids is not None:
+            raise NotImplementedError(self.KG_REFUSAL)
+        view, idx = self._rec_view(query_ids)
+        return view.full_sort_rank(idx, pos_off, pos_items, hist_off, hist_items, mask_pad)
+
+
+class TransH(_ProjectedKGEModel):
     """transh.py: TransE on rows projected per relation.  The second relation table `norm_vec` holds the hyperplane
     vector w; the reference's ``project`` is ``ent - (ent * w.sum()) * w`` (transh.py:73-74), applied to head and both
     tails before TransE's TripletMarginLoss (transh.py:76-107) and norm (transh.py:53-58).  Recommendation triples
     read ``relation_embedding.weight[-1]`` but ``norm_vec(ui_relation)`` (transh.py:63, 90): the kernels take one row
     for both, so a dataset whose [UI-Relation] token is not the last relation id is refused (hopwise's datasets append
-    the token last).  The reference scores users against items only; so does this class."""
+    the token last).  The reference scores users against items only; so does this class (``kge_transh_project``
+    writes the projected rows)."""
 
     KIND = "TransH"
     USER_TABLES = ("user_embedding",)
     ENTITY_TABLES = ("entity_embedding",)
     RELATION_TABLES = ("relation_embedding", "norm_vec")
+    KG_REFUSAL = "the reference TransH has no KG scoring entry points (transh.py)"
 
     def __init__(self, config, dataset):
         super().__init__(config, dataset)
@@ -1018,15 +1081,7 @@ class TransH(FusedKGEModel):
                 "relation_embedding.weight[-1] and norm_vec(ui_relation) would name different rows (transh.py:63, 90)")
 
     def predict_kg(self, interaction):
-        raise NotImplementedError("the reference TransH has no KG scoring entry points (transh.py)")
-
-    def full_sort_predict_kg(self, interaction):
-        raise NotImplementedError("the reference TransH has no KG scoring entry points (transh.py)")
-
-    # A large item set is scored as TransE over projected tables (users and items scaled by the user->item relation's
-    # factor, `kge_transh_project`): that is the route to the tensor-core top-k.  Dense rows and top-k always take
-    # the same route, so that the top-k of a user equals the top-k of its dense row bit for bit.
-    VIEW_MIN_ITEMS = 8192
+        raise NotImplementedError(self.KG_REFUSAL)
 
     def _project(self, family, ids):
         device = self._check_ready()
@@ -1042,62 +1097,14 @@ class TransH(FusedKGEModel):
         )
         return out
 
-    def _projected_items(self):
-        tabs = [self.entity_embedding.weight, self.norm_vec.weight]
-        key = (self._step, tuple(t.data_ptr() for t in tabs), tuple(t._version for t in tabs))
-        hit = self.__dict__.get("_items_cache")
-        if hit is None or hit[0] != key:
-            hit = (key, self._project("entity", torch.arange(self.n_items, device=tabs[0].device)))
-            self.__dict__["_items_cache"] = hit
-            view = self.__dict__.get("_view")
-            if view is not None:
-                view.invalidate_target_image()
-        return hit[1]
 
-    def invalidate_target_image(self):
-        super().invalidate_target_image()
-        self.__dict__.pop("_items_cache", None)
-
-    def _rec_view(self, user_ids):
-        view = self._transe_view(self._project("user", user_ids), self._projected_items())
-        return view, torch.arange(view.n_users, device=view.user_embedding.weight.device)
-
-    def full_sort_predict(self, interaction):
-        if self.n_items < self.VIEW_MIN_ITEMS:
-            return super().full_sort_predict(interaction)
-        view, idx = self._rec_view(interaction[self.USER_ID])
-        return view.full_sort_predict({self.USER_ID: idx})
-
-    def full_sort_topk(self, user_ids, k, hist_off=None, hist_items=None, mask_pad=True, return_scores=True,
-                       path="auto", _debug_scores=False, relation_ids=None, workspace_budget=TOPK_WORKSPACE_BUDGET):
-        if relation_ids is not None:
-            raise NotImplementedError("the reference TransH has no KG scoring entry points (transh.py)")
-        if self.n_items < self.VIEW_MIN_ITEMS:
-            return super().full_sort_topk(user_ids, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores,
-                                          workspace_budget=workspace_budget)
-        view, idx = self._rec_view(user_ids)
-        return view.full_sort_topk(idx, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores,
-                                   workspace_budget=workspace_budget)
-
-    def full_sort_rank(self, query_ids, pos_off, pos_items, hist_off=None, hist_items=None, mask_pad=True,
-                       relation_ids=None):
-        if relation_ids is not None:
-            raise NotImplementedError("the reference TransH has no KG scoring entry points (transh.py)")
-        if self.n_items < self.VIEW_MIN_ITEMS:
-            return super().full_sort_rank(query_ids, pos_off, pos_items, hist_off, hist_items, mask_pad)
-        view, idx = self._rec_view(query_ids)
-        return view.full_sort_rank(idx, pos_off, pos_items, hist_off, hist_items, mask_pad)
-
-
-class TransD(FusedKGEModel):
+class TransD(_ProjectedKGEModel):
     """transd.py: every table has an embedding and a transfer vector; ``forward(ent, ent_vec, rel_vec) = rel_vec *
     <ent, ent_vec> + ent`` (transd.py:86-91) projects head and both tails before TransE's TripletMarginLoss
-    (transd.py:93-133).  The train step is one fused kernel like the others (KGE_TRANSD).  Scoring composes two
-    library calls: ``kge_transd_project`` writes the projected rows, and since the projection of an item does not
-    depend on the user, the rest IS TransE on projected tables -- a private TransE view of those buffers runs
-    predict, dense full-sort and the fused top-k (tensor-core path included).  ``full_sort_predict_kg`` is refused:
-    the reference's version projects the head with <h, h> and broadcasts a relation per row over all tails
-    (transd.py:192-217), which no projected table expresses."""
+    (transd.py:93-133).  The train step is one fused kernel like the others (KGE_TRANSD); ``kge_transd_project``
+    writes the projected rows for scoring.  ``full_sort_predict_kg`` is refused: the reference's version projects the
+    head with <h, h> and broadcasts a relation per row over all tails (transd.py:192-217), which no projected table
+    expresses."""
 
     KIND = "TransD"
     USER_TABLES = ("user_embedding", "user_vec_embedding")
@@ -1105,8 +1112,9 @@ class TransD(FusedKGEModel):
     RELATION_TABLES = ("relation_embedding", "relation_vec_embedding")
     CREATION_ORDER = ("user_embedding", "entity_embedding", "relation_embedding", "user_vec_embedding",
                       "entity_vec_embedding", "relation_vec_embedding")   # transd.py:41-47
+    KG_REFUSAL = ("TransD scores users against items only: the reference's full_sort_predict_kg projects the head "
+                  "with <h, h> and a relation per row over all tails (transd.py:192-217); not built")
 
-    # ---- projected rows ---------------------------------------------------------------------------------------
     def _project(self, family, ids, rel_ids=None):
         """[len(ids), d] projected rows of `family` ("user" / "entity"); rel_ids None = the user->item relation."""
         device = self._check_ready()
@@ -1125,32 +1133,6 @@ class TransD(FusedKGEModel):
         )
         return out
 
-    def _projected_items(self):
-        """Rows [0, n_items) of the entity table projected with the user->item relation, cached per weight version."""
-        tabs = self._tables(self.ENTITY_TABLES) + [self.relation_vec_embedding.weight]
-        key = (self._step, tuple(t.data_ptr() for t in tabs), tuple(t._version for t in tabs))
-        hit = self.__dict__.get("_items_cache")
-        if hit is None or hit[0] != key:
-            ids = torch.arange(self.n_items, device=tabs[0].device)
-            hit = (key, self._project("entity", ids))
-            self.__dict__["_items_cache"] = hit
-            view = self.__dict__.get("_view")
-            if view is not None:
-                view.invalidate_target_image()
-        return hit[1]
-
-    def invalidate_target_image(self):
-        super().invalidate_target_image()
-        self.__dict__.pop("_items_cache", None)
-
-    # ---- scoring ----------------------------------------------------------------------------------------------
-    def predict(self, interaction):
-        users, items = interaction[self.USER_ID], interaction[self.ITEM_ID]
-        view = self._transe_view(self._project("user", users), self._project("entity", items))
-        view.invalidate_target_image()
-        idx = torch.arange(view.n_users, device=view.user_embedding.weight.device)
-        return view.predict({self.USER_ID: idx, self.ITEM_ID: idx})
-
     def predict_kg(self, interaction):
         heads, rels, tails = (interaction[k] for k in (self.HEAD_ENTITY_ID, self.RELATION_ID, self.TAIL_ENTITY_ID))
         both = torch.cat([self._project("entity", heads, rels), self._project("entity", tails, rels)])
@@ -1160,33 +1142,6 @@ class TransD(FusedKGEModel):
         idx = torch.arange(n, device=both.device)
         return view.predict_kg({self.HEAD_ENTITY_ID: idx, self.RELATION_ID: self._ids(rels, both.device),
                                 self.TAIL_ENTITY_ID: idx + n})
-
-    def _rec_view(self, user_ids):
-        view = self._transe_view(self._project("user", user_ids), self._projected_items())
-        return view, torch.arange(view.n_users, device=view.user_embedding.weight.device)
-
-    def full_sort_predict(self, interaction):
-        view, idx = self._rec_view(interaction[self.USER_ID])
-        return view.full_sort_predict({self.USER_ID: idx})
-
-    def full_sort_predict_kg(self, interaction):
-        raise NotImplementedError("TransD.full_sort_predict_kg: the reference projects the head with <h, h> and a "
-                                  "relation per row over all tails (transd.py:192-217); not built")
-
-    def full_sort_topk(self, user_ids, k, hist_off=None, hist_items=None, mask_pad=True, return_scores=True,
-                       path="auto", _debug_scores=False, relation_ids=None, workspace_budget=TOPK_WORKSPACE_BUDGET):
-        if relation_ids is not None:
-            raise NotImplementedError("TransD scores users against items only (see full_sort_predict_kg)")
-        view, idx = self._rec_view(user_ids)
-        return view.full_sort_topk(idx, k, hist_off, hist_items, mask_pad, return_scores, path, _debug_scores,
-                                   workspace_budget=workspace_budget)
-
-    def full_sort_rank(self, query_ids, pos_off, pos_items, hist_off=None, hist_items=None, mask_pad=True,
-                       relation_ids=None):
-        if relation_ids is not None:
-            raise NotImplementedError("TransD scores users against items only (see full_sort_predict_kg)")
-        view, idx = self._rec_view(query_ids)
-        return view.full_sort_rank(idx, pos_off, pos_items, hist_off, hist_items, mask_pad)
 
 
 MODELS = {"TransE": TransE, "DistMult": DistMult, "RotatE": RotatE, "ComplEx": ComplEx, "TorusE": TorusE,

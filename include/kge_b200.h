@@ -36,13 +36,15 @@ typedef void* kge_stream_t; /* cudaStream_t */
  * r and the hyperplane vector w (`norm_vec`); the reference's project() is ent - (ent * sum(w)) * w (transh.py:73-74:
  * the SUM of w's components, not <ent, w>), i.e. ent * (1 - sum(w) * w) element-wise, applied to head and both tails
  * before TransE's TripletMarginLoss / norm (transh.py:53-58, 76-107).  Recommendation triples take row
- * `ui_relation` of both parts.  Scoring: predict and full-sort over items (transh.py:109-145); the reference has no
- * KG scoring entry points for this model.  CUDA-core scoring paths only.
+ * `ui_relation` of both parts.  TRAIN STEP ONLY: scoring (predict and full-sort over items, transh.py:109-145; the
+ * reference has no KG scoring entry points for this model) goes through kge_transh_project, which writes projected
+ * rows, and the KGE_TRANSE scoring entry points on those.
  * KGE_TRANSD (transd.py): every table has two parts, the embedding and a transfer vector; an entity e with transfer
  * vector e_p is projected with the relation's r_p as e + r_p * <e, e_p> (transd.py:86-91) before TransE's
  * TripletMarginLoss (transd.py:93-133).  TRAIN STEP ONLY: scoring goes through kge_transd_project, which writes
  * projected rows, and the KGE_TRANSE scoring entry points on those (the projection of an item does not depend on the
- * user, so full-sort over items is TransE over a projected table). */
+ * user, so full-sort over items is TransE over a projected table).
+ * The scoring entry points refuse KGE_TRANSH and KGE_TRANSD with KGE_E_UNSUPPORTED. */
 enum kge_model_kind {
   KGE_TRANSE = 0, KGE_DISTMULT = 1, KGE_ROTATE = 2, KGE_COMPLEX = 3, KGE_TORUSE = 4, KGE_TRANSH = 5, KGE_TRANSD = 6
 };
@@ -216,8 +218,8 @@ int kge_transd_project(const float* emb, const float* vec, const int64_t* ids, i
                        kge_stream_t stream);
 
 /* kge_transh_project: out[i, :] = E[id_i] * (1 - sum(w) * w), w = W[rel_i]  (TransH.project, transh.py:73-74).
- * Lets full-sort over a large item set run as KGE_TRANSE over projected tables (tensor-core path included); the
- * KGE_TRANSH scoring entry points compute the same scores directly on the CUDA cores. */
+ * ids == NULL: rows 0..n-1 in order; rel_ids == NULL: relation row `rel_row` for every i.  TransH scores as
+ * KGE_TRANSE over these projected rows (tensor-core path included). */
 int kge_transh_project(const float* emb, const int64_t* ids, int64_t n, int32_t d, const float* norm_vec,
                        const int64_t* rel_ids, int64_t rel_row, float* out, kge_stream_t stream);
 

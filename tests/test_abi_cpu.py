@@ -123,6 +123,27 @@ def test_sweep_plan_sizes(kind, d, tn):
     assert lib.kge_mma_image_bytes(C.byref(m), n_targets, ord("x")) == -1
 
 
+@pytest.mark.parametrize("kind,project", [("TransH", b"kge_transh_project"), ("TransD", b"kge_transd_project")])
+def test_projected_models_are_refused_by_the_scorers(kind, project):
+    """TransH and TransD score as TransE over the rows their projection entry point writes: every scoring entry
+    point refuses the model kind itself (KGE_E_UNSUPPORTED, naming that entry point) before it looks at a table."""
+    from hopwise_b200 import _abi
+
+    lib = _abi.lib()
+    m = C.byref(_model_struct(kind, 16))
+    calls = {
+        "kge_predict": lambda: lib.kge_predict(m, None, None, None, 4, 1, None, None),
+        "kge_full_sort_scores": lambda: lib.kge_full_sort_scores(m, None, None, 4, 1, 100, None, None),
+        "kge_full_sort_topk": lambda: lib.kge_full_sort_topk(m, None, None, 4, 1, 100, None, None, 1, 10, None, None,
+                                                             None, 0, None),
+        "kge_full_sort_rank_counts": lambda: lib.kge_full_sort_rank_counts(m, None, None, 4, 1, 100, None, None, 1, None,
+                                                                           None, None, None, None, None, 0, None),
+    }
+    for name, call in calls.items():
+        assert call() == -2, name   # KGE_E_UNSUPPORTED
+        assert project in lib.kge_last_error(), name
+
+
 def test_product_has_no_cpu_fallback_and_no_oracle_import():
     import torch
 

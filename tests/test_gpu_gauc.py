@@ -87,8 +87,7 @@ def _transh_planes(m, R, d, rng):
                                       ("TorusE", 30, 1300), ("TorusE", 64, 2500), ("TransH", 64, 2000),
                                       ("TransH", 50, 9000), ("TransD", 30, 100), ("TransD", 64, 9000)])
 def test_rank_counts_equal_dense_counts(name, d, I):
-    """Every model, d % 4 != 0, fewer items than one 128-row tile, and >= 8,192 items for TransH / TransD (the
-    projected TransE view)."""
+    """Every model, d % 4 != 0, fewer items than one 128-row tile, and TransH / TransD also at >= 8,192 items."""
     U, E, R = 400, I + 300, 9
     m = make_product_model(name, U, I, E, R, d)
     rng = np.random.default_rng(11)

@@ -150,7 +150,7 @@ def test_reference_metric_known_answers():
 @pytest.mark.parametrize("name,d,I,k", [("TransE", 100, 3001, 10), ("DistMult", 64, 5000, 20), ("ComplEx", 32, 1599, 10),
                                         ("RotatE", 64, 777, 50), ("TransE", 22, 130, 128), ("TorusE", 64, 2500, 20),
                                         ("TransH", 64, 2000, 20), ("TransD", 64, 2500, 20), ("TransD", 64, 9000, 20),
-                                        ("TransH", 64, 9000, 20)])   # (>= 8192 items: TransE over projected tables)
+                                        ("TransH", 64, 9000, 20)])   # (>= 8192 items: "auto" takes the tensor cores)
 def test_topk_against_oracle(name, d, I, k):
     U, E, R = 400, I + 500, 9
     ora = make_oracle_model(name, U, I, E, R, d)
