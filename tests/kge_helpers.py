@@ -78,6 +78,45 @@ def to_cpu_batch(b):
     return {k: torch.as_tensor(np.asarray(v), dtype=torch.long) for k, v in b.items()}
 
 
+def closed_form_forward(name, tabs, b, w_rec, w_kg, ui_row, margin=1.0, families=None, chunk=65536):
+    """float64 closed form of one training forward pass (oracle.kge_numpy.pair_loss_and_grads on every pair).
+
+    tabs: {"user" | "entity" | "relation": [float64 table per part]}; b: one entry per (positive, negative) pair
+    (the tiled view of a K-negative batch, `tile_batch`); w_rec / w_kg: the weight of one pair in the scalar loss.
+    Returns (loss, g, a, active): g and a are per family lists shaped like the tables -- the gradient, and the scale of
+    its fp32 rounding: the sum over the contributing pairs of the pair's largest gradient term in that column (the
+    head and relation gradients of the translation models are differences of the two tails' terms, which cancel in
+    float64 where fp32 keeps their rounding; at d = 1 they cancel in every pair whose residuals share a sign) -- and
+    active[family] is a bool [rows] of the rows of a pair with a gradient (pairwise models: the hinge is open; the
+    user->item relation row belongs to every rec pair).  With `families`, g and a are accumulated for those families only."""
+    from oracle.kge_numpy import pair_loss_and_grads
+
+    g = {f: [np.zeros_like(t) for t in ts] for f, ts in tabs.items()}
+    a = {f: [np.zeros_like(t) for t in ts] for f, ts in tabs.items()}
+    active = {f: np.zeros(len(ts[0]), dtype=bool) for f, ts in tabs.items()}
+    loss = 0.0
+    n_rec = len(b["user_id"])
+    segs = (("user", b["user_id"], np.full(n_rec, ui_row), b["item_id"], b["neg_item_id"], w_rec),
+            ("entity", b["head_id"], b["relation_id"], b["tail_id"], b["neg_tail_id"], w_kg))
+    for hfam, hid, rid, tpid, tnid, w in segs:
+        fams = (hfam, "relation", "entity", "entity")
+        for s in range(0, len(hid), chunk):   # (chunks keep the float64 temporaries small)
+            ids = [np.asarray(x[s : s + chunk]) for x in (hid, rid, tpid, tnid)]
+            rows = [[t[i] for t in tabs[f]] for f, i in zip(fams, ids)]
+            l, *grads = pair_loss_and_grads(name, *rows, w, margin)
+            loss += l
+            act = np.any(np.stack([x != 0 for gs in grads for x in gs]), axis=(0, 2))
+            scale = np.max(np.stack([np.abs(x) for gs in grads for x in gs]), axis=0)
+            for f, i, gs in zip(fams, ids, grads):
+                if families is not None and f not in families:
+                    continue
+                for p, x in enumerate(gs):
+                    np.add.at(g[f][p], i, x)
+                    np.add.at(a[f][p], i, scale)
+                active[f][i[act]] = True
+    return loss, g, a, active
+
+
 def assert_weights_close(got, want, rtol=1e-5, atol=5e-7, outlier_frac=5e-4, outlier_atol=1e-4, err_msg=""):
     """Post-Adam weights: every element within rtol/atol, except a bounded few.
 

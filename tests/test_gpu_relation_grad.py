@@ -8,8 +8,8 @@ a relation table too large for the copies and a pass without gradients take the 
 import numpy as np
 import pytest
 
-from kge_helpers import make_product_model, to_device_batch
-from oracle.kge_numpy import pair_loss_and_grads, loss_weights
+from kge_helpers import closed_form_forward, make_product_model, to_device_batch
+from oracle.kge_numpy import loss_weights
 
 pytestmark = pytest.mark.gpu
 
@@ -43,30 +43,11 @@ def _tables(m, names):
 
 def _closed_form(m, name, b, R, margin=1.0):
     """float64 relation gradient [PR][R][d] of the scalar loss, and which relation rows got an active triple."""
-    u = _tables(m, m.USER_TABLES)
-    e = _tables(m, m.ENTITY_TABLES)
-    r = _tables(m, m.RELATION_TABLES)
-    n_rec, n_kg = len(b["user_id"]), len(b["head_id"])
-    w_rec, w_kg = loss_weights(name, n_rec, n_kg)
-    g = np.zeros((len(r), R, D))
-    active = np.zeros(R, dtype=bool)
-    ui = R - 1
-    segs = ((b["user_id"], np.full(n_rec, ui), b["item_id"], b["neg_item_id"], u, w_rec),
-            (b["head_id"], b["relation_id"], b["tail_id"], b["neg_tail_id"], e, w_kg))
-    for hid, rid, tpid, tnid, htab, w in segs:
-        for s in range(0, len(hid), 65536):   # (chunks keep the float64 temporaries small)
-            sl = slice(s, s + 65536)
-            h = [t[hid[sl]] for t in htab]
-            rr = [t[rid[sl]] for t in r]
-            tp = [t[tpid[sl]] for t in e]
-            tn = [t[tnid[sl]] for t in e]
-            _, _, gr, _, _ = pair_loss_and_grads(name, h, rr, tp, tn, w, margin)
-            for p in range(len(r)):
-                np.add.at(g[p], rid[sl], gr[p])
-            # a triple is active when its gradient is (pairwise models: the hinge is open)
-            act = np.any(np.stack([x != 0 for x in gr]), axis=(0, 2))
-            active[np.unique(rid[sl][act])] = True
-    return g, active
+    tabs = {"user": _tables(m, m.USER_TABLES), "entity": _tables(m, m.ENTITY_TABLES),
+            "relation": _tables(m, m.RELATION_TABLES)}
+    w_rec, w_kg = loss_weights(name, len(b["user_id"]), len(b["head_id"]))
+    _, g, _, active = closed_form_forward(name, tabs, b, w_rec, w_kg, R - 1, margin, families=("relation",))
+    return np.stack(g["relation"]), active["relation"]
 
 
 def _forward(m, b):
