@@ -13,7 +13,7 @@ import os
 
 from . import _build
 
-KGE_ABI_VERSION = 7
+KGE_ABI_VERSION = 8
 MODEL_KINDS = {"TransE": 0, "DistMult": 1, "RotatE": 2, "ComplEx": 3, "TorusE": 4, "TransH": 5, "TransD": 6}
 
 
@@ -133,6 +133,11 @@ PROTOTYPES = {
     ),
     "kge_topk_hits": (C.c_int, [_P, C.c_int64, C.c_int32, _P, _P, _P, _P]),
     "kge_topk_metric_sums": (C.c_int, [_P, C.c_int64, C.c_int32, _P, _P]),
+    "kge_candidate_select_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64]),
+    "kge_candidate_select": (
+        C.c_int,
+        [_P, _P, C.c_int64, _P, C.c_int64, C.c_int64, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_int64, _P],
+    ),
     "kge_gather_columns": (C.c_int, [_P, C.c_int32, C.c_int64, _P, C.c_int64, _P, _P, _P]),
     "kge_widen_ids_i32": (C.c_int, [_P, _P, C.c_int64, _P]),
     "kge_assemble_batch_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64, C.c_int32]),

@@ -1542,3 +1542,282 @@ extern "C" int kge_topk_metric_sums(const int32_t* rec_topk, int64_t n, int32_t 
   KGE_LAUNCH_CHECK();
   return 0;
 }
+
+// ---- sampled evaluation: per-row selection over a candidate list (uni-N / pop-N) ----------------------------------
+// The dense route scatters each row's candidate scores into a -inf row of n_targets columns, then runs torch.topk and
+// (for GAUC) a full sort over it.  Here a row is its candidate list only: keys are sorted in on-chip or workspace
+// memory, twice -- by id (duplicates collapse, positives find their scores, the padding finds the smallest
+// non-candidate ids) and then by (score desc, id asc) for the top k and the rank counts.  Rows pick their regime on
+// the device: up to CAND_WARP_MAX keys a warp sorts them in shared memory, up to CAND_CTA_MAX a CTA does, longer rows
+// sort in the workspace at their own candidate offset.
+namespace {
+constexpr int CAND_WARP_MAX = 512;
+constexpr int CAND_CTA_MAX = 8192;
+constexpr int CAND_THREADS = 256;
+
+struct CandArgs {
+  const float* scores;
+  const int64_t* items;
+  int64_t n_cand;
+  const int64_t* off;
+  int64_t n, n_targets;
+  const int64_t* pos_off;
+  const int64_t* pos_items;
+  int k;
+  int64_t* ids_out;
+  float* scores_out;
+  int64_t* greater_out;
+  int64_t* equal_out;
+  int64_t* n_unmasked_out;
+  uint64_t* ws;   // [n_cand] keys: rows above CAND_CTA_MAX sort at their candidate offset
+};
+
+__device__ __forceinline__ uint64_t rot32(uint64_t x) { return (x << 32) | (x >> 32); }
+
+template <bool BLOCK>
+__device__ __forceinline__ void group_sync() {
+  if (BLOCK) __syncthreads(); else __syncwarp();
+}
+
+// Sort buf[0, len) descending with a group of nt threads (a warp or the block).  Bitonic network over the next power
+// of two P >= len in the form whose every compare-exchange moves the larger key to the lower index (each merge starts
+// with the mirrored comparison): the keys past len are virtual zeros, the smallest key, which never move, so they
+// need no storage.
+template <bool BLOCK>
+__device__ void group_sort_desc(uint64_t* buf, int64_t len, int tid, int nt) {
+  int64_t P = 1;
+  while (P < len) P <<= 1;
+  for (int64_t size = 2; size <= P; size <<= 1) {
+    const int64_t half = size >> 1;
+    for (int64_t i = tid; i < P / 2; i += nt) {
+      const int64_t blk = i / half, j = i - blk * half;
+      const int64_t lo = blk * size + j, hi = blk * size + size - 1 - j;
+      if (hi < len) {
+        const uint64_t x = buf[lo], y = buf[hi];
+        if (x < y) {
+          buf[lo] = y;
+          buf[hi] = x;
+        }
+      }
+    }
+    group_sync<BLOCK>();
+    for (int64_t stride = size >> 2; stride > 0; stride >>= 1) {
+      for (int64_t i = tid; i < P / 2; i += nt) {
+        const int64_t lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
+        if (hi < len) {
+          const uint64_t x = buf[lo], y = buf[hi];
+          if (x < y) {
+            buf[lo] = y;
+            buf[hi] = x;
+          }
+        }
+      }
+      group_sync<BLOCK>();
+    }
+  }
+}
+
+// Drop the repeats of the sorted buf[0, len) in place; returns the number of distinct keys (group-uniform).  A round
+// reads all its keys before it writes, and writes land at or below the positions read, so later rounds read
+// untouched keys; the last key of a round is carried into the next (s_carry / s_cnt: block only).
+template <bool BLOCK>
+__device__ int64_t group_unique(uint64_t* buf, int64_t len, int tid, int nt, uint32_t* s_cnt, uint64_t* s_carry) {
+  const int lane = tid & 31, warp = tid >> 5;
+  int64_t w = 0;
+  uint64_t carry = 0ull;   // no key is 0
+  if (BLOCK) {
+    if (tid == 0) *s_carry = 0ull;
+    __syncthreads();
+  }
+  for (int64_t base = 0; base < len; base += nt) {
+    const int64_t i = base + tid;
+    const uint64_t x = i < len ? buf[i] : 0ull;
+    uint64_t prev;
+    if (BLOCK) {
+      prev = (tid == 0) ? *s_carry : (i < len ? buf[i - 1] : 0ull);
+    } else {
+      prev = __shfl_up_sync(0xffffffffu, x, 1);
+      if (lane == 0) prev = carry;
+    }
+    const bool keep = i < len && x != prev;
+    const unsigned b = __ballot_sync(0xffffffffu, keep);
+    const int below = __popc(b & ((1u << lane) - 1u));
+    if (BLOCK) {
+      if (lane == 0) s_cnt[warp] = __popc(b);
+      __syncthreads();   // every read of the round is done and the counts are in
+      int before = 0, total = 0;
+      for (int q = 0; q < (nt >> 5); ++q) {
+        const int c = (int)s_cnt[q];
+        before += q < warp ? c : 0;
+        total += c;
+      }
+      if (keep) buf[w + before + below] = x;
+      if (tid == nt - 1) *s_carry = x;
+      w += total;
+      __syncthreads();
+    } else {
+      if (keep) buf[w + below] = x;
+      w += __popc(b);
+      carry = __shfl_sync(0xffffffffu, x, 31);
+      __syncwarp();
+    }
+  }
+  return w;
+}
+
+// Number of keys of the descending buf[0, D) whose upper 32 bits are >= h (h <= 2^32).
+__device__ __forceinline__ int64_t count_hi_ge(const uint64_t* buf, int64_t D, uint64_t h) {
+  int64_t lo = 0, hi = D;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    if ((buf[mid] >> 32) >= h) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
+template <bool BLOCK>
+__device__ void cand_row(const CandArgs& a, int64_t row, int64_t c0, int64_t len, uint64_t* buf, int tid, int nt,
+                         uint32_t* s_cnt, uint64_t* s_carry) {
+  // 1. by id: key (~id << 32 | score bits), sorted descending = id ascending; equal ids carry equal scores
+  for (int64_t i = tid; i < len; i += nt)
+    buf[i] = rot32(make_key(__ldg(a.scores + c0 + i), (uint32_t)__ldg(a.items + c0 + i)));
+  group_sync<BLOCK>();
+  group_sort_desc<BLOCK>(buf, len, tid, nt);
+  const int64_t D = group_unique<BLOCK>(buf, len, tid, nt, s_cnt, s_carry);
+  if (a.n_unmasked_out && tid == 0) a.n_unmasked_out[row] = D;
+  const int64_t k = a.k;
+  // the padding of a row with fewer than k candidates: the smallest non-candidate ids, ascending, score -inf.  Id x
+  // that is not a candidate is non-candidate number x - #(candidates < x).
+  if (D < k && (a.ids_out || a.scores_out))
+    for (int64_t x = tid; x < k + D && x < a.n_targets; x += nt) {
+      const int64_t c = count_hi_ge(buf, D, 0x100000000ull - (uint64_t)x);   // candidates with id < x
+      const bool member = c < D && (buf[c] >> 32) == 0xFFFFFFFFull - (uint64_t)x;
+      const int64_t j = x - c;
+      if (!member && j < k - D) {
+        if (a.ids_out) a.ids_out[row * k + D + j] = x;
+        if (a.scores_out) a.scores_out[row * k + D + j] = -INFINITY;
+      }
+    }
+  // each positive's score bits, or -1 when it is not a candidate, parked in its own greater_out slot
+  const int64_t p0 = a.greater_out ? a.pos_off[row] : 0, p1 = a.greater_out ? a.pos_off[row + 1] : 0;
+  for (int64_t i = p0 + tid; i < p1; i += nt) {
+    const uint64_t h = 0xFFFFFFFFull - (uint64_t)(uint32_t)a.pos_items[i];
+    const int64_t c = count_hi_ge(buf, D, h + 1);
+    a.greater_out[i] = (c < D && (buf[c] >> 32) == h) ? (int64_t)(uint32_t)buf[c] : -1;
+  }
+  group_sync<BLOCK>();
+  // 2. by (score desc, id asc): make_key's layout
+  for (int64_t i = tid; i < D; i += nt) buf[i] = rot32(buf[i]);
+  group_sync<BLOCK>();
+  group_sort_desc<BLOCK>(buf, D, tid, nt);
+  const int64_t top = D < k ? D : k;
+  for (int64_t i = tid; i < top; i += nt) {
+    const uint64_t key = buf[i];
+    if (a.ids_out) a.ids_out[row * k + i] = key_id(key);
+    if (a.scores_out) a.scores_out[row * k + i] = key_score(key);
+  }
+  // the counts of kge_full_sort_rank_counts over the row's distinct candidates; the rest of the row is -inf
+  for (int64_t i = p0 + tid; i < p1; i += nt) {
+    const int64_t t = a.greater_out[i];
+    int64_t g = D, e = a.n_targets - D;
+    if (t >= 0) {
+      g = count_hi_ge(buf, D, (uint64_t)t + 1);
+      e = count_hi_ge(buf, D, (uint64_t)t) - g;
+    }
+    a.greater_out[i] = g;
+    a.equal_out[i] = e;
+  }
+  group_sync<BLOCK>();
+}
+
+__device__ __forceinline__ void cand_range(const CandArgs& a, int64_t row, int64_t& c0, int64_t& len) {
+  // (clamped to [0, n_cand]: a malformed offset list cannot send a row outside the candidates)
+  int64_t s = __ldg(a.off + row), e = __ldg(a.off + row + 1);
+  s = s < 0 ? 0 : (s > a.n_cand ? a.n_cand : s);
+  e = e < s ? s : (e > a.n_cand ? a.n_cand : e);
+  c0 = s;
+  len = e - s;
+}
+
+// One warp per row, rows of at most CAND_WARP_MAX candidates.
+__global__ void __launch_bounds__(CAND_THREADS) cand_select_warp_kernel(const CandArgs a) {
+  __shared__ uint64_t bufs[CAND_THREADS / 32][CAND_WARP_MAX];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t row = (int64_t)blockIdx.x * (CAND_THREADS / 32) + warp;
+  if (row >= a.n) return;
+  int64_t c0, len;
+  cand_range(a, row, c0, len);
+  if (len > CAND_WARP_MAX) return;
+  cand_row<false>(a, row, c0, len, bufs[warp], lane, 32, nullptr, nullptr);
+}
+
+// One CTA per row, rows above CAND_WARP_MAX candidates: in shared memory up to CAND_CTA_MAX, else in the workspace.
+// The CTAs stride over the rows (how many are long is only known on the device).
+__global__ void __launch_bounds__(CAND_THREADS) cand_select_cta_kernel(const CandArgs a) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ uint32_t s_cnt[CAND_THREADS / 32];
+  __shared__ uint64_t s_carry;
+  for (int64_t row = blockIdx.x; row < a.n; row += gridDim.x) {
+    int64_t c0, len;
+    cand_range(a, row, c0, len);
+    if (len <= CAND_WARP_MAX) continue;
+    uint64_t* buf = len <= CAND_CTA_MAX ? reinterpret_cast<uint64_t*>(smem_raw) : a.ws + c0;
+    cand_row<true>(a, row, c0, len, buf, threadIdx.x, blockDim.x, s_cnt, &s_carry);
+  }
+}
+}  // namespace
+
+extern "C" int64_t kge_candidate_select_workspace_bytes(int64_t n, int64_t n_cand) {
+  if (n < 0 || n_cand < 0) return -1;
+  return n_cand * 8;
+}
+
+extern "C" int kge_candidate_select(const float* scores, const int64_t* cand_items, int64_t n_cand,
+                                    const int64_t* cand_off, int64_t n, int64_t n_targets, const int64_t* pos_off,
+                                    const int64_t* pos_items, int32_t k, int64_t* ids_out, float* scores_out,
+                                    int64_t* greater_out, int64_t* equal_out, int64_t* n_unmasked_out,
+                                    void* workspace, int64_t workspace_bytes, kge_stream_t stream) {
+  KGE_REQUIRE(n >= 0 && n_cand >= 0, KGE_E_ARG, "negative n / n_cand");
+  KGE_REQUIRE(k >= 1, KGE_E_ARG, "k=%d below 1", k);
+  KGE_REQUIRE(n_targets >= 1 && n_targets < 0xFFFFFFFFll, KGE_E_ARG, "n_targets outside [1, 2^32-2]");
+  KGE_REQUIRE(k <= n_targets, KGE_E_ARG, "k=%d larger than the number of targets", k);
+  KGE_REQUIRE((greater_out == nullptr) == (equal_out == nullptr), KGE_E_ARG, "greater_out and equal_out go together");
+  if (n == 0) return 0;
+  KGE_REQUIRE(cand_off, KGE_E_ARG, "NULL cand_off");
+  KGE_REQUIRE(n_cand == 0 || (scores && cand_items), KGE_E_ARG, "NULL scores / cand_items");
+  KGE_REQUIRE(!greater_out || (pos_off && pos_items), KGE_E_ARG, "NULL pos_off / pos_items");
+  KGE_REQUIRE(workspace_bytes >= n_cand * 8 && (n_cand == 0 || workspace), KGE_E_ARG,
+              "workspace too small: need %lld bytes", (long long)(n_cand * 8));
+  CandArgs a;
+  a.scores = scores;
+  a.items = cand_items;
+  a.n_cand = n_cand;
+  a.off = cand_off;
+  a.n = n;
+  a.n_targets = n_targets;
+  a.pos_off = pos_off;
+  a.pos_items = pos_items;
+  a.k = k;
+  a.ids_out = ids_out;
+  a.scores_out = scores_out;
+  a.greater_out = greater_out;
+  a.equal_out = equal_out;
+  a.n_unmasked_out = n_unmasked_out;
+  a.ws = reinterpret_cast<uint64_t*>(workspace);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t rows_per_cta = CAND_THREADS / 32;
+  cand_select_warp_kernel<<<(unsigned)((n + rows_per_cta - 1) / rows_per_cta), CAND_THREADS, 0, st>>>(a);
+  KGE_LAUNCH_CHECK();
+  // rows above CAND_WARP_MAX need at least that many candidates each
+  int64_t g = n_cand / (CAND_WARP_MAX + 1);
+  const int64_t cap = (int64_t)kge_num_sms() * 3;
+  if (g > cap) g = cap;
+  if (g > n) g = n;
+  if (g >= 1) {
+    const size_t smem = (size_t)CAND_CTA_MAX * 8;
+    KGE_CUDA(cudaFuncSetAttribute(cand_select_cta_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cand_select_cta_kernel<<<(unsigned)g, CAND_THREADS, smem, st>>>(a);
+    KGE_LAUNCH_CHECK();
+  }
+  return 0;
+}

@@ -13,6 +13,10 @@ Host-side mirror of (paths under /root/reference/hopwise/):
 The dense [n_users, n_items] score matrix of the reference never exists here: the kernel keeps
 the per-user top-k on chip, and GAUC's ranks are counted during the same kind of sweep
 (kge_full_sort_rank_counts).  Tie order is (score desc, item id asc).
+
+Sampled evaluation (eval_args.mode uniN / popN: trainer.py's _neg_sample_batch_eval scatters the candidate scores
+into -inf rows of n_items columns) goes through collect_sampled: the loader's batches are concatenated on the device
+and every block of users takes one kge_candidate_select call over its candidate lists.
 """
 
 from __future__ import annotations
@@ -20,6 +24,7 @@ from __future__ import annotations
 import ctypes as C
 from collections import OrderedDict
 
+import numpy as np
 import torch
 
 from . import _abi
@@ -183,3 +188,65 @@ def evaluate_full_sort(model, user_ids, hist_off, hist_items, pos_off, pos_items
     if return_struct:
         return result, torch.cat(recs)
     return result
+
+
+def collect_sampled(model, batches, k: int, meanrank: bool = False, user_block: int | None = None):
+    """The collector's data of a sampled evaluation, without the [batch_users, n_items] score rows.
+
+    ``batches`` yields what hopwise's sampled loader yields and ``_neg_sample_batch_eval`` receives:
+    ``(interaction, row_idx, positive_u, positive_i)``, with the candidate rows of each batch user contiguous in
+    ``interaction`` and ``row_idx`` naming their batch-local user; the batch has ``positive_u[-1] + 1`` users.  It is
+    iterated exactly once (the loader draws fresh negatives on every pass).  Returns ``(struct, n_batches)``: struct
+    holds ``"rec.topk"`` (int32 [n, k+1]), ``"rec.items"`` (int64 [n, k]), ``"rec.users"`` (the interactions' user
+    column) and, with ``meanrank``, ``"rec.meanrank"`` (float32 [n, 3]); the rows are the batches' users in order.
+    Every block of ``user_block`` users (default: all) takes one kge_candidate_select call."""
+    device = next(model.parameters()).device
+    users, items, counts, pos_rows, pos_items = [], [], [], [], []
+    n = n_batches = 0
+    for interaction, row_idx, positive_u, positive_i in batches:
+        n_batches += 1
+        pu = torch.as_tensor(positive_u, dtype=torch.int64).cpu()
+        rows = torch.as_tensor(row_idx, dtype=torch.int64).cpu()
+        n_b = int(pu[-1]) + 1 if pu.numel() else 0   # trainer.py: batch_user_num = positive_u[-1] + 1
+        if rows.numel() and (bool((rows.diff() < 0).any()) or int(rows[-1]) >= n_b or int(rows[0]) < 0):
+            raise ValueError("the candidate rows of a batch must be grouped by user, in order, inside the batch's users")
+        counts.append(torch.bincount(rows, minlength=n_b))
+        users.append(torch.as_tensor(interaction[model.USER_ID]).to(device, non_blocking=True))
+        items.append(torch.as_tensor(interaction[model.ITEM_ID]).to(device, non_blocking=True))
+        pos_rows.append(pu + n)
+        pos_items.append(torch.as_tensor(positive_i, dtype=torch.int64).cpu())
+        n += n_b
+    cand_off = torch.zeros(n + 1, dtype=torch.int64)
+    if n:
+        torch.cumsum(torch.cat(counts), 0, out=cand_off[1:])
+    user_col = torch.cat(users) if users else torch.zeros(0, dtype=torch.int64, device=device)
+    item_col = torch.cat(items) if items else torch.zeros(0, dtype=torch.int64, device=device)
+    # the positives CSR, each (user, item) once: pos_matrix[positive_u, positive_i] = 1 (collector.py)
+    pr = torch.cat(pos_rows).numpy() if pos_rows else np.zeros(0, np.int64)
+    pi = torch.cat(pos_items).numpy() if pos_items else np.zeros(0, np.int64)
+    span = int(max(model.n_items, pi.max() + 1 if pi.size else 1))
+    packed = np.unique(pr * span + pi)
+    prow = packed // span
+    pos_off = np.zeros(n + 1, dtype=np.int64)
+    np.cumsum(np.bincount(prow, minlength=n), out=pos_off[1:])
+    pos_items_d = torch.from_numpy(packed - prow * span).to(device)
+    pos_off_d = torch.from_numpy(pos_off).to(device)
+    block = max(1, user_block or n)
+    topk, ids_all, mr = [], [], []
+    for s in range(0, n, block):
+        e = min(n, s + block)
+        c0, c1, p0, p1 = int(cand_off[s]), int(cand_off[e]), int(pos_off[s]), int(pos_off[e])
+        po, pv = pos_off_d[s : e + 1] - p0, pos_items_d[p0:p1]
+        ids, _, greater, equal, n_unmasked = model._candidate_select(
+            user_col[c0:c1], item_col[c0:c1], cand_off[s : e + 1] - c0, k, True, False,
+            po if meanrank else None, pv if meanrank else None)
+        topk.append(topk_hits(ids, po, pv))
+        ids_all.append(ids)
+        if meanrank:
+            mr.append(model._meanrank_rows(greater, equal, n_unmasked, po, pv))
+    struct = {"rec.topk": torch.cat(topk) if topk else torch.zeros(0, k + 1, dtype=torch.int32, device=device),
+              "rec.items": torch.cat(ids_all) if ids_all else torch.zeros(0, k, dtype=torch.int64, device=device),
+              "rec.users": user_col}
+    if meanrank:
+        struct["rec.meanrank"] = torch.cat(mr) if mr else torch.zeros(0, 3, device=device)
+    return struct, n_batches

@@ -903,6 +903,10 @@ class FusedKGEModel(KnowledgeRecommender):
                              "user_len is the argmin of the sorted row")
         greater, equal, n_unmasked = self.full_sort_rank(query_ids, pos_off, pos_items, hist_off, hist_items, mask_pad,
                                                          relation_ids)
+        return self._meanrank_rows(greater, equal, n_unmasked, pos_off, pos_items)
+
+    def _meanrank_rows(self, greater, equal, n_unmasked, pos_off, pos_items):
+        """rec.meanrank rows from rank counts: a duplicate positive of a row counts once, float64 sums."""
         device = greater.device
         pos_off, pos_items = self._ids(pos_off, device), self._ids(pos_items, device)
         n, n_pos = n_unmasked.numel(), pos_items.numel()
@@ -914,6 +918,74 @@ class FusedKGEModel(KnowledgeRecommender):
         rank_sum = torch.zeros(n, dtype=torch.float64, device=device).index_add_(0, row, avg_rank * once)
         pos_len = torch.zeros(n, dtype=torch.float64, device=device).index_add_(0, row, once)
         return torch.stack([rank_sum, n_unmasked.double(), pos_len], dim=1).float()
+
+    # ------------------------------------------------------------------ sampled evaluation over candidate lists
+    def _candidate_select(self, user_col, item_col, cand_off, k: int, want_ids=True, want_scores=False,
+                          pos_off=None, pos_items=None):
+        """predict on the candidate rows, then kge_candidate_select.  Returns (ids, scores, greater, equal,
+        n_unmasked), None where not asked for (the rank counts are asked for with the positives CSR)."""
+        k = int(k)
+        if k < 1:
+            raise ValueError(f"k={k} below 1")
+        n_cand = len(item_col)
+        if len(user_col) != n_cand:
+            raise ValueError("user_col and item_col must have one entry per candidate")
+        cand_off = torch.as_tensor(cand_off)
+        if cand_off.dim() != 1 or cand_off.numel() < 1:
+            raise ValueError("cand_off must be a 1-d tensor of n_users + 1 offsets")
+        first, last = (int(x) for x in cand_off[[0, -1]].tolist())   # (a host read: a sync when on the device)
+        if first != 0 or last != n_cand:
+            raise ValueError(f"cand_off must run from 0 to the number of candidates ({n_cand}), got {first}..{last}")
+        if k > self.n_items:
+            raise ValueError(f"k={k} larger than the number of items ({self.n_items})")
+        device = self._check_ready()
+        n = cand_off.numel() - 1
+        cand_off = self._ids(cand_off.to(device), device)
+        users, items = self._ids(user_col, device), self._ids(item_col, device)
+        scores = self.predict({self.USER_ID: users, self.ITEM_ID: items})
+        ids = torch.empty(n, k, dtype=torch.int64, device=device) if want_ids else None
+        top = torch.empty(n, k, dtype=torch.float32, device=device) if want_scores else None
+        greater = equal = n_unmasked = None
+        if pos_off is not None:
+            pos_off, pos_items = self._ids(pos_off, device), self._ids(pos_items, device)
+            if pos_off.numel() != n + 1:
+                raise ValueError("pos_off must have n_users + 1 entries")
+            greater = torch.empty(pos_items.numel(), dtype=torch.int64, device=device)
+            equal = torch.empty_like(greater)
+            n_unmasked = torch.empty(n, dtype=torch.int64, device=device)
+        lib = _abi.lib()
+        need = lib.kge_candidate_select_workspace_bytes(n, n_cand)
+        ws = torch.empty(max(need, 8), dtype=torch.uint8, device=device)
+        _abi.check(
+            lib.kge_candidate_select(
+                scores.data_ptr(), items.data_ptr(), n_cand, cand_off.data_ptr(), n, self.n_items, _abi.ptr(pos_off),
+                _abi.ptr(pos_items), k, _abi.ptr(ids), _abi.ptr(top), _abi.ptr(greater), _abi.ptr(equal),
+                _abi.ptr(n_unmasked), ws.data_ptr(), ws.numel(), _abi.stream_ptr(),
+            ),
+            "kge_candidate_select",
+        )
+        return ids, top, greater, equal, n_unmasked
+
+    def candidate_topk(self, user_col, item_col, cand_off, k: int, return_scores: bool = True):
+        """Sampled evaluation's top-k without the [n_users, n_items] score matrix: ``predict`` on the candidate rows
+        (trainer.py ``_neg_sample_batch_eval``), the scatter into -inf rows and ``torch.topk`` (collector.py).
+
+        ``user_col`` / ``item_col`` are the loader's candidate rows (the interaction's user and item columns); row r
+        of the result is candidates ``[cand_off[r], cand_off[r+1])``, which may repeat an item (it counts once).
+        Returns (ids [n,k] int64, scores [n,k] fp32 or None) by (score desc, id asc) over the row's distinct
+        candidates; a row with fewer than k is padded with the smallest non-candidate ids, ascending, score -inf.
+        ``cand_off`` must run from 0 to the number of candidates (checked on the host)."""
+        ids, scores, *_ = self._candidate_select(user_col, item_col, cand_off, k, True, return_scores)
+        return ids, scores
+
+    def candidate_meanrank(self, user_col, item_col, cand_off, pos_off, pos_items):
+        """float32 [n, 3] rows ``(pos_rank_sum, user_len, pos_len)`` of the collector's ``rec.meanrank`` over the
+        scattered candidate rows (full_sort_meanrank's rows, for the rows candidate_topk sees): every non-candidate
+        scores -inf, ``user_len`` is the number of distinct candidates.  ``pos_off`` [n+1] / ``pos_items`` (sorted
+        per row) are the positives; a duplicate counts once."""
+        _, _, greater, equal, n_unmasked = self._candidate_select(user_col, item_col, cand_off, 1, False, False,
+                                                                  pos_off, pos_items)
+        return self._meanrank_rows(greater, equal, n_unmasked, pos_off, pos_items)
 
     def forward(self, *args, **kwargs):  # the reference's forward is the scorer on gathered rows
         raise NotImplementedError("use calculate_loss / predict / full_sort_predict")

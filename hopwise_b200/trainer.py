@@ -29,10 +29,14 @@ checkpoints, early stopping, logging are inherited unchanged) and overrides only
                             history / positives (built once per loader), the ``rec.topk`` rows -- and for GAUC the
                             ``rec.meanrank`` rows, from the exact full-catalogue ranks of the positives -- handed to
                             the reference ``Evaluator`` unchanged, so the metric dictionary is the reference's own.
-                            Anything the fused kernels do not cover (sampled evaluation, sequential loaders, the
-                            labelled value metrics that read ``rec.score`` / ``data.label``) goes through the
-                            inherited dense path.  Any cutoff is covered: above k = 128 the fused top-k keeps
-                            per-row buffers in a workspace instead of sorted lists in shared memory.
+                            Sampled ranking evaluation of the REC task (``eval_args.mode`` uniN / popN,
+                            ``NegSampleEvalDataLoader``) iterates the loader once, as the reference does, and
+                            selects over each user's candidate list (evaluator.collect_sampled) instead of
+                            scattering the scores into [batch_users, n_items] rows.  Anything the fused kernels do
+                            not cover (sampled link-prediction loaders, sequential loaders, the labelled value
+                            metrics that read ``rec.score`` / ``data.label``) goes through the inherited dense path.
+                            Any cutoff is covered: above k = 128 the fused top-k keeps per-row buffers in a
+                            workspace instead of sorted lists in shared memory.
 
 ``install()`` registers the classes with hopwise's own factories, so ``run_hopwise(model="TransE", ...)`` and the
 ``hopwise train`` CLI pick them up without edits: ``get_model`` (utils/utils.py:65-98) resolves
@@ -51,17 +55,17 @@ import numpy as np
 import torch
 
 try:
-    from hopwise.data.dataloader import FullSortLPEvalDataLoader, FullSortRecEvalDataLoader
+    from hopwise.data.dataloader import FullSortLPEvalDataLoader, FullSortRecEvalDataLoader, NegSampleEvalDataLoader
     from hopwise.data.dataloader.abstract_dataloader import NegSampleDataLoader
     from hopwise.data.dataloader.knowledge_dataloader import KGDataLoaderState
     from hopwise.trainer import KGTrainer
     from hopwise.trainer import trainer as _ref_trainer
-    from hopwise.utils import KnowledgeEvaluationType
+    from hopwise.utils import EvaluatorType, KnowledgeEvaluationType
 except ImportError as exc:  # pragma: no cover
     raise ImportError("hopwise_b200.trainer plugs into hopwise's trainer: hopwise must be importable") from exc
 
 from . import recommender as _rec
-from .evaluator import topk_hits
+from .evaluator import collect_sampled, topk_hits
 from .loader import DevicePrefetcher
 
 # hopwise's Config compares `model_class.type` / `.input_type` with ITS enums (configurator.py:219-224).  When
@@ -195,7 +199,36 @@ class FusedKGTrainer(KGTrainer):
         eval_data.__dict__["_kge_fused_plan"] = plan
         return plan
 
+    def _fused_sampled(self, eval_data, task) -> bool:
+        """Whether a sampled (uniN / popN) evaluation goes through the candidate-list selection."""
+        if not self.fused_eval or task != KnowledgeEvaluationType.REC:
+            return False
+        if not isinstance(eval_data, NegSampleEvalDataLoader) or getattr(eval_data, "is_sequential", False):
+            return False
+        if self.config["eval_type"] != EvaluatorType.RANKING or torch.device(self.device).type != "cuda":
+            return False
+        reg = self.eval_collector.register
+        return not any(reg.need(key) for key in ("rec.score", "data.label"))
+
+    def _sampled_eval_loop(self, eval_data):
+        collector, reg, struct = self.eval_collector, self.eval_collector.register, self.eval_collector.data_struct
+        # trainer.py _neg_sample_batch_eval + collector.py eval_batch_collect over all batches: one pass of the
+        # loader (it draws the negatives from the shared random stream), one selection call per user block
+        data, n_batches = collect_sampled(self.model, eval_data, max(collector.topk),
+                                          meanrank=bool(reg.need("rec.meanrank")), user_block=max(1, self.user_block))
+        for key in ("rec.users", "rec.items", "rec.topk", "rec.meanrank"):
+            if reg.need(key):
+                struct.update_tensor(key, data[key])
+        collector.model_collect(self.model)
+        result = self.evaluator.evaluate(collector.get_data_struct())
+        if not self.config["single_spec"]:
+            result = self._map_reduce(result, 4 * n_batches)   # as the full-sort branch below
+        self.wandblogger.log_eval_metrics(result, head="eval")
+        return result
+
     def evaluate_data_loop(self, eval_data, task, tot_target_num, target_tensor, show_progress=True):
+        if self._fused_sampled(eval_data, task):
+            return self._sampled_eval_loop(eval_data)
         plan = self._fused_plan(eval_data, task)
         if plan is None:
             return super().evaluate_data_loop(eval_data, task, tot_target_num, target_tensor,

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define KGE_ABI_VERSION 7
+#define KGE_ABI_VERSION 8
 
 typedef void* kge_stream_t; /* cudaStream_t */
 
@@ -303,6 +303,27 @@ int kge_full_sort_topk_mma(const kge_model_t* model, const int64_t* heads, const
  * Any k >= 1. */
 int kge_topk_hits(const int64_t* ids, int64_t n, int32_t k, const int64_t* pos_off, const int64_t* pos_items,
                   int32_t* out, kge_stream_t stream);
+
+/* ---- sampled evaluation (uni-N / pop-N) ---------------------------------------------------------------
+ * kge_candidate_select: what trainer.py's _neg_sample_batch_eval (torch.full(-inf) + the scatter of the candidate
+ * scores) and the collector's rec.topk / rec.meanrank branches read, from the candidate lists alone.  Row r's
+ * candidates are entries [cand_off[r], cand_off[r+1]) of scores / cand_items (cand_off[0] = 0, non-decreasing, ending
+ * at n_cand; offsets are clamped to [0, n_cand]); ids lie in [0, n_targets) and may repeat (a repeated id carries the
+ * same score and counts once); every other target of the row scores -inf.  Every output may be NULL:
+ *   ids_out[n,k] (int64) / scores_out[n,k]: the row's distinct candidates by (score desc, id asc); a row with fewer
+ *     than k of them is padded with the smallest non-candidate ids, ascending, score -inf (full-sort's order for
+ *     masked targets);
+ *   greater_out / equal_out (both or neither): for every entry of the positives CSR (pos_off[n+1], pos_items), the
+ *     counts of kge_full_sort_rank_counts over the row: a positive that is not a candidate scores -inf, so
+ *     greater = the distinct candidates and equal = n_targets - the distinct candidates;
+ *   n_unmasked_out[n]: the row's distinct candidates.
+ * Rows pick a warp, a CTA or the workspace to sort in on the device, by length.  1 <= k <= n_targets < 2^32 - 1.
+ * workspace: kge_candidate_select_workspace_bytes(n, n_cand) bytes. */
+int64_t kge_candidate_select_workspace_bytes(int64_t n, int64_t n_cand);
+int kge_candidate_select(const float* scores, const int64_t* cand_items, int64_t n_cand, const int64_t* cand_off,
+                         int64_t n, int64_t n_targets, const int64_t* pos_off, const int64_t* pos_items, int32_t k,
+                         int64_t* ids_out, float* scores_out, int64_t* greater_out, int64_t* equal_out,
+                         int64_t* n_unmasked_out, void* workspace, int64_t workspace_bytes, kge_stream_t stream);
 
 /* kge_topk_metric_sums: metrics.py:67-69,93-101,164-165,191-207,231-232 summed over users:
  * sums[5*k] float64 = per-cutoff sums of recall, mrr, ndcg, hit, precision (caller zeroes).
