@@ -14,14 +14,15 @@
 //   DistMult q = h * r                      score = q . t
 //   ComplEx  q = (hr*rr | hi*rr + hr*ri - hi*ri)   score = q . t        (complex.py:53-62 as written)
 //   TorusE   q = frac(h) + frac(r)          score = -4 * sum(min(x^2, 1 - x^2)), x = q - frac(t)
-// so one tile kernel serves them all: a CTA owns BU=32 query rows (q kept in shared memory for
-// the whole sweep) and streams target tiles of BT=128 rows through shared memory in K-chunks
-// of 32 floats; each thread accumulates a 4x4 register block.  The epilogue either stores
-// the dense [n, n_targets] scores (API parity: the unchanged trainer mutates that tensor) or
-// keeps a per-row sorted top-k list of 64-bit (score, ~id) keys in shared memory, so the dense
-// matrix never exists (800 GB at 1M x 200k).  Order: score descending, id ascending.  A third
-// epilogue counts, for listed targets (the positives), the targets scoring above and equal to
-// them over the whole masked row: the exact ranks GAUC reads (collector.py's rec.meanrank).
+// so one tile kernel serves them all: a CTA owns BU query rows (q kept in shared memory for
+// the whole sweep; BU = 32, or 16 when 32 rows of q do not fit) and streams target tiles of
+// BT=128 rows through shared memory in K-chunks of 32 floats; each thread accumulates a
+// (BU/8)x4 register block.  The epilogue either stores the dense [n, n_targets] scores (API
+// parity: the unchanged trainer mutates that tensor) or keeps a per-row sorted top-k list of
+// 64-bit (score, ~id) keys in shared memory, so the dense matrix never exists (800 GB at
+// 1M x 200k).  Order: score descending, id ascending.  A third epilogue counts, for listed
+// targets (the positives), the targets scoring above and equal to them over the whole masked
+// row: the exact ranks GAUC reads (collector.py's rec.meanrank).
 // TransH and TransD have no scorer here: transh_project_kernel / transd_project_kernel write projected rows, which
 // the caller scores as TransE (check_score_model refuses both model kinds).
 #include <math.h>
@@ -31,7 +32,6 @@
 
 namespace {
 
-constexpr int BU = 32;    // query rows per CTA
 constexpr int BT = 128;   // target rows per tile
 constexpr int KC = 32;    // K chunk (floats)
 constexpr int TS = KC + 4;  // padded row stride of the target tile: conflict-free LDS.128
@@ -297,6 +297,7 @@ __device__ __forceinline__ void block_bitonic_sort_desc(uint64_t* buf, int64_t P
     }
 }
 
+template <int BU>
 __device__ __forceinline__ void build_queries(const ScoreArgs& a, const int64_t* rowid, int nrows, int kpad, float* Qs) {
   const int d = a.m.d;
   const int parts = (a.m.model == KGE_ROTATE || a.m.model == KGE_COMPLEX) ? 2 : 1;
@@ -338,12 +339,15 @@ __device__ __forceinline__ void load_target_chunk(const float* __restrict__ W, i
 
 // MODE: how a (query, target) pair of rows is contracted (score_common.cuh).  EPI: what the sweep does with the scores.
 // The rank epilogue asks for two CTAs per SM (128 registers): under the compiler's default budget it spills.
-template <int MODE, int EPI>
+// BU: query rows per CTA (plan_tiles); warp w owns rows RU*w .. RU*w + RU-1 of the block.
+template <int MODE, int EPI, int BU>
 __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_TOPK_LARGE) ? 2 : 0) fullsort_tile_kernel(const TileArgs a) {
   constexpr bool DIST = MODE == MODE_DIST;
   constexpr bool TOPK = EPI == EPI_TOPK, RANK = EPI == EPI_RANK, LARGE = EPI == EPI_TOPK_LARGE;
   constexpr bool SEL = TOPK || LARGE;         // a top-k epilogue: candidate keys staged per tile
   constexpr bool MASKED = EPI != EPI_DENSE;   // the trainer's masking: column 0 and the history -> -inf
+  constexpr int RU = BU / (TILE_THREADS / 32);   // query rows of a thread's register block
+  static_assert(BU == 32 || BU == 16, "query blocks of 32 or 16 rows");
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int model = a.s.m.model;
   const int parts = (model == KGE_ROTATE || model == KGE_COMPLEX) ? 2 : 1;
@@ -372,7 +376,7 @@ __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_T
   if (RANK && a.pos_off[a.s.n] > a.rank_cap) return;   // (the workspace was sized for fewer positives)
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int tu = warp;  // users 4*tu .. 4*tu+3
+  const int tu = warp;  // users RU*tu .. RU*tu+RU-1
 
   const int64_t n_tiles = (a.n_targets + BT - 1) / BT;
   const int64_t tile_lo = (int64_t)blockIdx.y * a.tiles_per_split;
@@ -385,7 +389,7 @@ __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_T
   for (int u = threadIdx.x; u < BU; u += blockDim.x)
     rowid[u] = u < nrows ? (a.row_map ? (int64_t)__ldg(a.row_map + row0 + u) : row0 + u) : 0;
   __syncthreads();
-  build_queries(a.s, rowid, nrows, kpad, Qs);
+  build_queries<BU>(a.s, rowid, nrows, kpad, Qs);
   if (RANK) {
     for (int u = threadIdx.x; u < BU; u += blockDim.x) {
       int64_t base = 0, m = 0;
@@ -404,8 +408,8 @@ __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_T
       }
     }
   }
-  // unmasked targets and targets scoring -inf of the thread's four rows (rank epilogue)
-  uint32_t n_unm[4] = {0u, 0u, 0u, 0u}, n_ninf[4] = {0u, 0u, 0u, 0u};
+  // unmasked targets and targets scoring -inf of the thread's RU rows (rank epilogue)
+  uint32_t n_unm[RU] = {}, n_ninf[RU] = {};
   if (MASKED) {
     for (int u = threadIdx.x; u < BU; u += blockDim.x) {
       if (SEL) {
@@ -431,9 +435,9 @@ __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_T
 
   for (int64_t tile = tile_lo; tile < tile_hi; ++tile) {
     const int64_t t0 = tile * BT;
-    float acc[4][4];
+    float acc[RU][4];
 #pragma unroll
-    for (int x = 0; x < 4; ++x)
+    for (int x = 0; x < RU; ++x)
 #pragma unroll
       for (int y = 0; y < 4; ++y) acc[x][y] = 0.f;
 
@@ -470,16 +474,16 @@ __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_T
         __syncthreads();  // previous chunk consumed
         load_target_chunk<MODE == MODE_TORUS>(W, d, a.n_targets, t0, c0, Ts);
         __syncthreads();
-        const float* qbase = Qs + (4 * tu) * qstride + p * kpad + c0;
+        const float* qbase = Qs + (RU * tu) * qstride + p * kpad + c0;
 #pragma unroll
         for (int kk = 0; kk < KC; kk += 4) {
-          float4 qv[4], tv[4];
+          float4 qv[RU], tv[4];
 #pragma unroll
-          for (int x = 0; x < 4; ++x) qv[x] = *reinterpret_cast<const float4*>(qbase + x * qstride + kk);
+          for (int x = 0; x < RU; ++x) qv[x] = *reinterpret_cast<const float4*>(qbase + x * qstride + kk);
 #pragma unroll
           for (int y = 0; y < 4; ++y) tv[y] = *reinterpret_cast<const float4*>(Ts + (lane + 32 * y) * TS + kk);
 #pragma unroll
-          for (int x = 0; x < 4; ++x)
+          for (int x = 0; x < RU; ++x)
 #pragma unroll
             for (int y = 0; y < 4; ++y) {
               if (DIST) {
@@ -511,8 +515,8 @@ __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_T
     // ---- epilogue of this tile ------------------------------------------------------------
     const float margin = (model == KGE_ROTATE) ? a.s.m.margin : 0.f;
 #pragma unroll
-    for (int x = 0; x < 4; ++x) {
-      const int u = 4 * tu + x;
+    for (int x = 0; x < RU; ++x) {
+      const int u = RU * tu + x;
       if (u >= nrows) continue;
 #pragma unroll
       for (int y = 0; y < 4; ++y) {
@@ -633,8 +637,8 @@ __global__ void __launch_bounds__(TILE_THREADS, (EPI == EPI_RANK || EPI == EPI_T
   if (RANK) {
     // this split's counts, added exactly (integer atomics: the result does not depend on the order)
 #pragma unroll
-    for (int x = 0; x < 4; ++x) {
-      const int u = 4 * tu + x;
+    for (int x = 0; x < RU; ++x) {
+      const int u = RU * tu + x;
       const unsigned unm = __reduce_add_sync(0xffffffffu, n_unm[x]);
       const unsigned ninf = __reduce_add_sync(0xffffffffu, n_ninf[x]);
       if (lane == 0 && u < nrows) {
@@ -1079,29 +1083,42 @@ int check_score_model(const kge_model_t* m) {
   const int pr = m->model == KGE_COMPLEX ? 2 : 1;
   for (int p = 0; p < ph; ++p) KGE_REQUIRE(m->user.w[p] && m->entity.w[p], KGE_E_ARG, "NULL weight table");
   for (int p = 0; p < pr; ++p) KGE_REQUIRE(m->relation.w[p], KGE_E_ARG, "NULL relation table");
-  KGE_REQUIRE(m->d >= 1, KGE_E_UNSUPPORTED, "embedding_size %d unsupported", m->d);
+  KGE_REQUIRE(m->d >= 1 && m->d <= KGE_MAX_D, KGE_E_UNSUPPORTED, "embedding_size %d unsupported (1 to %d)", m->d,
+              KGE_MAX_D);
   return 0;
 }
 
 struct TilePlan {
-  int kpad, n_splits, tiles_per_split;
+  int kpad, bu, n_splits, tiles_per_split;
   size_t smem;
   int64_t n_blocks;
 };
 
-int plan_tiles(const kge_model_t* m, int64_t n, int64_t n_targets, int k, int epi, TilePlan& pl) {
-  const int parts = (m->model == KGE_ROTATE || m->model == KGE_COMPLEX) ? 2 : 1;
-  pl.kpad = (m->d + KC - 1) / KC * KC;
-  size_t smem = (size_t)BU * parts * pl.kpad * 4 + (size_t)BT * TS * 4;
+// Shared memory of the tile kernel with a query block of BU rows.
+size_t tile_smem(int BU, int parts, int kpad, int k, int epi) {
+  size_t smem = (size_t)BU * parts * kpad * 4 + (size_t)BT * TS * 4;
   if (epi == EPI_TOPK) smem += (size_t)BU * k * 8 + (size_t)BU * BT * 8 + BU * 8 + BU * (BT / 32) * 4 + BU * 4 * 2 + BU * 8;
   if (epi == EPI_TOPK_LARGE)   // the same without the lists: cand, thr, maskbits, cnt, llen, cursor
     smem += (size_t)BU * BT * 8 + BU * 8 + BU * (BT / 32) * 4 + BU * 4 * 2 + BU * 8;
   if (epi == EPI_RANK)   // maskbits, cursor | rbase, rthr, rcnt, rlo, rm
     smem += BU * (BT / 32) * 4 + BU * 8 + BU * 8 + (size_t)BU * RANK_SM * 4 * 3 + BU * 4 * 2;
   smem += BU * 8;   // rowid
+  return smem;
+}
+
+int plan_tiles(const kge_model_t* m, int64_t n, int64_t n_targets, int k, int epi, TilePlan& pl) {
+  KGE_REQUIRE(m->d >= 1 && m->d <= KGE_MAX_D, KGE_E_UNSUPPORTED, "embedding_size %d unsupported (1 to %d)", m->d,
+              KGE_MAX_D);
+  const int parts = (m->model == KGE_ROTATE || m->model == KGE_COMPLEX) ? 2 : 1;
+  pl.kpad = (m->d + KC - 1) / KC * KC;
+  // 32 query rows where they fit; 16 above (the two-part models from d = 545 to 801 on, by epilogue and k).  Sixteen
+  // rows need at most 183 KB (parts * kpad = 2,048, k = 128), so no smaller block is needed up to KGE_MAX_D.
+  pl.bu = 32;
+  if (tile_smem(32, parts, pl.kpad, k, epi) > 220 * 1024) pl.bu = 16;
+  const size_t smem = tile_smem(pl.bu, parts, pl.kpad, k, epi);
   pl.smem = smem;
   KGE_REQUIRE(smem <= 220 * 1024, KGE_E_UNSUPPORTED, "embedding_size %d needs %zu bytes of shared memory", m->d, smem);
-  pl.n_blocks = (n + BU - 1) / BU;
+  pl.n_blocks = (n + pl.bu - 1) / pl.bu;
   const int64_t n_tiles = (n_targets + BT - 1) / BT;
   int splits = 1;
   if (epi != EPI_DENSE) {
@@ -1137,7 +1154,8 @@ extern "C" int kge_predict(const kge_model_t* model, const int64_t* heads, const
   if (n == 0) return 0;
   KGE_REQUIRE(heads && tails && out, KGE_E_ARG, "NULL heads / tails / out");
   RowCfg c = {};
-  KGE_REQUIRE(kge_pick_rowcfg(model->d, c), KGE_E_UNSUPPORTED, "embedding_size %d unsupported", model->d);
+  KGE_REQUIRE(kge_pick_rowcfg(model->d, c), KGE_E_UNSUPPORTED, "embedding_size %d unsupported (1 to %d)", model->d,
+              KGE_MAX_D);
   ScoreArgs a;
   a.m = *model;
   a.heads = heads;
@@ -1172,7 +1190,7 @@ extern "C" int kge_transd_project(const float* emb, const float* vec, const int6
   if (n == 0) return 0;
   KGE_REQUIRE(emb && vec && rel_vec && out && (rel_ids || rel_row >= 0), KGE_E_ARG, "NULL argument");
   RowCfg c = {};
-  KGE_REQUIRE(kge_pick_rowcfg(d, c), KGE_E_UNSUPPORTED, "embedding_size %d unsupported", d);
+  KGE_REQUIRE(kge_pick_rowcfg(d, c), KGE_E_UNSUPPORTED, "embedding_size %d unsupported (1 to %d)", d, KGE_MAX_D);
   const int threads = 256;
   int64_t g = (n + threads / c.g - 1) / (threads / c.g);
   const int64_t cap = (int64_t)kge_num_sms() * 8;
@@ -1192,7 +1210,7 @@ extern "C" int kge_transh_project(const float* emb, const int64_t* ids, int64_t 
   if (n == 0) return 0;
   KGE_REQUIRE(emb && norm_vec && out && (rel_ids || rel_row >= 0), KGE_E_ARG, "NULL argument");
   RowCfg c = {};
-  KGE_REQUIRE(kge_pick_rowcfg(d, c), KGE_E_UNSUPPORTED, "embedding_size %d unsupported", d);
+  KGE_REQUIRE(kge_pick_rowcfg(d, c), KGE_E_UNSUPPORTED, "embedding_size %d unsupported (1 to %d)", d, KGE_MAX_D);
   const int threads = 256;
   int64_t g = (n + threads / c.g - 1) / (threads / c.g);
   const int64_t cap = (int64_t)kge_num_sms() * 8;
@@ -1207,9 +1225,9 @@ extern "C" int kge_transh_project(const float* emb, const int64_t* ids, int64_t 
 
 template <int MODE, int EPI>
 static int launch_tile(const TileArgs& a, const TilePlan& pl, cudaStream_t st) {
-  auto kern = fullsort_tile_kernel<MODE, EPI>;
+  auto kern = pl.bu == 32 ? fullsort_tile_kernel<MODE, EPI, 32> : fullsort_tile_kernel<MODE, EPI, 16>;
   KGE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
-  // blockIdx.x is limited to 2^31-1 rows/BU: fine for any table that fits the device
+  // blockIdx.x is limited to 2^31-1 rows/pl.bu: fine for any table that fits the device
   dim3 grid((unsigned)pl.n_blocks, (unsigned)pl.n_splits);
   kern<<<grid, TILE_THREADS, pl.smem, st>>>(a);
   KGE_LAUNCH_CHECK();
@@ -1472,9 +1490,13 @@ int kge_topk_rows_indirect(const kge_model_t* model, const int64_t* heads, const
   a.row_map = row_map;
   a.row_count = row_count;
   const int mode = tile_mode(model->model);
-  auto kern = mode == MODE_DIST ? fullsort_tile_kernel<MODE_DIST, EPI_TOPK>
-                                : (mode == MODE_TORUS ? fullsort_tile_kernel<MODE_TORUS, EPI_TOPK>
-                                                      : fullsort_tile_kernel<MODE_DOT, EPI_TOPK>);
+  const int bu = fp.tp.bu;
+  auto kern = bu == 32 ? (mode == MODE_DIST ? fullsort_tile_kernel<MODE_DIST, EPI_TOPK, 32>
+                                            : (mode == MODE_TORUS ? fullsort_tile_kernel<MODE_TORUS, EPI_TOPK, 32>
+                                                                  : fullsort_tile_kernel<MODE_DOT, EPI_TOPK, 32>))
+                       : (mode == MODE_DIST ? fullsort_tile_kernel<MODE_DIST, EPI_TOPK, 16>
+                                            : (mode == MODE_TORUS ? fullsort_tile_kernel<MODE_TORUS, EPI_TOPK, 16>
+                                                                  : fullsort_tile_kernel<MODE_DOT, EPI_TOPK, 16>));
   KGE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fp.tp.smem));
   const int warps = 8;
   const int64_t ra = n < FB_SPLIT_ROWS ? n : FB_SPLIT_ROWS;
@@ -1485,7 +1507,7 @@ int kge_topk_rows_indirect(const kge_model_t* model, const int64_t* heads, const
   a.tiles_per_split = fp.tiles_per_split;
   a.row_begin = 0;
   a.row_end = ra;
-  kern<<<dim3((unsigned)((ra + BU - 1) / BU), (unsigned)fp.splits), TILE_THREADS, fp.tp.smem, st>>>(a);
+  kern<<<dim3((unsigned)((ra + bu - 1) / bu), (unsigned)fp.splits), TILE_THREADS, fp.tp.smem, st>>>(a);
   KGE_LAUNCH_CHECK();
   topk_merge_kernel<<<(unsigned)((ra + warps - 1) / warps), warps * 32, (size_t)warps * k * 8, st>>>(
       a.part_keys, n, a.n_splits, k, ids_out, scores_out, row_map, row_count, 0, ra);
@@ -1496,7 +1518,7 @@ int kge_topk_rows_indirect(const kge_model_t* model, const int64_t* heads, const
     a.tiles_per_split = (int)((n_targets + BT - 1) / BT);
     a.row_begin = ra;
     a.row_end = n;
-    int64_t g = (n - ra + BU - 1) / BU;
+    int64_t g = (n - ra + bu - 1) / bu;
     const int64_t cap = (int64_t)kge_num_sms() * 2;
     if (g > cap) g = cap;
     kern<<<dim3((unsigned)g, 1), TILE_THREADS, fp.tp.smem, st>>>(a);

@@ -1025,7 +1025,7 @@ int check_model(const kge_model_t* m, bool need_state, bool need_rows = true) {
   for (int p = 0; p < pr; ++p) KGE_REQUIRE(m->relation.w[p], KGE_E_ARG, "NULL relation table");
   RowCfg c = {};
   KGE_REQUIRE(kge_pick_rowcfg(m->d, c), KGE_E_UNSUPPORTED,
-              "embedding_size %d unsupported (max 512, or 256 when not a multiple of 4)", m->d);
+              "embedding_size %d unsupported (1 to %d)", m->d, KGE_MAX_D);
   if (need_state) {
     KGE_REQUIRE(table_has_state(m->user, need_rows) && table_has_state(m->entity, need_rows) &&
                     table_has_state(m->relation, need_rows), KGE_E_STATE, "optimiser state buffers missing");

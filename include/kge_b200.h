@@ -73,7 +73,7 @@ typedef struct {
 
 typedef struct {
   int32_t model;                /* enum kge_model_kind */
-  int32_t d;                    /* embedding_size */
+  int32_t d;                    /* embedding_size, 1 .. 1024 on every entry point */
   float margin;                 /* TransE / DistMult / RotatE */
   int32_t ui_relation;          /* relation row for user->item triples in loss / predict
                                    (transe.py:63, distmult.py:57: weight[-1]; rotate.py:43,
