@@ -77,11 +77,11 @@ class kge_adam_t(C.Structure):
         ("step", C.c_int32),
         ("replay_cap", C.c_int32),
         ("optimizer", C.c_int32),
-        ("reserved", C.c_int32),
+        ("weight_decay", C.c_float),
     ]
 
 
-OPTIMIZERS = {"adam": 0, "sgd": 1, "adagrad": 2, "rmsprop": 3}   # enum kge_optimizer
+OPTIMIZERS = {"adam": 0, "sgd": 1, "adagrad": 2, "rmsprop": 3, "adamw": 4}   # enum kge_optimizer
 
 
 _P = C.c_void_p

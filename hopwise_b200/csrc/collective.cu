@@ -129,8 +129,9 @@ __global__ void __launch_bounds__(256) multimem_all_reduce_fused_kernel(float* _
 // the SUM of the N gradient copies of its slice straight from the switch (multimem.ld_reduce), takes the Adam step for
 // those elements with its (sharded) moments, and multicasts the new weights to every
 // replica (multimem.st).  Every rank moves 1/N of the gradient in and 1/N of the weights out, and does 1/N of the
-// optimiser arithmetic; torch.optim.Adam's dense semantics (every element, every step), which is what the reference
-// trains with (trainer/trainer.py:131-170 builds optim.Adam over all parameters; DDP averages the gradients first).
+// optimiser arithmetic; torch.optim.Adam's (or AdamW's) dense semantics (every element, every step), which is what the
+// reference trains with (trainer/trainer.py:131-170 builds optim.Adam over all parameters; DDP averages the gradients
+// first).
 struct OwnerAdam {
   float* g_mc;        // multicast address of the flat gradient buffer
   float* w_mc;        // multicast address of the flat weight buffer
@@ -141,6 +142,8 @@ struct OwnerAdam {
   float scale;        // 1 / world (DDP's mean) times the caller's loss scale
   float lr_c, rsq_c;  // lr / (1 - b1^t), 1 / sqrt(1 - b2^t)
   float b2, omb1, omb2, eps;
+  int decays;         // AdamW: the weights are multiplied by `decay` = fp32(1 - lr * weight_decay) first
+  float decay;
 };
 
 __device__ __forceinline__ void owner_adam_quad(const OwnerAdam& a, int64_t q, float4 g, float4 w4, float4 m4,
@@ -150,6 +153,7 @@ __device__ __forceinline__ void owner_adam_quad(const OwnerAdam& a, int64_t q, f
 #pragma unroll
   for (int e = 0; e < 4; ++e) {   // the arithmetic of adam_row (train.cu), element for element
     const float ge = gv[e] * a.scale;
+    if (a.decays) wv[e] *= a.decay;
     mv[e] += a.omb1 * (ge - mv[e]);
     vv[e] = vv[e] * a.b2 + a.omb2 * ge * ge;
     const float den = sqrt_nonneg(vv[e]) * a.rsq_c + a.eps;
@@ -276,6 +280,9 @@ extern "C" int kge_owner_adam_step(void* grad_multicast, float* grad_local, void
                 reinterpret_cast<uintptr_t>(v)) & 15) == 0, KGE_E_ARG, "buffers must be 16-byte aligned");
   KGE_REQUIRE(signal_pads_dev && local_flags && slot_base >= 0 && epoch != 0 && adam->step >= 1, KGE_E_ARG,
               "bad barrier / step arguments");
+  if (int e = kge_check_optimizer(adam)) return e;
+  KGE_REQUIRE(adam->optimizer == KGE_OPT_ADAM || adam->optimizer == KGE_OPT_ADAMW, KGE_E_UNSUPPORTED,
+              "the owner-sharded step implements Adam and AdamW (optimizer %d)", adam->optimizer);
   const int64_t quads = n_floats / 4;
   const int64_t per = (quads + world - 1) / world;
   const int64_t lo = per * rank < quads ? per * rank : quads, hi = lo + per < quads ? lo + per : quads;
@@ -296,6 +303,8 @@ extern "C" int kge_owner_adam_step(void* grad_multicast, float* grad_local, void
   a.omb1 = (float)(1.0 - (double)adam->beta1);
   a.omb2 = (float)(1.0 - (double)adam->beta2);
   a.eps = adam->eps;
+  a.decays = adam->weight_decay != 0.f;   // (AdamW: kge_check_optimizer refuses decay under Adam)
+  a.decay = (float)(1.0 - (double)adam->lr * (double)adam->weight_decay);
   const int threads = 256;
   int64_t grid = hi > lo ? (hi - lo + threads - 1) / threads : 1;   // (a thread per quad until the grid is full)
   const int64_t cap = (int64_t)kge_num_sms() * 2;   // co-resident at 128 registers (the grid spins on a flag block 0 raises)

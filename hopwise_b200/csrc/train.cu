@@ -24,6 +24,8 @@
 // Kernel B (adam_apply_kernel): lanes scan row_state (8 B per row, coalesced), ballot the rows
 // marked in this step and a lane group updates each: replay the zero-gradient steps the row
 // skipped (dense Adam keeps moving a row after its last gradient), apply the real step, zero g.
+// Weight decay (AdamW, SGD) moves every row in every step, touched or not: it is replayed the same way, and every
+// kernel that brings rows up to date has an instantiation with it (DECAY) and one without.
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
@@ -38,9 +40,12 @@ struct AdamDev {
   float lr, b1, b2, eps, omb1, omb2;
   int step;  // update being produced
   int cap;
-  int opt;   // enum kge_optimizer
+  int opt;   // enum kge_optimizer; AdamW runs as KGE_OPT_ADAM with `decays` set
   const float2* table;  // {lr/(1-b1^j), 1/sqrt(1-b2^j)}
   int tlen;
+  int decays;   // weight decay on (AdamW, or SGD with weight_decay > 0): every row moves in every step
+  float decay;  // AdamW: f = fp32(1 - lr * weight_decay), the factor of one step (also the closed-form tail's base)
+  float wd;     // SGD: weight_decay
 };
 struct TrainArgs {
   kge_model_t m;
@@ -57,11 +62,20 @@ __device__ __forceinline__ float2 adam_consts(const AdamDev& A, int j) {
   return make_float2(A.lr, 1.f);
 }
 
+// f^n for n >= 0 by squaring: any sign of f (powf is NaN for f < 0, and lr * weight_decay >= 1 gives f <= 0)
+__device__ __forceinline__ float pow_int(float f, int n) {
+  float r = 1.f;
+  for (; n > 0; n >>= 1, f *= f)
+    if (n & 1) r *= f;
+  return r;
+}
+
 // Zero-gradient Adam steps s+1 .. t_end on one row fragment (torch.optim.Adam with g = 0:
-// m.lerp_(0, 1-b1); v.mul_(b2); p.addcdiv_(m, sqrt(v)/sqrt(1-b2^j) + eps, -lr/(1-b1^j))).
+// m.lerp_(0, 1-b1); v.mul_(b2); p.addcdiv_(m, sqrt(v)/sqrt(1-b2^j) + eps, -lr/(1-b1^j))), each after
+// AdamW's p.mul_(1 - lr * weight_decay) under DECAY (weight decay on: AdamDev::decays).
 // After `cap` steps m has decayed by b1^cap (7e-10 at cap 200) and the remaining movement is
-// below fp32 resolution of the weights; m and v then decay in closed form.
-template <int E>
+// below fp32 resolution of the weights; m and v then decay in closed form, and the weights by f^n.
+template <int E, bool DECAY>
 __device__ __forceinline__ void adam_replay(float (&p)[E], float (&m)[E], float (&v)[E], int s, int t_end,
                                             const AdamDev& A) {
   const int n = t_end - s;
@@ -71,6 +85,7 @@ __device__ __forceinline__ void adam_replay(float (&p)[E], float (&m)[E], float 
     const float2 c = adam_consts(A, j);
 #pragma unroll
     for (int e = 0; e < E; ++e) {
+      if (DECAY) p[e] *= A.decay;
       m[e] -= A.omb1 * m[e];
       v[e] *= A.b2;
       const float den = sqrt_approx(v[e]) * c.y + A.eps;
@@ -79,11 +94,32 @@ __device__ __forceinline__ void adam_replay(float (&p)[E], float (&m)[E], float 
   }
   if (n > nrep) {
     const float f1 = powf(A.b1, (float)(n - nrep)), f2 = powf(A.b2, (float)(n - nrep));
+    const float fp = DECAY ? pow_int(A.decay, n - nrep) : 1.f;
 #pragma unroll
     for (int e = 0; e < E; ++e) {
       m[e] *= f1;
       v[e] *= f2;
+      if (DECAY) p[e] *= fp;
     }
+  }
+}
+
+// n steps of weight decay alone on one row fragment (A.decays): SGD's idle step p.add_(wd * p, alpha=-lr), or AdamW on
+// a row whose moments are zero (no gradient has reached it yet, so its Adam step is zero) p.mul_(f).  `cap` steps
+// exactly, then the closed-form tail p *= f^(n - cap).
+template <int E>
+__device__ __forceinline__ void decay_replay(float (&p)[E], int n, const AdamDev& A) {
+  if (n <= 0) return;
+  const int nrep = n < A.cap ? n : A.cap;
+  const bool sgd = A.opt == KGE_OPT_SGD;
+  for (int j = 0; j < nrep; ++j) {
+#pragma unroll
+    for (int e = 0; e < E; ++e) p[e] = sgd ? __fmaf_rn(-A.lr, A.wd * p[e], p[e]) : p[e] * A.decay;
+  }
+  if (n > nrep) {
+    const float fp = pow_int(A.decay, n - nrep);
+#pragma unroll
+    for (int e = 0; e < E; ++e) p[e] *= fp;
   }
 }
 
@@ -105,7 +141,10 @@ __device__ __forceinline__ void touch_row(const kge_table_t& T, int64_t row, int
 // the Adam kernel then brings it up to date with a zero-gradient step (exactly what dense Adam does to it), so
 // the lag of a row that keeps being referenced by inactive triples stays bounded -- without this every forward
 // pass would replay the same (growing, up to the cap) run of skipped steps for it again.
-template <int VEC, int G, int NCH>
+// DECAY: weight decay is on (AdamDev::decays); every row then moves in every step, also one no gradient has reached.
+// It is a template parameter of the kernels so that their register-tuned instantiations without decay carry none of
+// its code.
+template <int VEC, int G, int NCH, bool DECAY>
 __device__ __forceinline__ void catch_up(const kge_table_t& T, int part, int64_t row, int2 st, int d, int gl,
                                          const AdamDev& A, float (&x)[VEC * NCH], int mark) {
   const int last = st.x;
@@ -113,8 +152,12 @@ __device__ __forceinline__ void catch_up(const kge_table_t& T, int part, int64_t
     float m[VEC * NCH], v[VEC * NCH];
     frag_load<VEC, G, NCH>(T.m[part], row, d, gl, m);
     frag_load<VEC, G, NCH>(T.v[part], row, d, gl, v);
-    adam_replay<VEC * NCH>(x, m, v, last, A.step - 1, A);
+    adam_replay<VEC * NCH, DECAY>(x, m, v, last, A.step - 1, A);
     if (mark && part == 0) touch_row(T, row, st.y, A.step, gl);   // (last >= 0: the table has states)
+  } else if (DECAY && last < A.step - 1 && T.row_state) {
+    // weight decay alone: SGD's, or AdamW's on a row no gradient has reached (last = -1: decayed since step 0)
+    decay_replay<VEC * NCH>(x, A.step - 1 - (last < 0 ? 0 : last), A);
+    if (mark && part == 0) touch_row(T, row, st.y, A.step, gl);
   }
 }
 
@@ -144,7 +187,7 @@ inline size_t warp_racc_smem_bytes(int64_t rows, int parts, int d) {
 // shared memory with plain loads and stores and leave once per CTA, one float4 RED per 4 columns of each touched
 // row -- instead of one RED per triple onto the few lines of the ~20 KG relation rows, which every L2 slice holding
 // them has to serialise.  (A CTA-wide copy would need float atomics on shared memory: a CAS loop on sm_100a.)
-template <int MODEL, int VEC, int G, int NCH, bool WARP_RACC = false>
+template <int MODEL, int VEC, int G, int NCH, bool WARP_RACC = false, bool DECAY = false>
 __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) train_fwd_kernel(const TrainArgs a) {
   constexpr int E = VEC * NCH;
   constexpr int PH = (MODEL == KGE_ROTATE || MODEL == KGE_COMPLEX || MODEL == KGE_TRANSD) ? 2 : 1;  // head / tail parts
@@ -231,11 +274,11 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
 #pragma unroll
     for (int p = 0; p < PH; ++p) frag_load<VEC, G, NCH>(ET.w[p], tn_id, d, gl, tnx[p]);
 #pragma unroll
-    for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH>(HT, p, h_id, sh, d, gl, a.adam, h[p], a.with_grad);
+    for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH, DECAY>(HT, p, h_id, sh, d, gl, a.adam, h[p], a.with_grad);
 #pragma unroll
-    for (int p = 0; p < PR; ++p) catch_up<VEC, G, NCH>(RT, p, r_id, sr, d, gl, a.adam, r[p], a.with_grad);
+    for (int p = 0; p < PR; ++p) catch_up<VEC, G, NCH, DECAY>(RT, p, r_id, sr, d, gl, a.adam, r[p], a.with_grad);
 #pragma unroll
-    for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH>(ET, p, tp_id, stp, d, gl, a.adam, tp[p], a.with_grad);
+    for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH, DECAY>(ET, p, tp_id, stp, d, gl, a.adam, tp[p], a.with_grad);
 
     // gradient fragments of the anchor, relation and positive tail
     float gh[PH][E], gr[PR][E], gtp[PH][E];
@@ -380,7 +423,7 @@ __global__ void __launch_bounds__(256, FwdBounds<MODEL, VEC, G, NCH>::MIN_CTAS) 
           for (int p = 0; p < PH; ++p) frag_load<VEC, G, NCH>(ET.w[p], tn_id, d, gl, tnx[p]);
         }
 #pragma unroll
-        for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH>(ET, p, t_id, st, d, gl, a.adam, t[p], a.with_grad);
+        for (int p = 0; p < PH; ++p) catch_up<VEC, G, NCH, DECAY>(ET, p, t_id, st, d, gl, a.adam, t[p], a.with_grad);
       }
 
       if (MODEL == KGE_TRANSD) {
@@ -800,7 +843,7 @@ struct ApplyArgs {
   int win[3];              // scan window per table
 };
 
-template <int VEC, int G, int NCH>
+template <int VEC, int G, int NCH, bool DECAY>
 __device__ __forceinline__ void adam_row(const kge_table_t& T, int64_t row, int last, int d, int gl, const AdamDev& A,
                                          float scale) {
   constexpr int E = VEC * NCH;
@@ -817,10 +860,12 @@ __device__ __forceinline__ void adam_row(const kge_table_t& T, int64_t row, int 
     frag_load_cg<VEC, G, NCH>(T.g[part], row, d, gl, g);
     float z[E];
     if (A.opt == KGE_OPT_ADAM) {
-      if (last >= 0 && last < A.step - 1) adam_replay<E>(p, m, v, last, A.step - 1, A);
+      if (last >= 0 && last < A.step - 1) adam_replay<E, DECAY>(p, m, v, last, A.step - 1, A);
+      else if (DECAY && last < 0) decay_replay<E>(p, A.step - 1, A);   // (AdamW, first gradient: m = v = 0)
 #pragma unroll
       for (int e = 0; e < E; ++e) {
         const float ge = g[e] * scale;
+        if (DECAY) p[e] *= A.decay;
         m[e] += A.omb1 * (ge - m[e]);
         v[e] = v[e] * A.b2 + A.omb2 * ge * ge;
         const float den = sqrt_nonneg(v[e]) * c.y + A.eps;
@@ -829,11 +874,13 @@ __device__ __forceinline__ void adam_row(const kge_table_t& T, int64_t row, int 
       }
       frag_store<VEC, G, NCH>(T.m[part], row, d, gl, m);
     } else {
+      if (DECAY) decay_replay<E>(p, A.step - 1 - (last < 0 ? 0 : last), A);   // (SGD: the skipped steps' decay)
 #pragma unroll
       for (int e = 0; e < E; ++e) {
         const float ge = g[e] * scale;
         if (A.opt == KGE_OPT_SGD) {
-          p[e] -= A.lr * ge;
+          if (DECAY) p[e] = __fmaf_rn(-A.lr, __fmaf_rn(A.wd, p[e], ge), p[e]);   // p -= lr * (g + wd * p)
+          else p[e] -= A.lr * ge;
         } else {
           v[e] = A.opt == KGE_OPT_ADAGRAD ? __fmaf_rn(ge, ge, v[e]) : __fmaf_rn(A.omb2 * ge, ge, v[e] * lag_decay * A.b2);
           p[e] -= A.lr * div_pos_den(ge, sqrt_nonneg(v[e]) + A.eps);
@@ -848,7 +895,7 @@ __device__ __forceinline__ void adam_row(const kge_table_t& T, int64_t row, int 
   if (gl == 0) T.row_state[2 * row] = A.step;  // last_step; touch_step keeps `step` (stale from step+1 on)
 }
 
-template <int VEC, int G, int NCH>
+template <int VEC, int G, int NCH, bool DECAY>
 __global__ void __launch_bounds__(256) adam_apply_kernel(const ApplyArgs a) {
   const int gl = (threadIdx.x & 31) % G;
   const int step = a.adam.step;
@@ -856,27 +903,34 @@ __global__ void __launch_bounds__(256) adam_apply_kernel(const ApplyArgs a) {
   auto marked = [step](int2 st) { return st.y == step; };
   // (the tables are kernel parameters: index them by name, a pointer array would copy them to local memory)
   for_selected_rows<G>(a.m.user, a.win[0], marked, [&](int64_t row, int last) {
-    adam_row<VEC, G, NCH>(a.m.user, row, last, a.m.d, gl, a.adam, scale);
+    adam_row<VEC, G, NCH, DECAY>(a.m.user, row, last, a.m.d, gl, a.adam, scale);
   });
   for_selected_rows<G>(a.m.entity, a.win[1], marked, [&](int64_t row, int last) {
-    adam_row<VEC, G, NCH>(a.m.entity, row, last, a.m.d, gl, a.adam, scale);
+    adam_row<VEC, G, NCH, DECAY>(a.m.entity, row, last, a.m.d, gl, a.adam, scale);
   });
   for_selected_rows<G>(a.m.relation, a.win[2], marked, [&](int64_t row, int last) {
-    adam_row<VEC, G, NCH>(a.m.relation, row, last, a.m.d, gl, a.adam, scale);
+    adam_row<VEC, G, NCH, DECAY>(a.m.relation, row, last, a.m.d, gl, a.adam, scale);
   });
 }
 
 // ---- dense catch-up of every row to adam.step (before weights are read by others) ------------
-template <int VEC, int G, int NCH>
+template <int VEC, int G, int NCH, bool DECAY>
 __global__ void __launch_bounds__(256) adam_flush_kernel(const kge_table_t T, int d, const AdamDev A, int win) {
   constexpr int E = VEC * NCH;
   const int gl = (threadIdx.x & 31) % G;
   const int step = A.step;
+  // (with weight decay every row lags, including those no gradient has reached: last = -1, current for step 0)
   for_selected_rows<G>(
-      T, win, [step](int2 st) { return st.x >= 0 && st.x < step; },
+      T, win, [step](int2 st) { return st.x < step && (st.x >= 0 || DECAY); },
       [&](int64_t row, int last) {
         for (int part = 0; part < T.parts; ++part) {
           float p[E], m[E], v[E];
+          if (DECAY && (A.opt != KGE_OPT_ADAM || last < 0)) {   // decay alone: SGD, or AdamW with m = v = 0
+            frag_load<VEC, G, NCH>(T.w[part], row, d, gl, p);
+            decay_replay<E>(p, A.step - (last < 0 ? 0 : last), A);
+            frag_store<VEC, G, NCH>(T.w[part], row, d, gl, p);
+            continue;
+          }
           if (A.opt != KGE_OPT_ADAM) {   // the weights of an idle row do not move; RMSprop's second moment decays
             if (A.opt == KGE_OPT_RMSPROP) {
               frag_load<VEC, G, NCH>(T.v[part], row, d, gl, v);
@@ -890,7 +944,7 @@ __global__ void __launch_bounds__(256) adam_flush_kernel(const kge_table_t T, in
           frag_load<VEC, G, NCH>(T.w[part], row, d, gl, p);
           frag_load<VEC, G, NCH>(T.m[part], row, d, gl, m);
           frag_load<VEC, G, NCH>(T.v[part], row, d, gl, v);
-          adam_replay<E>(p, m, v, last, A.step, A);
+          adam_replay<E, DECAY>(p, m, v, last, A.step, A);
           frag_store<VEC, G, NCH>(T.w[part], row, d, gl, p);
           frag_store<VEC, G, NCH>(T.m[part], row, d, gl, m);
           frag_store<VEC, G, NCH>(T.v[part], row, d, gl, v);
@@ -982,12 +1036,34 @@ AdamDev make_adam_dev(const kge_model_t* m, const kge_adam_t* a) {
   A.omb1 = (float)(1.0 - (double)a->beta1);
   A.omb2 = (float)(1.0 - (double)a->beta2);
   A.step = a->step;
-  A.opt = a->optimizer;
+  A.opt = a->optimizer == KGE_OPT_ADAMW ? KGE_OPT_ADAM : a->optimizer;
   A.cap = a->replay_cap > 0 ? a->replay_cap : 200;
   A.table = reinterpret_cast<const float2*>(m->adam_table);
   A.tlen = m->adam_table ? m->adam_table_len : 0;
+  // (kge_check_optimizer admits weight decay under AdamW and SGD only)
+  A.decays = a->weight_decay != 0.f;
+  A.wd = a->weight_decay;
+  A.decay = (float)(1.0 - (double)a->lr * (double)a->weight_decay);   // torch: param.mul_(1 - lr * weight_decay)
   return A;
 }
+
+}  // namespace
+
+int kge_check_optimizer(const kge_adam_t* a) {
+  KGE_REQUIRE(a, KGE_E_ARG, "adam is NULL");
+  KGE_REQUIRE(a->optimizer >= KGE_OPT_ADAM && a->optimizer <= KGE_OPT_ADAMW, KGE_E_ARG, "unknown optimizer %d",
+              a->optimizer);
+  KGE_REQUIRE(isfinite(a->weight_decay) && a->weight_decay >= 0.f, KGE_E_UNSUPPORTED,
+              "weight_decay %g unsupported (finite and >= 0)", (double)a->weight_decay);
+  KGE_REQUIRE(a->weight_decay == 0.f || a->optimizer == KGE_OPT_ADAMW || a->optimizer == KGE_OPT_SGD,
+              KGE_E_UNSUPPORTED,
+              "weight_decay %g under optimizer %d unsupported: the coupled L2 term of Adam, Adagrad and RMSprop moves "
+              "every element every step (no row-lazy form); weight decay is supported with KGE_OPT_ADAMW "
+              "(decoupled) and KGE_OPT_SGD", (double)a->weight_decay, a->optimizer);
+  return 0;
+}
+
+namespace {
 
 int grid_for(int64_t n_groups_needed, int groups_per_cta, int ctas_per_sm) {
   int64_t g = (n_groups_needed + groups_per_cta - 1) / groups_per_cta;
@@ -1060,8 +1136,7 @@ extern "C" int kge_train_forward(const kge_model_t* model, const kge_batch_t* b,
   KGE_REQUIRE(b && adam && loss_out, KGE_E_ARG, "NULL batch / adam / loss_out");
   KGE_REQUIRE(b->n_rec >= 0 && b->n_kg >= 0 && b->k_rec >= 1 && b->k_kg >= 1, KGE_E_ARG, "bad batch sizes");
   KGE_REQUIRE(adam->step >= 1, KGE_E_ARG, "adam.step is 1-based");
-  KGE_REQUIRE(adam->optimizer >= KGE_OPT_ADAM && adam->optimizer <= KGE_OPT_RMSPROP, KGE_E_ARG, "unknown optimizer %d",
-              adam->optimizer);
+  if (int e = kge_check_optimizer(adam)) return e;
   const int64_t n_total = b->n_rec + b->n_kg;
   if (n_total == 0) return 0;
   KGE_REQUIRE(b->n_rec == 0 || (b->user && b->item && b->neg_item), KGE_E_ARG, "NULL rec id array");
@@ -1111,53 +1186,59 @@ extern "C" int kge_train_forward(const kge_model_t* model, const kge_batch_t* b,
   // Two triples per warp with gradients: relation gradients go through per-warp copies in shared memory when those
   // fit at the residency the kernel's register budget is shaped for.  The grid is then sized to what is resident,
   // so that every CTA zeroes and flushes its copies once.
-  bool warp_racc = false;
-  if (two_per_warp && with_grad) {
-    const size_t ws = warp_racc_smem_bytes(model->relation.rows, model->relation.parts, model->d);
-    auto kern = kind == KGE_TRANSE ? train_fwd_kernel<KGE_TRANSE, 4, 16, 2, true>
-                                   : train_fwd_kernel<KGE_DISTMULT, 4, 16, 2, true>;
-    const int min_ctas = kind == KGE_TRANSE ? FwdBounds<KGE_TRANSE, 4, 16, 2>::MIN_CTAS
-                                            : FwdBounds<KGE_DISTMULT, 4, 16, 2>::MIN_CTAS;
-    int dev = 0, optin = 0, resident = 0;
-    KGE_CUDA(cudaGetDevice(&dev));
-    KGE_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-    if (ws <= (size_t)optin) {
-      KGE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ws));
-      KGE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, threads, ws));
+  // (D: weight decay is on -- the kernels that carry its catch-up code; see catch_up)
+  auto launch = [&](auto decay_tag) -> int {
+    constexpr bool D = decltype(decay_tag)::value;
+    bool warp_racc = false;
+    if (two_per_warp && with_grad) {
+      const size_t ws = warp_racc_smem_bytes(model->relation.rows, model->relation.parts, model->d);
+      auto kern = kind == KGE_TRANSE ? train_fwd_kernel<KGE_TRANSE, 4, 16, 2, true, D>
+                                     : train_fwd_kernel<KGE_DISTMULT, 4, 16, 2, true, D>;
+      const int min_ctas = kind == KGE_TRANSE ? FwdBounds<KGE_TRANSE, 4, 16, 2>::MIN_CTAS
+                                              : FwdBounds<KGE_DISTMULT, 4, 16, 2>::MIN_CTAS;
+      int dev = 0, optin = 0, resident = 0;
+      KGE_CUDA(cudaGetDevice(&dev));
+      KGE_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+      if (ws <= (size_t)optin) {
+        KGE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ws));
+        KGE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, threads, ws));
+      }
+      if (resident >= min_ctas) {
+        warp_racc = true;
+        smem = ws;
+        grid = grid_for(n_total, threads / 16, resident);
+      }
     }
-    if (resident >= min_ctas) {
-      warp_racc = true;
-      smem = ws;
-      grid = grid_for(n_total, threads / 16, resident);
+#define CALL(V, G, N)                                                                                         \
+  switch (kind) {                                                                                             \
+    case KGE_TRANSE: train_fwd_kernel<KGE_TRANSE, V, G, N, false, D><<<grid, threads, smem, st>>>(a); break;     \
+    case KGE_DISTMULT: train_fwd_kernel<KGE_DISTMULT, V, G, N, false, D><<<grid, threads, smem, st>>>(a); break; \
+    case KGE_ROTATE: train_fwd_kernel<KGE_ROTATE, V, G, N, false, D><<<grid, threads, smem, st>>>(a); break;     \
+    case KGE_TRANSH: train_fwd_kernel<KGE_TRANSH, V, G, N, false, D><<<grid, threads, smem, st>>>(a); break;     \
+    case KGE_TRANSD: train_fwd_kernel<KGE_TRANSD, V, G, N, false, D><<<grid, threads, smem, st>>>(a); break;     \
+    default: train_fwd_kernel<KGE_COMPLEX, V, G, N, false, D><<<grid, threads, smem, st>>>(a); break;            \
+  }
+    if (warp_racc) {
+      if (kind == KGE_TRANSE) train_fwd_kernel<KGE_TRANSE, 4, 16, 2, true, D><<<grid, threads, smem, st>>>(a);
+      else train_fwd_kernel<KGE_DISTMULT, 4, 16, 2, true, D><<<grid, threads, smem, st>>>(a);
+    } else if (two_per_warp) {
+      if (kind == KGE_TRANSE) train_fwd_kernel<KGE_TRANSE, 4, 16, 2, false, D><<<grid, threads, smem, st>>>(a);
+      else train_fwd_kernel<KGE_DISTMULT, 4, 16, 2, false, D><<<grid, threads, smem, st>>>(a);
+    } else {
+      KGE_DISPATCH_ROWCFG(c, CALL);
     }
-  }
-#define CALL(V, G, N)                                                                                   \
-  switch (kind) {                                                                                       \
-    case KGE_TRANSE: train_fwd_kernel<KGE_TRANSE, V, G, N><<<grid, threads, smem, st>>>(a); break;      \
-    case KGE_DISTMULT: train_fwd_kernel<KGE_DISTMULT, V, G, N><<<grid, threads, smem, st>>>(a); break;  \
-    case KGE_ROTATE: train_fwd_kernel<KGE_ROTATE, V, G, N><<<grid, threads, smem, st>>>(a); break;      \
-    case KGE_TRANSH: train_fwd_kernel<KGE_TRANSH, V, G, N><<<grid, threads, smem, st>>>(a); break;      \
-    case KGE_TRANSD: train_fwd_kernel<KGE_TRANSD, V, G, N><<<grid, threads, smem, st>>>(a); break;      \
-    default: train_fwd_kernel<KGE_COMPLEX, V, G, N><<<grid, threads, smem, st>>>(a); break;             \
-  }
-  if (warp_racc) {
-    if (kind == KGE_TRANSE) train_fwd_kernel<KGE_TRANSE, 4, 16, 2, true><<<grid, threads, smem, st>>>(a);
-    else train_fwd_kernel<KGE_DISTMULT, 4, 16, 2, true><<<grid, threads, smem, st>>>(a);
-  } else if (two_per_warp) {
-    if (kind == KGE_TRANSE) train_fwd_kernel<KGE_TRANSE, 4, 16, 2><<<grid, threads, smem, st>>>(a);
-    else train_fwd_kernel<KGE_DISTMULT, 4, 16, 2><<<grid, threads, smem, st>>>(a);
-  } else {
-    KGE_DISPATCH_ROWCFG(c, CALL);
-  }
 #undef CALL
-  KGE_LAUNCH_CHECK();
-  return 0;
+    KGE_LAUNCH_CHECK();
+    return 0;
+  };
+  return a.adam.decays ? launch(std::true_type{}) : launch(std::false_type{});
 }
 
 extern "C" int kge_adam_apply(const kge_model_t* model, const kge_adam_t* adam, float grad_scale,
                               const float* grad_scale_dev, kge_stream_t stream) {
   if (int e = check_model(model, true)) return e;
   KGE_REQUIRE(adam && adam->step >= 1, KGE_E_ARG, "bad adam");
+  if (int e = kge_check_optimizer(adam)) return e;
   ApplyArgs a;
   a.m = *model;
   a.adam = make_adam_dev(model, adam);
@@ -1172,7 +1253,9 @@ extern "C" int kge_adam_apply(const kge_model_t* model, const kge_adam_t* adam, 
   a.win[2] = 4;
   const int grid = scan_grid(max_rows, scan_window(max_rows), 4);
   cudaStream_t st = (cudaStream_t)stream;
-#define CALL(V, G, N) adam_apply_kernel<V, G, N><<<grid, threads, 0, st>>>(a)
+#define CALL(V, G, N)                                                  \
+  if (a.adam.decays) adam_apply_kernel<V, G, N, true><<<grid, threads, 0, st>>>(a); \
+  else adam_apply_kernel<V, G, N, false><<<grid, threads, 0, st>>>(a)
   KGE_DISPATCH_ROWCFG(c, CALL);
 #undef CALL
   KGE_LAUNCH_CHECK();
@@ -1189,6 +1272,7 @@ extern "C" int kge_train_step(const kge_model_t* model, const kge_batch_t* b, co
 extern "C" int kge_adam_flush(const kge_model_t* model, const kge_adam_t* adam, kge_stream_t stream) {
   if (int e = check_model(model, true)) return e;
   KGE_REQUIRE(adam && adam->step >= 0, KGE_E_ARG, "bad adam");
+  if (int e = kge_check_optimizer(adam)) return e;
   if (adam->step == 0) return 0;
   AdamDev A = make_adam_dev(model, adam);
   RowCfg c = {};
@@ -1199,7 +1283,9 @@ extern "C" int kge_adam_flush(const kge_model_t* model, const kge_adam_t* adam, 
   for (int t = 0; t < 3; ++t) {
     const int win = scan_window(tabs[t]->rows);
     const int grid = scan_grid(tabs[t]->rows, win, 8);
-#define CALL(V, G, N) adam_flush_kernel<V, G, N><<<grid, threads, 0, st>>>(*tabs[t], model->d, A, win)
+#define CALL(V, G, N)                                                                              \
+  if (A.decays) adam_flush_kernel<V, G, N, true><<<grid, threads, 0, st>>>(*tabs[t], model->d, A, win); \
+  else adam_flush_kernel<V, G, N, false><<<grid, threads, 0, st>>>(*tabs[t], model->d, A, win)
     KGE_DISPATCH_ROWCFG(c, CALL);
 #undef CALL
     KGE_LAUNCH_CHECK();

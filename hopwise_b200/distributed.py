@@ -133,8 +133,8 @@ class RowSparseExchange:
 
         if model._state is not None:
             raise RuntimeError("multimem exchange must be enabled before the first training step")
-        if owner_adam and getattr(model, "learner", "adam") != "adam":
-            raise NotImplementedError("owner-sharded optimiser step implements Adam only")
+        if owner_adam and getattr(model, "learner", "adam") not in ("adam", "adamw"):
+            raise NotImplementedError("owner-sharded optimiser step implements Adam and AdamW only")
         group = self.group if self.group is not None else dist.group.WORLD
         ex = self
 

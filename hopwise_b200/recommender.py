@@ -186,7 +186,8 @@ class FusedKGEModel(KnowledgeRecommender):
         learner = str(_cfg_get(config, "learner", "adam")).lower()
         if learner == "sparse_adam":
             raise NotImplementedError("learner 'sparse_adam' needs sparse embedding gradients (nn.Embedding(sparse=True))")
-        if learner == "adamw":
+        weight_decay = float(_cfg_get(config, "weight_decay", 0.0) or 0.0)
+        if learner == "adamw" and weight_decay == 0.0:
             learner = "adam"
         if learner not in _abi.OPTIMIZERS:
             import warnings
@@ -194,8 +195,15 @@ class FusedKGEModel(KnowledgeRecommender):
             warnings.warn(f"unrecognized learner {learner!r}: Adam, as the reference trainer does (trainer.py:203-205)")
             learner = "adam"
         self.learner = learner
-        if float(_cfg_get(config, "weight_decay", 0.0) or 0.0) != 0.0:
-            raise NotImplementedError("fused KGE step implements weight_decay 0.0 only")
+        # weight decay is linear in the weights under AdamW (decoupled) and SGD (L2 term), so the rows a step does not
+        # touch can be caught up lazily; Adam's, Adagrad's and RMSprop's coupled L2 term cannot be
+        if weight_decay != 0.0 and learner not in ("adamw", "sgd"):
+            raise NotImplementedError(
+                f"fused KGE step: weight_decay with learner {learner!r} is not supported (its L2 term needs a dense "
+                "step over every element); use learner 'adamw' (decoupled decay) or 'sgd'")
+        if not (math.isfinite(weight_decay) and weight_decay >= 0.0):
+            raise NotImplementedError(f"fused KGE step: weight_decay {weight_decay} must be finite and >= 0")
+        self.weight_decay = weight_decay
         if _cfg_get(config, "clip_grad_norm", None):
             raise NotImplementedError("clip_grad_norm is not supported by the fused KGE step")
         if _cfg_get(config, "enable_amp", False) or _cfg_get(config, "enable_scaler", False):
@@ -378,11 +386,11 @@ class FusedKGEModel(KnowledgeRecommender):
         return m
 
     def _adam_struct(self, step: int) -> _abi.kge_adam_t:
-        hp = (self.learning_rate, self.betas[0], self.betas[1], self.adam_eps, self.replay_cap)
+        hp = (self.learning_rate, self.betas[0], self.betas[1], self.adam_eps, self.replay_cap, self.weight_decay)
         a = self.__dict__.get("_adam_cache")
         if a is None or a[0] != hp:   # one struct per hyper-parameter set; only the step changes between calls
             s = _abi.kge_adam_t()
-            s.lr, s.beta1, s.beta2, s.eps, s.replay_cap = hp
+            s.lr, s.beta1, s.beta2, s.eps, s.replay_cap, s.weight_decay = hp
             s.optimizer = _abi.OPTIMIZERS[self.learner]
             a = (hp, s)
             self.__dict__["_adam_cache"] = a
@@ -566,6 +574,9 @@ class FusedKGEModel(KnowledgeRecommender):
         a = self._adam_struct(self._step)
         _abi.check(lib.kge_adam_flush(C.byref(m), C.byref(a), _abi.stream_ptr()), "kge_adam_flush")
         self._dirty = False
+        # (the flush wrote weights -- under weight decay every row -- without a new step number: images keyed on the
+        # step must not outlive it)
+        self.invalidate_target_image()
 
     # ------------------------------------------------------------------ nn.Module hooks
     def train(self, mode: bool = True):

@@ -109,19 +109,25 @@ typedef struct {
 /* The optimiser hopwise's trainer builds (trainer/trainer.py:165-206), applied to the touched rows:
  *   KGE_OPT_ADAM     torch.optim.Adam(lr) (also AdamW with weight_decay 0): beta1, beta2, eps; rows that skipped steps
  *                    are caught up with the zero-gradient steps dense Adam gives them
- *   KGE_OPT_SGD      torch.optim.SGD(lr): p -= lr * g
+ *   KGE_OPT_SGD      torch.optim.SGD(lr, weight_decay): p -= lr * (g + weight_decay * p)
  *   KGE_OPT_ADAGRAD  torch.optim.Adagrad(lr): v += g^2; p -= lr * g / (sqrt(v) + eps)          (eps 1e-10)
  *   KGE_OPT_RMSPROP  torch.optim.RMSprop(lr): v = beta2 * v + (1 - beta2) * g^2; p -= lr * g / (sqrt(v) + eps)
  *                    (beta2 = alpha 0.99, eps 1e-8; v of a row that skipped n steps decays by alpha^n)
- * Under the last three a row without a gradient does not move, so nothing is replayed. */
-enum kge_optimizer { KGE_OPT_ADAM = 0, KGE_OPT_SGD = 1, KGE_OPT_ADAGRAD = 2, KGE_OPT_RMSPROP = 3 };
+ *   KGE_OPT_ADAMW    torch.optim.AdamW(lr, weight_decay): p *= (1 - lr * weight_decay), then KGE_OPT_ADAM's step
+ * Weight decay (KGE_OPT_ADAMW, KGE_OPT_SGD) reaches every row in every step, as a dense gradient does: rows that
+ * skipped steps, and rows no gradient ever touched (row_state -1), are caught up with the decay of every skipped step
+ * (exactly up to replay_cap steps, then p *= (1 - lr * weight_decay)^n).  Under Adagrad, RMSprop and SGD without decay a
+ * row without a gradient does not move, so nothing is replayed.  weight_decay must be finite and >= 0, and 0 under
+ * KGE_OPT_ADAM, KGE_OPT_ADAGRAD and KGE_OPT_RMSPROP (their coupled L2 term moves every element every step along a path
+ * with no closed form): every entry point that takes a kge_adam_t returns KGE_E_UNSUPPORTED otherwise. */
+enum kge_optimizer { KGE_OPT_ADAM = 0, KGE_OPT_SGD = 1, KGE_OPT_ADAGRAD = 2, KGE_OPT_RMSPROP = 3, KGE_OPT_ADAMW = 4 };
 
 typedef struct {
   float lr, beta1, beta2, eps;
   int32_t step;       /* 1-based index of the update this batch produces */
   int32_t replay_cap; /* zero-gradient steps replayed exactly per row before the closed-form tail */
   int32_t optimizer;  /* enum kge_optimizer */
-  int32_t reserved;
+  float weight_decay; /* KGE_OPT_ADAMW: decoupled decay; KGE_OPT_SGD: L2 term; 0 = none */
 } kge_adam_t;
 
 int kge_abi_version(void);
