@@ -230,14 +230,26 @@ __device__ __forceinline__ ImgScale img_scale(const float* header) {
 //   K 2^-22 (nqs tms 1.001 + 2^8 c)    fp32 accumulation of K products (one truncated ulp each, partial sums bounded by
 //                                      the sum of magnitudes)
 //   3 * 2^-14 c                        the hi/mid/lo split of W (exact up to the subnormal floor of each piece)
+//   (K + 2) 2^-24 chain                the rescore's own fp32 chain: the top-k is decided by its scores, not by the real
+//                                      ones, and one sequential chain over <= K - 2 columns is off by at most (K + 2)
+//                                      2^-24 times the sum of its terms' magnitudes -- chain = S |q| tmax (q . t), or
+//                                      S (|q| + tmax)^2 / 2 (a = (|q|^2 - |q - t|^2) / 2).  Without it a row whose |q|
+//                                      dwarfs every |t| (L2 models) ranks targets the fp32 chain cannot tell apart, and
+//                                      the id order among those ties picks members the filter dropped.  (K >= P + 3
+//                                      columns for the L2 models: the spare covers the rounding of sqrtf(acc) as well.)
+//   2^-23 last                         RotatE's reported score margin - sqrtf(acc) is rounded once more, to ulps of
+//                                      the margin: targets whose |q - t| differ by less than that tie, which is
+//                                      |margin| (|q| + tmax) 2^-24 in the units of a; last = S |margin| (|q| + tmax).
 // and 1 % on top for the fp32 evaluation of the bound itself.
-__device__ __forceinline__ float row_eps(float nqs, float tms, int kp, float c) {
+__device__ __forceinline__ float row_eps(float nqs, float tms, int kp, float c, float chain, float last) {
   const float K = (float)kp;
   float e = (9.765625e-4f + 9.5367431640625e-7f) * nqs * tms;
   e += 6.103515625e-5f * sqrtf(K) * (nqs + tms) * 1.001f;
   e += K * 3.725290298461914e-9f;
   e += K * 2.384185791015625e-7f * (nqs * tms * 1.001f + 256.f * c);
   e += 3.f * 6.103515625e-5f * c;
+  e += (K + 2.f) * 5.9604644775390625e-8f * chain;
+  e += 1.1920928955078125e-7f * last;
   return e * 1.01f;
 }
 
@@ -612,7 +624,11 @@ __global__ void __launch_bounds__(sweep_threads(NH, NCOL, NMMA), (NBUF == 1 && N
     }
     if (lane == 0) {
       const float nqs = scalbnf(sqrtf(nq) * 1.0001f, e_i), tms = scalbnf(isc.tmax, isc.e_t);
-      const float eps = bad ? INFINITY : row_eps(nqs, tms, kp, a.dist ? scalbnf(1.0f, e_c) : 0.f);
+      // S (|q| + tmax)^2 = ((|q| + tmax) 2^e_i) ((|q| + tmax) 2^e_t)
+      const float qt_i = nqs + scalbnf(isc.tmax, e_i);   // (|q| + tmax) 2^e_i
+      const float chain = a.dist ? 0.5f * qt_i * (scalbnf(sqrtf(nq) * 1.0001f, isc.e_t) + tms) : nqs * tms;
+      const float last = a.s.m.model == KGE_ROTATE ? fabsf(a.s.m.margin) * scalbnf(qt_i, isc.e_t) : 0.f;
+      const float eps = bad ? INFINITY : row_eps(nqs, tms, kp, a.dist ? scalbnf(1.0f, e_c) : 0.f, chain, last);
       const float inv = scalbnf(1.0f, -(e_i + isc.e_t));
       eps_row[u] = eps;
       inv_row[u] = inv;

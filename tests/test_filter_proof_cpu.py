@@ -34,19 +34,25 @@ def _exp_for(maxabs):
     return 0 if maxabs <= 0 else int(np.clip(7 - int(np.floor(np.log2(maxabs))), -60, 60))
 
 
-def row_eps(nqs, tms, kp, c):
-    """csrc/mma_topk.cu row_eps(), term by term."""
+def row_eps(nqs, tms, kp, c, chain, last):
+    """csrc/mma_topk.cu row_eps(), term by term.  chain: the magnitude of the exact fp32 chain's terms; last: RotatE's
+    S |margin| (|q| + tmax), for the rounding of margin - sqrtf(acc) (both 0 for the fp16 sweep's own error)."""
     e = (2.0 ** -10 + 2.0 ** -20) * nqs * tms
     e += 2.0 ** -14 * np.sqrt(kp) * (nqs + tms) * 1.001
     e += kp * 2.0 ** -28
     e += kp * 2.0 ** -22 * (nqs * tms * 1.001 + 256.0 * c)
     e += 3.0 * 2.0 ** -14 * c
+    e += (kp + 2) * 2.0 ** -24 * chain
+    e += 2.0 ** -23 * last
     return e * 1.01
 
 
-def sweep_operands(Q, T, dist):
+def sweep_operands(Q, T, dist, margin=0.0, sweep_only=False):
     """What the image kernel and the sweep's setup build: scaled fp16 operands, per-row scale S_i and eps_i.
-    Returns (ahat [rows, n] fp32 in scaled units, S [rows], eps [rows] scaled)."""
+    Returns (ahat [rows, n] fp32 in scaled units, S [rows], eps [rows] scaled).  margin: RotatE's (0 for the other
+    models); sweep_only: eps without the rescore's terms (chain and last), i.e. the bound of |a^ - S a| alone.  A row the fp16 scaling cannot hold
+    (a non-finite |q|^2, or an L2 row whose c_i = 2^e_c is no normal fp16 number) gets eps = inf and a nan ahat row:
+    the kernel flags it for the exact path."""
     d = T.shape[1]
     kd = d + (3 if dist else 0)
     kp = (kd + 15) // 16 * 16
@@ -57,44 +63,66 @@ def sweep_operands(Q, T, dist):
     Th = _f16(np.ldexp(T.astype(np.float32), e_t))
     if dist:
         W = np.ldexp(np.float32(-0.5) * tn2, e_w).astype(np.float32)
-        hi = _f16(W)
-        mid = _f16(W - hi)
-        lo = _f16(W - hi - mid)
+        with np.errstate(over="ignore", invalid="ignore"):   # (|t|^2 / 2 > 2^68: e_w is clamped, W overflows fp16)
+            hi = _f16(W)
+            mid = _f16(W - hi)
+            lo = _f16(W - hi - mid)
     ahat, S, eps = [], [], []
     for q in Q:
-        e_i = _exp_for(np.abs(q).max())
+        with np.errstate(over="ignore", invalid="ignore"):
+            bad = not np.isfinite((q.astype(np.float32) ** 2).sum(dtype=np.float32))
+            e_i = _exp_for(np.abs(q).max()) if not bad else 0
         e_c = 0
         if dist:
             e_c = e_i + e_t - e_w
             if e_c > 15:
                 e_i -= e_c - 15
                 e_c = 15
-            assert e_c >= -14
+            bad = bad or e_c < -14 or e_i < -60
+        S.append(2.0 ** (e_i + e_t))
+        if bad:
+            ahat.append(np.full(len(T), np.nan, dtype=np.float32))
+            eps.append(np.inf)
+            continue
         qh = _f16(np.ldexp(q.astype(np.float32), e_i))
         row = (qh[None, :].astype(np.float64) @ Th.astype(np.float64).T)[0]
         if dist:
             c = np.float64(2.0 ** e_c)
-            row = row + c * (hi.astype(np.float64) + mid + lo)
+            with np.errstate(invalid="ignore"):
+                row = row + c * (hi.astype(np.float64) + mid + lo)
         ahat.append(row.astype(np.float32))          # (fp32 accumulation: the bound has a term for it)
         nq = np.sqrt((q.astype(np.float64) ** 2).sum()) * 1.0001
-        S.append(2.0 ** (e_i + e_t))
-        eps.append(row_eps(nq * 2.0 ** e_i, float(tmax) * 2.0 ** e_t, kp, 2.0 ** e_c if dist else 0.0))
+        nqs, tms = nq * 2.0 ** e_i, float(tmax) * 2.0 ** e_t
+        qt_i = nqs + float(tmax) * 2.0 ** e_i
+        chain = 0.5 * qt_i * (nq * 2.0 ** e_t + tms) if dist else nqs * tms
+        last = abs(margin) * qt_i * 2.0 ** e_t
+        if sweep_only:
+            chain = last = 0.0
+        eps.append(row_eps(nqs, tms, kp, 2.0 ** e_c if dist else 0.0, chain, last))
     return np.stack(ahat), np.array(S), np.array(eps)
 
 
-def _filter_row(ahat, eps, k, masked, trig=CAND - 5):
-    """One row of the sweep: returns (set of kept (chunk, group) pairs, flagged)."""
+def _filter_row(ahat, eps, k, masked, trig=CAND - 5, lists=None, stats=None):
+    """One row of the sweep and of the rescore's selection: returns (set of kept (chunk, group) pairs, flagged).
+
+    `lists` = the row's candidate lists, one per (target split, column slice): each a sequence of tiles, each tile the
+    ids of the chunks the list sees in it (a list is checked for compaction at the end of every tile).  Default: one
+    list of every chunk, four chunks per tile.  `stats`, when given, receives what the rescore kernel sees: E (entries
+    of all lists), groups (groups it scores), tau and thr (its final threshold, scaled units)."""
     n = len(ahat)
     n_chunks = (n + CH - 1) // CH
-    pad = np.full(n_chunks * CH, 0.0, dtype=np.float32)   # the image pads the last tile with zero rows
+    if lists is None:
+        lists = [[tuple(range(c, min(c + 4, n_chunks))) for c in range(0, n_chunks, 4)]]
+    top = max(c for lst in lists for tile in lst for c in tile) + 1
+    pad = np.full(max(top, n_chunks) * CH, 0.0, dtype=np.float32)   # the image pads the last tile with zero rows
     pad[:n] = ahat
-    unsafe = np.zeros(n_chunks, dtype=bool)
+    unsafe = np.zeros(len(pad) // CH, dtype=bool)
     for j in np.nonzero(masked)[0]:
         unsafe[j // CH] = True
     if n % CH:
         unsafe[n // CH:] = True
-    entries, thr = [], -np.inf       # entry = (chunk max, chunk id, group mask, unsafe)
-    flagged = False
+    unsafe[n_chunks:] = True
+    entries, thr0 = [], -np.inf      # entry = (chunk max, chunk id, group mask, unsafe)
 
     def compact(entries):
         safe = sorted((e[0] for e in entries if not e[3]), reverse=True)
@@ -102,22 +130,28 @@ def _filter_row(ahat, eps, k, masked, trig=CAND - 5):
         new_thr = np.float32(tau) - np.float32(2.0) * np.float32(eps)
         return [e for e in entries if e[0] >= new_thr], new_thr
 
-    for c in range(n_chunks):
-        blk = pad[c * CH:(c + 1) * CH].reshape(CH // GRP, GRP)
-        gm = blk.max(axis=1)
-        tm = gm.max()
-        if tm >= thr:
-            entries.append((tm, c, gm >= thr, bool(unsafe[c])))
-        if (c % 4 == 3 or c == n_chunks - 1) and len(entries) > trig:   # checked once per 128-target tile
-            entries, thr = compact(entries)
-            if len(entries) > CAND - ROOM:
-                return set(), True
-    # re-score side: final tau over everything that survived, then the groups of the surviving chunks
-    safe = sorted((e[0] for e in entries if not e[3] and e[0] >= thr), reverse=True)
+    for lst in lists:
+        mine, thr = [], -np.inf
+        for tile in lst:
+            for c in tile:
+                gm = pad[c * CH:(c + 1) * CH].reshape(CH // GRP, GRP).max(axis=1)
+                tm = gm.max()
+                if tm >= thr:
+                    mine.append((tm, c, gm >= thr, bool(unsafe[c])))
+            if len(mine) > trig:
+                mine, thr = compact(mine)
+                if len(mine) > CAND - ROOM:
+                    return set(), True
+        entries += mine
+        thr0 = max(thr0, thr)
+    # re-score side: final tau over everything that clears every list's threshold, then the groups of the survivors
+    safe = sorted((e[0] for e in entries if not e[3] and e[0] >= thr0), reverse=True)
     tau = safe[k - 1] if len(safe) >= k else -np.inf
-    final_thr = max(thr, np.float32(tau) - np.float32(2.0) * np.float32(eps))
+    final_thr = max(thr0, np.float32(tau) - np.float32(2.0) * np.float32(eps))
     kept = {(e[1], g) for e in entries if e[0] >= final_thr for g in np.nonzero(e[2])[0]}
-    return kept, flagged
+    if stats is not None:
+        stats.update(E=len(entries), groups=len(kept), tau=tau, thr=final_thr)
+    return kept, False
 
 
 # enough targets for several compactions per row (a list fills after 123 appended chunks of 32 targets)

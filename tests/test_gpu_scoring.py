@@ -288,6 +288,17 @@ def test_mma_raw_scores_match_fp16_emulation(name, d):
     scale = np.abs(want).max()
     np.testing.assert_allclose(raw, want, rtol=0, atol=3e-4 * scale)   # q of RotatE differs by sincos ulps
     assert np.abs(raw - want).mean() < 3e-5 * scale
+    # the bound the filter rests on, per element: |a^ - S a| <= eps_i (csrc/mma_topk.cu row_eps, restated in numpy,
+    # without the terms for the rescore's own rounding)
+    from test_filter_proof_cpu import sweep_operands
+
+    dist = name in ("TransE", "RotatE")
+    exact = qc.astype(np.float64) @ tc.astype(np.float64).T
+    if dist:
+        exact = exact - 0.5 * (tc.astype(np.float64) ** 2).sum(1)[None, :]
+    _, S, eps = sweep_operands(qc, tc, dist, sweep_only=True)
+    err = np.abs(raw.astype(np.float64) * S[:, None] - S[:, None] * exact)
+    assert np.all(err <= eps[:, None]), f"max |a^ - S a| / eps = {(err / eps[:, None]).max():.3f}"
 
 
 @pytest.mark.parametrize("name,d,I,k", [("DistMult", 64, 20000, 20), ("ComplEx", 64, 9000, 20), ("TransE", 100, 12000, 10),
