@@ -1256,7 +1256,16 @@ extern "C" int kge_adam_apply(const kge_model_t* model, const kge_adam_t* adam, 
 #define CALL(V, G, N)                                                  \
   if (a.adam.decays) adam_apply_kernel<V, G, N, true><<<grid, threads, 0, st>>>(a); \
   else adam_apply_kernel<V, G, N, false><<<grid, threads, 0, st>>>(a)
-  KGE_DISPATCH_ROWCFG(c, CALL);
+  // Rows of 17..32 float4 (d = 68..128) with user and entity tables in L2 (the forward's two-triples-per-warp regime):
+  // nearly every row is touched, and a warp that updates one row at a time waits one L2 round trip per row.  Half-warp
+  // groups with two fragments per lane update two rows at once.  The update is element-wise, so the rows come out the
+  // same bit for bit.
+  const double table_bytes = ((double)model->user.rows + (double)model->entity.rows) * model->d * 16.0;
+  if (c.vec == 4 && c.g == 32 && c.nch == 1 && table_bytes < 96e6) {
+    CALL(4, 16, 2);
+  } else {
+    KGE_DISPATCH_ROWCFG(c, CALL);
+  }
 #undef CALL
   KGE_LAUNCH_CHECK();
   return 0;
